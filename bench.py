@@ -4,6 +4,13 @@
     python bench.py --gpus 1 --steps 20 --warmup 3                 # this repo's CUDA path on cuda:0
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU: BASELINE configs[2], global batch 256
     python bench.py --impl reference --steps 3 --warmup 1           # the UNMODIFIED reference step on the host cores
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs out/  # also write the last timed step's outputs
+
+--dump-outputs DIR writes, right after the timed steps, what a caller of the timed path holds after its last step:
+losses.npy (the [K, 4] loss rows MultiGeneratorGAN.step returned) and generator<i>_state.npy (discriminator_state.npy
+at gan-native), every floating-point state_dict entry of that model after the update, flattened in state_dict order;
+infer-1080p writes sr.npy, a fixed sample of the upscaled frames.  On N > 1 GPUs rank 0 writes them.  Inputs and initial
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (N=1): BASELINE.json configs[1] -- K=3 generators (count inferred from src/main.py:28), each doing the
 reference's train_generator step (SRResNet fwd+bwd, ReconstructionLoss, Adam) on one batch of 16x3x96x96 synthetic LR
@@ -60,7 +67,15 @@ def parse():
                     "streaming chunks of frames (A/B; materialises every frame's activations)")
     ap.add_argument("--no-graphs", action="store_true", help="enqueue every kernel from the host instead of replaying "
                     "one captured CUDA graph per generator step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last "
+                    "timed step returned and the model state it left as DIR/<name>.npy (float32, at most 64 MB in all), "
+                    "so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's CUDA path (--impl ours)")
+    return a
 
 
 def geometry(a):
@@ -81,6 +96,35 @@ def workload_name(a):
     cfg = "cfg2" if world == 1 else f"cfg3 (global batch {b * world} over {world} GPUs)"
     return (f"{cfg}: {a.generators} generators x train_generator (SRResNet fwd+bwd + ReconstructionLoss + Adam), "
             f"{b}x3x{h}x{w} LR -> x4 HR per GPU, pixel-loss mode (reference D invalid at this HR size)")
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes every tensor of ``arrays`` as ``path/<name>.npy`` in float32, 64 MB in all at most.  Tensors are taken
+    smallest first and each may use an equal part of the budget still left; one larger than its part is written as
+    the flat elements at a fixed set of indices (numpy default_rng(0), sorted, duplicates dropped), so that runs with
+    the same arguments write the same elements."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BUDGET_BYTES - 1024 * len(arrays)         # room for the .npy headers
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        t = t.detach().float()
+        share = left // (len(arrays) - i) // 4
+        if t.numel() > share:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), share))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        left -= 4 * t.numel()
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
+def state_vector(module):
+    """Every floating-point entry of ``module.state_dict()`` (parameters and BatchNorm running statistics), flattened
+    and concatenated in state_dict order."""
+    import torch
+    return torch.cat([v.detach().reshape(-1).float() for v in module.state_dict().values() if v.is_floating_point()])
 
 
 def peaks():
@@ -152,7 +196,7 @@ def cpu_reference_steps(a, steps, warmup, budget_s=150.0):
     kind = "port"
     try:
         from oracle import make_ref
-        if make_ref.available() or os.path.isdir("/root/reference/src"):
+        if make_ref.available():
             models, train, utils = make_ref.import_reference()
             kind = "reference"
     except Exception:
@@ -263,6 +307,8 @@ def run_infer(a):
         e1.record()
         torch.cuda.synchronize()
         clocks = sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"sr": y})
     ms = e0.elapsed_time(e1) / a.steps
     flop = 4436352.0 * H * W * B
     pk, src = peaks()
@@ -426,8 +472,10 @@ def run_ours(a):
         barrier()
         return float(ms.item())
 
+    step_losses = [None]
+
     def step_resident():
-        trainer.step(lr_dev, hr_dev)
+        step_losses[0] = trainer.step(lr_dev, hr_dev)
 
     d2h_bytes = [0]
     e2e_steps = [a.steps]
@@ -473,6 +521,13 @@ def run_ours(a):
         sampler.start()
     total_ms = timed(step_resident, a.steps)
     clocks = sampler.stop() if rank == 0 else {}
+    if rank == 0 and a.dump_outputs:
+        # the later legs below keep training the same models: the state is taken here, right after the timed steps
+        outputs = {"losses": step_losses[0]}
+        outputs.update({f"generator{i}_state": state_vector(g) for i, g in enumerate(gens)})
+        if disc is not None:
+            outputs["discriminator_state"] = state_vector(disc)
+        dump_outputs(a.dump_outputs, outputs)
     launches = L.srg_total_launches() - launches0
     if use_graphs and trainer.launches_per_step():
         launches = trainer.launches_per_step() * a.steps      # replayed graph nodes (counted once at capture)

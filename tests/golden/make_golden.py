@@ -77,9 +77,9 @@ def make_adversarial_fixture(models, train, utils):
             torch.autograd.set_detect_anomaly(False)
         arrays[f"{tag}/d_real0"] = real0.numpy()
         arrays[f"{tag}/d_fake0"] = fake0.numpy()
-        for k in ("model.0.weight", "model.0.bias", "model.4.weight", "model.4.bias"):
+        for k in ("model.0.weight", "model.0.bias", "model.4.bias"):
             arrays[f"{tag}/d_grad/{k}"] = grads[k].numpy()
-        for k in ("model.8.weight", "model.12.weight"):
+        for k in ("model.4.weight", "model.8.weight", "model.12.weight"):
             arrays[f"{tag}/d_grad_sub/{k}"] = grads[k].flatten()[::97].numpy()      # strided sample of the large tensors
         rec = {"lr_shape": [1, 3, h, w], "hr_shape": [1, 3, 4 * h, 4 * w], "seeds": {"g": 14, "d": 15, "data": 16},
                "d_losses": d_losses, "d_grad_norms": {k: float(v.double().norm()) for k, v in grads.items()},
@@ -119,14 +119,26 @@ def make_adversarial_fixture(models, train, utils):
 def make_checkpoint_fixture(models):
     """A checkpoint written the way the reference writes it under DDP (src/train.py:123-125 saves
     ``generator.state_dict()`` of the DDP-wrapped model: every key carries the ``module.`` prefix), for the f-1
-    interop test.  Tiny SRResNet (2 residual blocks) to keep the file small.  python tests/golden/make_golden.py checkpoint"""
+    interop test.  Tiny SRResNet (2 residual blocks).  Its parameters are the reference's default initialisation under
+    seed 21, which oracle.srgan_oracle.init_srresnet_state reproduces bit for bit, so only the entries that initialisation
+    does not give (the BatchNorm buffers moved by one training pass) are stored, in reference_ddp_checkpoint_buffers.pth;
+    reference_ddp_checkpoint.json records the key order and a sha256 of every entry, against which tests/conftest.py
+    rebuilds the whole checkpoint.  python tests/golden/make_golden.py checkpoint"""
+    import hashlib
     torch.manual_seed(21)
     g = models.SRResNet(num_residuals=2)
+    init = {k: v.clone() for k, v in g.state_dict().items()}
     g.train()
     with torch.no_grad():
         g(torch.rand(1, 3, 8, 8))             # one training-mode pass: BatchNorm buffers / num_batches_tracked move
     sd = {"module." + k: v for k, v in g.state_dict().items()}
-    torch.save(sd, os.path.join(HERE, "reference_ddp_checkpoint.pth"))
+    torch.save({k: v for k, v in sd.items() if not torch.equal(v, init[k[len("module."):]])},
+               os.path.join(HERE, "reference_ddp_checkpoint_buffers.pth"))
+    meta = {"seed": 21, "num_residuals": 2, "keys": list(sd),
+            "entries": {k: [str(v.dtype), list(v.shape), hashlib.sha256(v.numpy().tobytes()).hexdigest()]
+                        for k, v in sd.items()}}
+    with open(os.path.join(HERE, "reference_ddp_checkpoint.json"), "w") as f:
+        json.dump(meta, f, indent=1)
     g.eval()
     x = torch.linspace(0, 1, 3 * 12 * 10).reshape(1, 3, 12, 10)
     with torch.no_grad():
@@ -202,14 +214,15 @@ def main():
     grads = {k: p.grad for k, p in g.named_parameters()}
     sel = ["conv1.weight", "conv1.bias", "residual_blocks.0.conv1.weight", "residual_blocks.0.bn1.weight",
            "residual_blocks.0.bn1.bias", "residual_blocks.7.conv2.weight", "residual_blocks.15.bn2.weight",
-           "conv2.weight", "upsample.0.weight", "upsample.3.weight", "upsample.3.bias", "conv3.weight",
-           "conv3.bias"]
+           "conv2.weight", "upsample.3.bias", "conv3.weight", "conv3.bias"]
+    sel_sub = ["upsample.0.weight", "upsample.3.weight"]      # the largest gradients: strided sample, file under 1 MB
     np.savez_compressed(
         os.path.join(HERE, "generator_tiny.npz"),
         y_eval=y_eval.numpy(), y_train=y_train.detach().numpy(),
         com=np.float64(com.item()), tv=np.float64(tv.item()),
         bn_rm=g.residual_blocks[0].bn1.running_mean.numpy(), bn_rv=g.residual_blocks[0].bn1.running_var.numpy(),
         **{"grad/" + k: grads[k].numpy() for k in sel},
+        **{"grad_sub/" + k: grads[k].flatten()[::97].numpy() for k in sel_sub},
     )
     out["generator_tiny"] = {
         "seed": 1, "lr_shape": [2, 3, 16, 24], "hr_shape": [2, 3, 64, 96], "init_checksum": init_ck,

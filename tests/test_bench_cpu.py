@@ -39,6 +39,34 @@ def test_workload_per_gpu_count_follows_baseline_configs(monkeypatch, world, per
     assert B.geometry(_args(workload="gan-native")) == (12, 128, 256)  # src/train.py:94, src/transformers.py:74
 
 
+def test_dump_outputs_keeps_small_arrays_and_samples_large_ones_the_same_way(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    B = _bench_module()
+    monkeypatch.setattr(B, "DUMP_BUDGET_BYTES", 1 << 20)
+    big = torch.arange(1 << 20, dtype=torch.float64)
+    for run in ("a", "b"):
+        B.dump_outputs(str(tmp_path / run), {"losses": torch.ones(3, 4), "state": big})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["losses.npy", "state.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 1 << 20
+    losses = np.load(tmp_path / "a" / "losses.npy")
+    assert losses.dtype == np.float32 and losses.shape == (3, 4)
+    state = np.load(tmp_path / "a" / "state.npy")
+    assert state.dtype == np.float32 and 0 < state.size < big.numel()
+    share = ((1 << 20) - 2 * 1024 - losses.nbytes) // 4             # the budget left once the small array is whole
+    idx = np.unique(np.random.default_rng(0).integers(0, big.numel(), share))
+    assert np.array_equal(state, idx.astype(np.float32))            # element i of the arange is i
+    assert np.array_equal(state, np.load(tmp_path / "b" / "state.npy"))
+
+
+def test_steps_below_one_and_dumps_of_the_reference_arm_are_refused():
+    for flags in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *flags], cwd=ROOT, capture_output=True,
+                           text=True, timeout=60)
+        assert r.returncode == 2 and "error" in r.stderr, flags
+
+
 def _run_reference_arm(env_extra, *flags):
     env = dict(os.environ)
     env.update(env_extra)

@@ -238,10 +238,10 @@ def test_adversarial_steps_match_reference_fixtures(S, golden_dir):
             assert abs(loss - ref) < b["loss"] * abs(ref) + 1e-4, (tag, i, loss, ref)
             if i == 0:
                 grads = {k: p.grad.detach().clone() for k, p in d.named_parameters()}
-        for k in ("model.0.weight", "model.4.weight"):
+        for k in ("model.0.weight",):
             c, r = _cos(grads[k], torch.from_numpy(z[f"{tag}/d_grad/{k}"]))
             assert c > b["dcos"] and abs(r - 1) < b["dratio"], (tag, k, c, r)
-        for k in ("model.8.weight", "model.12.weight"):
+        for k in ("model.4.weight", "model.8.weight", "model.12.weight"):
             c, _ = _cos(grads[k].flatten()[::97], torch.from_numpy(z[f"{tag}/d_grad_sub/{k}"]))
             r = float(grads[k].double().norm()) / rec["d_grad_norms"][k]
             assert c > b["dcos"] and abs(r - 1) < b["dratio"], (tag, k, c, r)

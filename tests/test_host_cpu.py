@@ -186,13 +186,12 @@ def test_conv9_rows_schedule_applies_every_row_tap_once_per_output_row():
     assert L.srg_conv9_rows_window(16, None, None, None, None) != 0
 
 
-def test_reference_written_checkpoint_fixture_loads_on_cpu(golden_dir):
+def test_reference_written_checkpoint_fixture_loads_on_cpu(reference_ddp_checkpoint):
     """f-1 on the host side: the reference-written DDP checkpoint (module. prefix) maps onto the drop-in module's keys."""
-    import os
     import torch
     import srgan_b200 as S
     g = S.SRResNet(num_residuals=2)
-    sd = torch.load(os.path.join(golden_dir, "reference_ddp_checkpoint.pth"), map_location="cpu", weights_only=True)
+    sd = torch.load(reference_ddp_checkpoint, map_location="cpu", weights_only=True)
     assert all(k.startswith("module.") for k in sd)
     res = S.load_reference_checkpoint(g, sd)
     assert not res.missing_keys and not res.unexpected_keys

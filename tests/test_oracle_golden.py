@@ -42,9 +42,11 @@ def test_generator_forward_loss_grads(gj, golden_dir):
     np.testing.assert_allclose(sd["residual_blocks.0.bn1.running_mean"].numpy(), z["bn_rm"], atol=1e-7)
     np.testing.assert_allclose(sd["residual_blocks.0.bn1.running_var"].numpy(), z["bn_rv"], atol=1e-7)
     for k in z.files:
-        if k.startswith("grad/"):
+        if k.startswith(("grad/", "grad_sub/")):
             ref = z[k]
-            got = grads[k[5:]].numpy()
+            got = grads[k.split("/", 1)[1]].numpy()
+            if k.startswith("grad_sub/"):
+                got = got.flatten()[::97]          # the fixture holds a strided sample of the largest gradients
             assert np.abs(got - ref).max() <= 1e-5 * max(np.abs(ref).max(), 1e-6) + 1e-9, k
     for k, n in gj["generator_tiny"]["grad_norms"].items():
         # biases feeding a training-mode BatchNorm have a mathematically zero gradient: only fp32 noise (~1e-9) there

@@ -41,9 +41,9 @@ def main():
             if i == 0:
                 grads = {k: p.grad.detach().clone() for k, p in d.named_parameters()}
         print("  d_losses ours", losses, "ref", rec["d_losses"])
-        for k in ("model.0.weight", "model.4.weight"):
+        for k in ("model.0.weight",):
             print(f"  d grad {k}: cos/ratio {cos(grads[k], torch.from_numpy(z[f'{tag}/d_grad/{k}']))}")
-        for k in ("model.8.weight", "model.12.weight"):
+        for k in ("model.4.weight", "model.8.weight", "model.12.weight"):
             print(f"  d grad {k} (1/97 sample): cos/ratio {cos(grads[k].flatten()[::97], torch.from_numpy(z[f'{tag}/d_grad_sub/{k}']))}  "
                   f"norm ours {float(grads[k].double().norm()):.5f} ref {rec['d_grad_norms'][k]:.5f}")
         # GAN-mode generator step with the INITIAL discriminator
