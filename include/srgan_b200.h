@@ -301,6 +301,18 @@ int srg_adam_step_dev(float* params, const float* grads, float* exp_avg, float* 
 int srg_image_enhance(const float* x_nchw, int N, int C, int H, int W, float factor, float* out_nchw, void* stream);
 /* out1[0] (DEVICE double) = mean((a - b)^2); calculate_psnr (src/utils.py:141-144) = 10 * log10(1 / mse) */
 int srg_mse(const float* a, const float* b, int64_t n, void* scratch, size_t scratch_bytes, double* out1, void* stream);
+/* replaces the per-image metric loop of compute_score (src/train.py:263-294) over calculate_psnr / calculate_ssim
+ * (src/utils.py:141-151), for N images of 3 x H x W fp32 (NCHW) at once, both metrics in one pass over sr and hr:
+ *   psnr_out[n] (DEVICE double) = 10 * log10(1 / mean((sr_n - hr_n)^2)), +inf for identical images (data_range 1)
+ *   ssim_out[n] (DEVICE double) = skimage structural_similarity(sr_n, hr_n, win_size=3) with the array taken as a 3-D
+ *                volume (channel_axis None): 3x3x3 uniform window, sample covariance (27/26), C1 = 1e-4, C2 = 9e-4, the
+ *                map cropped by 1 on every axis = the mean of S over channel 1, rows 1..H-2, columns 1..W-2.
+ * Needs C == 3, H >= 3, W >= 3, N >= 1 and scratch_bytes >= srg_image_metrics_scratch_bytes(N, H, W) (caller-owned,
+ * 8-byte aligned); checked before any CUDA call.  An image's results do not depend on N or on its position in the batch.
+ * Two kernel launches, no allocation, copy or synchronisation: capturable into a CUDA graph. */
+size_t srg_image_metrics_scratch_bytes(int N, int H, int W); /* 0 for invalid sizes */
+int srg_image_metrics(const float* sr, const float* hr, int N, int C, int H, int W, void* scratch, size_t scratch_bytes,
+                      double* psnr_out, double* ssim_out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Image-size transforms either side of the path (src/transformers.py:73-82, applied per image in src/utils.py:34-47):

@@ -14,13 +14,13 @@ from .optim import Adam
 from .policy import (GAN, PIXEL, MultiGeneratorPolicy, PolicyConfig, decide, gan_probability, interpolate_models,
                      shuffle_lists_in_same_order)
 from .train import (DevicePrefetcher, GraphedDiscriminatorStep, GraphedGeneratorStep, GraphedMultiGeneratorStep, MultiGeneratorGAN, joint_pixel_generator_steps, train_discriminator, train_discriminator_async, train_generator,
-                    train_generator_async, train_one_epoch, setup_training)
+                    train_generator_async, train_one_epoch, compute_score, setup_training)
 from . import parallel
 from . import transformers
 from .vgg import VGGFeatureExtractor, perceptal_loss, perceptual_loss
-from .evaluation import (ImageEnhancer, calculate_psnr, load_reference_checkpoint, resume_learning_rates,
-                         save_reference_checkpoint, strip_module_prefix)
+from .evaluation import (ImageEnhancer, calculate_psnr, calculate_ssim, image_metrics, load_reference_checkpoint,
+                         resume_learning_rates, save_reference_checkpoint, strip_module_prefix)
 
 __all__ = ["joint_pixel_generator_steps", "SRResNet", "ResidualBlock", "Discriminator", "ReconstructionLoss", "tanh_mean", "Adam", "train_generator",
-           "train_discriminator", "train_one_epoch", "DevicePrefetcher", "MultiGeneratorGAN", "GraphedGeneratorStep", "MultiGeneratorPolicy", "PolicyConfig",
+           "train_discriminator", "train_one_epoch", "compute_score", "image_metrics", "calculate_ssim", "DevicePrefetcher", "MultiGeneratorGAN", "GraphedGeneratorStep", "MultiGeneratorPolicy", "PolicyConfig",
            "build", "lib", "parallel"]

@@ -16,7 +16,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 # SRG_LIB_SO: developer override for same-box A/B runs against an older build of the library (never rebuilt)
 SO_PATH = os.environ.get("SRG_LIB_SO") or os.path.join(HERE, "libsrgan_b200.so")
-SOURCES = ["conv_gemm.cu", "conv_ops.cu", "vgg_ops.cu", "resample.cu", "trunk_fused.cu", "wgrad_gemm.cu", "elementwise.cu", "peer_sync.cu", "generator.cu", "discriminator.cu", "api.cu"]
+SOURCES = ["conv_gemm.cu", "conv_ops.cu", "vgg_ops.cu", "resample.cu", "trunk_fused.cu", "wgrad_gemm.cu", "elementwise.cu", "peer_sync.cu", "generator.cu", "discriminator.cu", "metrics.cu", "api.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC"]
 
@@ -174,6 +174,9 @@ EXPORTS = {
     "srg_point_loss": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_float, c_void_p]),
     "srg_image_enhance": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
     "srg_mse": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p]),
+    "srg_image_metrics_scratch_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "srg_image_metrics": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p, c_void_p,
+                                  c_void_p]),
     "srg_adam_step_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_float, c_float, c_float,
                                   c_void_p, c_float, c_void_p]),
     "srg_adam_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_float, c_float, c_float, c_float,

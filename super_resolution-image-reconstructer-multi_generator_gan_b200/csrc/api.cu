@@ -10,6 +10,7 @@
 #include "elementwise.cuh"
 #include "discriminator.cuh"
 #include "generator.cuh"
+#include "metrics.cuh"
 #include "peer_sync.cuh"
 #include "resample.cuh"
 #include "trunk_fused.cuh"
@@ -409,6 +410,20 @@ int srg_mse(const float* a, const float* b, int64_t n, void* scratch, size_t scr
   if (scratch_bytes < srg_recon_loss_scratch_bytes()) { set_error("mse: scratch too small"); return -5; }
   if (!a || !b || !out1) { set_error("mse: null pointer"); return -6; }
   return launch_mse(a, b, n, reinterpret_cast<double*>(scratch), out1, S(stream));
+}
+size_t srg_image_metrics_scratch_bytes(int N, int H, int W) { return image_metrics_scratch_bytes(N, H, W); }
+int srg_image_metrics(const float* sr, const float* hr, int N, int C, int H, int W, void* scratch, size_t scratch_bytes,
+                      double* psnr_out, double* ssim_out, void* stream) {
+  if (N < 1 || C != 3 || H < 3 || W < 3) {
+    set_error("image_metrics: need N >= 1 images of 3 x H x W with H, W >= 3 (got N=%d C=%d H=%d W=%d)", N, C, H, W);
+    return -100;
+  }
+  if (!sr || !hr || !scratch || !psnr_out || !ssim_out) { set_error("image_metrics: null pointer"); return -6; }
+  if (scratch_bytes < image_metrics_scratch_bytes(N, H, W)) {
+    set_error("image_metrics: scratch too small (%zu < %zu bytes)", scratch_bytes, image_metrics_scratch_bytes(N, H, W));
+    return -5;
+  }
+  return launch_image_metrics(sr, hr, N, H, W, reinterpret_cast<double*>(scratch), psnr_out, ssim_out, S(stream));
 }
 
 }  // extern "C"

@@ -6,6 +6,8 @@
 * ``resume_learning_rates``: the ``continue_training`` protocol (src/train.py:51-59) divides both learning rates by 5.
 * ``ImageEnhancer``: src/models.py:28-41 (Laplacian sharpening + clamp), one fused kernel.
 * ``calculate_psnr``: src/utils.py:141-144 (skimage PSNR with data_range=1 over the whole tensor) on the device.
+* ``calculate_ssim``: src/utils.py:148-151 (skimage SSIM, win_size=3, the 3 x H x W array as one 3-D volume).
+* ``image_metrics``: both per image for a whole batch in one pass, without a host sync (train.compute_score).
 """
 from __future__ import annotations
 
@@ -78,3 +80,41 @@ def calculate_psnr(img1: torch.Tensor, img2: torch.Tensor) -> float:
                     c_void_p(out.data_ptr()), stream_ptr()), "srg_mse")
     mse = float(out.item())
     return float("inf") if mse == 0 else 10.0 * math.log10(1.0 / mse)
+
+
+_METRICS_SCRATCH = {}
+
+
+def image_metrics(sr: torch.Tensor, hr: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per-image ``(psnr, ssim)`` of an N x 3 x H x W batch pair as two float64 CUDA tensors of shape [N], without a host
+    sync (capturable into a CUDA graph once warmed up).  ``psnr[n]`` equals ``calculate_psnr(sr[n], hr[n])`` (+inf for
+    identical images) and ``ssim[n]`` equals ``calculate_ssim(sr[n], hr[n])``; an image's values do not depend on the
+    rest of the batch.  The fp64 scratch of the reduction is cached per device, stream and (N, H, W)."""
+    if sr.shape != hr.shape or sr.dim() != 4:
+        raise RuntimeError(f"image_metrics: two N x 3 x H x W tensors of the same shape, got {tuple(sr.shape)} and {tuple(hr.shape)}")
+    if not sr.is_cuda or not hr.is_cuda or sr.device != hr.device:
+        raise RuntimeError("image_metrics: CUDA tensors on one device only (libsrgan_b200 has no CPU path)")
+    a, b = sr.contiguous().float(), hr.contiguous().float()
+    N, C, H, W = a.shape
+    L = _lib.lib()
+    key = (a.device, torch.cuda.current_stream(a.device).cuda_stream, N, H, W)    # stream-ordered reuse only
+    scratch = _METRICS_SCRATCH.get(key)
+    if scratch is None:
+        scratch = torch.empty(max(int(L.srg_image_metrics_scratch_bytes(N, H, W)), 8), dtype=torch.uint8, device=a.device)
+        _METRICS_SCRATCH[key] = scratch
+    out = torch.empty(2, N, dtype=torch.float64, device=a.device)
+    check(L.srg_image_metrics(c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), N, C, H, W, c_void_p(scratch.data_ptr()),
+                              scratch.numel(), c_void_p(out[0].data_ptr()), c_void_p(out[1].data_ptr()), stream_ptr()),
+          "srg_image_metrics")
+    return out[0], out[1]
+
+
+def calculate_ssim(img1: torch.Tensor, img2: torch.Tensor) -> float:
+    """skimage.metrics.structural_similarity(img1, img2, win_size=3, multichannel=True) as called at src/utils.py:148-151
+    on one 3 x H x W image pair: under scikit-image 0.25 ``multichannel`` is swallowed by ``**kwargs``, so the array is
+    one 3-D volume (3x3x3 window over channels, rows and columns; data_range 1)."""
+    if img1.shape != img2.shape or not img1.is_cuda:
+        raise RuntimeError("calculate_ssim: two CUDA tensors of the same shape")
+    if img1.dim() != 3:
+        raise RuntimeError(f"calculate_ssim: one 3 x H x W image pair, got {tuple(img1.shape)}")
+    return float(image_metrics(img1[None], img2[None])[1].item())

@@ -152,6 +152,36 @@ def train_one_epoch(generator, train_loader, g_optimizer, vgg_extractor, g_crite
     return avg
 
 
+def compute_score(generator, val_loader, device, num_batches: int = 30) -> Tuple[float, float]:
+    """Validation metric of src/train.py:263-294 (called every epoch, :117): the generator in eval mode over the first
+    ``num_batches`` ``(hr, lr)`` batches of ``val_loader``; returns ``(avg_psnr, avg_ssim)`` averaged over images, for this
+    rank only (as upstream).  The reference scores every image on the host with calculate_psnr / calculate_ssim
+    (src/utils.py:141-151); here both come from one ``image_metrics`` pass per batch, summed on the device and read back
+    once.  This signature is the package's own; the generator's train / eval mode is restored and its parameters and
+    BatchNorm buffers are left untouched."""
+    import itertools
+    from .evaluation import image_metrics
+    was_training = generator.training
+    generator.eval()
+    sums = torch.zeros(2, dtype=torch.float64, device=device)
+    images = 0
+    try:
+        with torch.no_grad():
+            for hr_imgs, lr_imgs in itertools.islice(val_loader, num_batches):     # islice pulls no extra batch
+                hr_imgs = hr_imgs.to(device, non_blocking=True)
+                lr_imgs = lr_imgs.to(device, non_blocking=True)
+                psnr, ssim = image_metrics(generator(lr_imgs), hr_imgs)
+                sums[0] += psnr.sum()
+                sums[1] += ssim.sum()
+                images += hr_imgs.shape[0]
+    finally:
+        generator.train(was_training)
+    if images == 0:
+        raise ValueError("compute_score: the validation loader yielded no batch")
+    avg_psnr, avg_ssim = (sums / images).tolist()          # the only device->host copy
+    return avg_psnr, avg_ssim
+
+
 def setup_training(rank: int, world_size: int, num_epochs: int, continue_training: bool = False, prefix: str = "Training",
                    results_dir: str = "results", num_generators: int = 1, init_process_group: bool = True,
                    capturable: bool = True):
