@@ -65,6 +65,19 @@ int srg_generator_forward(srg_generator_t* g, const float* lr_nchw, float* sr_nc
 /* replaces autograd through SRResNet inside g_loss.backward() (src/train.py:195): d(loss)/d(sr) in, every
  * parameter gradient out (written to the bound flat `grads`; biases feeding a training-mode BatchNorm get 0). */
 int srg_generator_backward(srg_generator_t* g, const float* dsr_nchw, void* stream);
+/* a fixed generator inside a larger differentiable pipeline (SRResNet in eval() fed an input that requires grad, whose
+ * BatchNorm layers use their running statistics as in src/models.py:16,19 under model.eval()): eval-mode (running-
+ * statistics) BatchNorm on a training-bound workspace, keeping what the backward needs; running statistics are read,
+ * never updated and never exchanged across ranks.  The output differs from the eval-bound srg_generator_forward in bf16
+ * rounding only (BatchNorm is a separate pass over the stored conv output instead of the conv epilogue). */
+int srg_generator_forward_frozen(srg_generator_t* g, const float* lr_nchw, float* sr_nchw, void* stream);
+/* backward of the last forward (training or frozen) through SRResNet (src/models.py:53-87), as autograd computes it for
+ * the reference's nn.Module.  param_grads == 0: no parameter gradient is computed or written (the flat `grads` buffer
+ * is not touched); dlr_nchw (may be NULL) receives d(loss)/d(lr) as fp32 N x 3 x H x W.  After a frozen forward the
+ * biases of the trunk convs get their real gradient (a BatchNorm with fixed statistics passes it on).
+ * srg_generator_backward(g, dsr, stream) == srg_generator_backward_ex(g, dsr, 1, NULL, stream).  Fails before any CUDA
+ * call on a null engine or dsr_nchw, an unbound or eval-bound workspace, or param_grads == 0 with dlr_nchw == NULL. */
+int srg_generator_backward_ex(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream);
 
 /* named intermediates inside the workspace (per-layer parity checks): dtype 0 = bf16 NHWC, dims = N,H,W,C */
 int srg_generator_num_tensors(const srg_generator_t* g);

@@ -130,6 +130,14 @@ int srg_generator_forward(srg_generator_t* g, const float* lr_nchw, float* sr_nc
 int srg_generator_backward(srg_generator_t* g, const float* dsr_nchw, void* stream) {
   return generator_backward(G(g), dsr_nchw, S(stream));
 }
+int srg_generator_forward_frozen(srg_generator_t* g, const float* lr_nchw, float* sr_nchw, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_forward_frozen: null engine"); return -1; }
+  return generator_forward_frozen(G(g), lr_nchw, sr_nchw, S(stream));
+}
+int srg_generator_backward_ex(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_backward_ex: null engine"); return -1; }
+  return generator_backward_ex(G(g), dsr_nchw, param_grads, dlr_nchw, S(stream));
+}
 int srg_generator_num_tensors(const srg_generator_t* g) { return int(G(g)->tensors.size()); }
 int srg_generator_tensor_info(const srg_generator_t* g, int i, char* name, int name_cap, int64_t* byte_offset, int* dims4,
                               int* dtype) {

@@ -162,6 +162,16 @@ __device__ __forceinline__ void finalize_channels(const ReduceFinalize& f, int c
     f.out0[c] = float(sc);
     f.out1[c] = float(-sc * inv * dg / f.count);
     f.out2[c] = float(-sc * db / f.count + sc * inv * mean * dg / f.count);
+  } else if (f.mode == RF_BN_BWD_FROZEN) {
+    // y_hat = (y - running_mean) * inv does not depend on the batch: dy = gamma * inv * dz
+    const double rm = f.save_mean[c], inv = f.save_inv[c];
+    const double sc = double(f.gamma[c]) * inv;
+    if (f.dgamma) f.dgamma[c] = float(inv * (s2 - rm * s1));
+    if (f.dbeta) f.dbeta[c] = float(s1);
+    if (f.dbias) f.dbias[c] = float(sc * s1);
+    f.out0[c] = float(sc);
+    f.out1[c] = 0.f;
+    f.out2[c] = 0.f;
   } else {
     f.out0[c] = float(s1);                          // RF_SUM: bias gradient
   }
@@ -417,6 +427,29 @@ int launch_bn_eval_coeffs_all(const float* master, const float* buffers, const v
   if (n_bn <= 0) return 0;
   bn_eval_coeffs_all_kernel<<<n_bn, 64, 0, st>>>(master, buffers, reinterpret_cast<const int4*>(tab), eps, coef);
   SRG_LAUNCH_CHECK("bn_eval_coeffs_all");
+  return 0;
+}
+
+// frozen BatchNorm (eval-mode statistics on the training workspace): the convs keep their own bias, so the shift does not
+// absorb it; running_mean and inv go to the save_mean / save_inv slots the backward reads
+__global__ void bn_frozen_coeffs_all_kernel(const float* __restrict__ master, const float* __restrict__ buffers,
+                                            const int4* __restrict__ tab, float eps, float* __restrict__ coef) {
+  const int l = blockIdx.x, c = threadIdx.x;
+  const int4 t = tab[l];                      // {gamma, beta, running_mean, (conv bias: unused)} offsets
+  const float* rm = buffers + t.z;
+  const float inv = 1.f / sqrtf(rm[64 + c] + eps);
+  const float sc = master[t.x + c] * inv;
+  float* o = coef + size_t(l) * 256;
+  o[c] = sc;
+  o[64 + c] = master[t.y + c] - rm[c] * sc;
+  o[128 + c] = rm[c];
+  o[192 + c] = inv;
+}
+int launch_bn_frozen_coeffs_all(const float* master, const float* buffers, const void* tab, int n_bn, float eps, float* coef,
+                                cudaStream_t st) {
+  if (n_bn <= 0) return 0;
+  bn_frozen_coeffs_all_kernel<<<n_bn, 64, 0, st>>>(master, buffers, reinterpret_cast<const int4*>(tab), eps, coef);
+  SRG_LAUNCH_CHECK("bn_frozen_coeffs_all");
   return 0;
 }
 

@@ -14,7 +14,10 @@ int reduce_blocks(int64_t pixels);
 int l2_hints();   // SRG_L2_HINTS: 0 none, 1 BatchNorm chain, 2 + convolution stores
 int launch_chan_reduce(const void* a, const void* b, int64_t pixels, float* partials, cudaStream_t st);
 // Fused variant: reduction + fixed-order partial sum + per-channel finalize in ONE launch (last block done).
-enum ReduceFinalizeMode : int { RF_BN_FWD = 0, RF_BN_BWD = 1, RF_SUM = 2 };
+// RF_BN_BWD_FROZEN: backward of an eval-mode (running-statistics) BatchNorm; save_mean / save_inv hold running_mean and
+// 1 / sqrt(running_var + eps), the coefficients are A = gamma * inv, B = C = 0 and `dbias` (optional) receives the
+// gradient of the preceding conv's bias, A * sum(dz)
+enum ReduceFinalizeMode : int { RF_BN_FWD = 0, RF_BN_BWD = 1, RF_SUM = 2, RF_BN_BWD_FROZEN = 3 };
 struct ReduceFinalize {
   int mode;
   double count;                 // elements per channel
@@ -31,6 +34,7 @@ struct ReduceFinalize {
   float* out1;                  // FWD: shift | BWD: coefB
   float* out2;                  // FWD: save_mean | BWD: coefC
   float* out3;                  // FWD: save_inv
+  float* dbias;                 // RF_BN_BWD_FROZEN: preceding conv's bias gradient (optional)
 };
 // Two-launch form used on the hot path: any producer of [rows][128] fp32 partials (launch_chan_reduce, or the conv
 // epilogue's fused statistics) followed by ONE 1024-thread block that sums them in a fixed order and finalizes.
@@ -58,6 +62,11 @@ int launch_bn_eval_coeffs(const float* gamma, const float* beta, const float* ru
 // conv bias} float offsets into master / buffers; coef[l][256] = {scale[64], shift[64] with the conv bias folded in, ...}
 int launch_bn_eval_coeffs_all(const float* master, const float* buffers, const void* tab, int n_bn, float eps, float* coef,
                               cudaStream_t st);
+// eval-mode BatchNorm on the training path (the conv adds its own bias): coef[l][256] = {scale = gamma * inv,
+// shift = beta - running_mean * scale, running_mean, inv = 1 / sqrt(running_var + eps)}; tab as launch_bn_eval_coeffs_all
+// (the conv-bias column is not read)
+int launch_bn_frozen_coeffs_all(const float* master, const float* buffers, const void* tab, int n_bn, float eps, float* coef,
+                                cudaStream_t st);
 // out = act(scale*y + shift) (+ skip);  relu: 0/1
 int launch_bn_apply(const void* y, const float* scale, const float* shift, const void* skip, int relu, void* out,
                     int64_t pixels, cudaStream_t st);

@@ -44,6 +44,8 @@ struct Layout {
   size_t g[4];                           // P-sized gradient buffers
   std::vector<size_t> dup;               // gradient of each upsample stage output
   size_t Ud;                             // unfolded d(SR)
+  size_t c1d = 0;                        // packed conv1 data-gradient filter (input-gradient backward only)
+  size_t frozen_tab = 0;                 // int4 BatchNorm offset rows of the frozen (running-statistics) forward
   // debug (keep_grads): every inter-layer gradient in its own buffer instead of the 3 rotating ones
   std::vector<size_t> kd_y2, kd_p1, kd_y1, kd_in;
   size_t kd_last, kd_c1;
@@ -51,6 +53,7 @@ struct Layout {
 };
 
 size_t t64(int64_t pixels) { return size_t(pixels) * 128; }
+constexpr int64_t kConv1DgradElems = 9 * 32 * 64;   // pack_conv1_dgrad: [9 row taps][32][64] bf16
 
 int64_t wgrad_max_floats(int n_up) {
   // splits * n_blocks * n_pairs * 8192, with splits = SMs / n_blocks  => <= 148 * n_pairs * 8192
@@ -124,6 +127,8 @@ Layout make_layout(const GeneratorEngine& e, bool training) {
     for (int j = 0; j < e.n_up; ++j) L.dup[j] = c.take(t64(P << (2 * (j + 1))));
     const int64_t Hs = int64_t(e.H) << e.n_up, Ws = int64_t(e.W) << e.n_up;
     L.Ud = c.take(size_t(e.N) * (Hs + 1) * Ws * 128);
+    L.c1d = c.take(size_t(kConv1DgradElems) * 2);
+    L.frozen_tab = c.take(size_t(2 * e.n_res + 1) * 16);
   }
   L.total = c.off;
   return L;
@@ -209,6 +214,13 @@ void pack_conv3_fwd(std::vector<int>& idx, int64_t base) {
     for (int n = 0; n < 32; ++n)
       for (int ci = 0; ci < 64; ++ci) idx.push_back(n < 27 ? widx(base, 64, 9, n % 3, ci, r, n / 3) : -1);
 }
+void pack_conv1_dgrad(std::vector<int>& idx, int64_t base) {
+  // fold9 form of conv1's data gradient (a 9x9 64 -> 3 conv over d(pre-LeakyReLU) with the transposed, flipped filter):
+  // [r = kh'][n = s*3 + c (32)][co] = W1[co][c][8-r][8-s]
+  for (int r = 0; r < 9; ++r)
+    for (int n = 0; n < 32; ++n)
+      for (int co = 0; co < 64; ++co) idx.push_back(n < 27 ? widx(base, 3, 9, co, n % 3, 8 - r, 8 - n / 3) : -1);
+}
 void pack_conv3_dgrad(std::vector<int>& idx, int64_t base) {
   // [r][ci][(dr, s, co)] = W3[co][ci][8-2r-dr][8-s]
   for (int r = 0; r < 5; ++r)
@@ -238,7 +250,10 @@ struct EngineImpl : GeneratorEngine {
   PackOffsets po;
   Layout L;
   // host copies of the constant index maps; uploaded at the first bind (create() needs no device)
-  std::vector<int> h_pack_idx, h_bias_idx, h_wg_c3x3, h_wg_up, h_wg_conv1, h_wg_conv3;
+  std::vector<int> h_pack_idx, h_bias_idx, h_wg_c3x3, h_wg_up, h_wg_conv1, h_wg_conv3, h_conv1_dgrad;
+  int* d_conv1_dgrad_idx = nullptr;
+  bool last_frozen = false;     // the last forward on the training workspace used running BatchNorm statistics
+  ~EngineImpl() override { cudaFree(d_conv1_dgrad_idx); }
   // fused trunk (trunk_fused.cu): set at bind when the workspace layout is uniformly strided and the geometry fits
   bool trunk_ok = false;
   int trunk_act_buffers = 0, trunk_grad_buffers = 0;
@@ -417,7 +432,7 @@ void fill_trunk_gen(EngineImpl* e, TrunkGen& t) {
 }
 
 // one launch for the trunks of `n` engines of identical geometry / configuration (n = 1: the nn.Module path)
-int run_trunk_multi(EngineImpl* const* es, int n, int bwd, int update_running, cudaStream_t st) {
+int run_trunk_multi(EngineImpl* const* es, int n, int bwd, int update_running, cudaStream_t st, bool param_grads = true) {
   EngineImpl* e = es[0];
   const Layout& L = e->L;
   const int64_t P = int64_t(e->N) * e->H * e->W;
@@ -438,13 +453,16 @@ int run_trunk_multi(EngineImpl* const* es, int n, int bwd, int update_running, c
       return -65;
     }
     fill_trunk_gen(o, a.gen[i]);
+    if (!param_grads) a.gen[i].grads = nullptr;
     o->prof_layers = a.n_layers;
   }
   e->launches += 1;
   ProfScope ps(e, st);
   return launch_trunk(a, st);
 }
-int run_trunk(EngineImpl* e, int bwd, int update_running, cudaStream_t st) { return run_trunk_multi(&e, 1, bwd, update_running, st); }
+int run_trunk(EngineImpl* e, int bwd, int update_running, cudaStream_t st, bool param_grads = true) {
+  return run_trunk_multi(&e, 1, bwd, update_running, st, param_grads);
+}
 
 // ------------------------------------------------------------------ grouped per-layer trunk
 // Large geometries (several tiles per SM, where the fused trunk kernel loses to per-layer launches): the SAME trunk layer of
@@ -918,6 +936,7 @@ GeneratorEngine* generator_create(int N, int H, int W, int n_res, int n_up) {
   mc3 = invert(mc3, size_t(1) * 3 * 8192);
   e->h_pack_idx.swap(idx); e->h_bias_idx.swap(bidx);
   e->h_wg_c3x3.swap(m33); e->h_wg_up.swap(mup); e->h_wg_conv1.swap(mc1); e->h_wg_conv3.swap(mc3);
+  pack_conv1_dgrad(e->h_conv1_dgrad, poff(*e, "conv1.weight"));
   e->workspace_bytes_train = make_layout(*e, true).total;
   e->workspace_bytes_eval = make_layout(*e, false).total;
   return e;
@@ -937,6 +956,7 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
     e->d_wg_idx_up = upload(e->h_wg_up);
     e->d_wg_idx_conv1 = upload(e->h_wg_conv1);
     e->d_wg_idx_conv3 = upload(e->h_wg_conv3);
+    e->d_conv1_dgrad_idx = upload(e->h_conv1_dgrad);
     {
       std::vector<long long> off;
       char wn[96];
@@ -952,7 +972,8 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
         return -23;
       }
     }
-    if (!e->d_pack_idx || !e->d_bias_idx || !e->d_wg_idx_c3x3 || !e->d_wg_idx_up || !e->d_wg_idx_conv1 || !e->d_wg_idx_conv3) {
+    if (!e->d_pack_idx || !e->d_bias_idx || !e->d_wg_idx_c3x3 || !e->d_wg_idx_up || !e->d_wg_idx_conv1 || !e->d_wg_idx_conv3 ||
+        !e->d_conv1_dgrad_idx) {
       set_error("generator_bind: device allocation of index maps failed: %s", cudaGetErrorString(cudaGetLastError()));
       return -29;
     }
@@ -962,8 +983,10 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
   e->L = make_layout(*e, training != 0);
   if (cudaMemset(e->ws + e->L.ticket, 0, 256) != cudaSuccess) { set_error("generator_bind: memset failed"); return -29; }
   e->trunk_ok = false;
-  if (!training && e->n_res > 0) {
-    // eval mode: offsets of every BatchNorm's parameters / statistics / preceding conv bias for launch_bn_eval_coeffs_all
+  e->last_frozen = false;
+  if (e->n_res > 0) {
+    // offsets of every BatchNorm's parameters / statistics / preceding conv bias: launch_bn_eval_coeffs_all (eval
+    // workspace) or launch_bn_frozen_coeffs_all (training workspace)
     std::vector<int> tab;
     char nm[96];
     for (int b = 0; b < e->n_res; ++b)
@@ -973,7 +996,8 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
         snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.running_mean", b, k); tab.push_back(int(boff(*e, nm)));
         snprintf(nm, sizeof(nm), "residual_blocks.%d.conv%d.bias", b, k); tab.push_back(int(poff(*e, nm)));
       }
-    if (cudaMemcpy(e->ws + e->L.trunk_tab, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice) != cudaSuccess) {
+    const size_t tab_off = training ? e->L.frozen_tab : e->L.trunk_tab;
+    if (cudaMemcpy(e->ws + tab_off, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice) != cudaSuccess) {
       set_error("generator_bind: upload of the BatchNorm offset table failed");
       return -29;
     }
@@ -1040,11 +1064,15 @@ int generator_forward(GeneratorEngine* g, const float* lr, float* sr, int traini
   return generator_forward_phases(g, lr, sr, training, update_running, kPhaseAll, st);
 }
 
-int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int training, int update_running, int phases,
-                             cudaStream_t st) {
-  EngineImpl* e = static_cast<EngineImpl*>(g);
+namespace {
+// frozen: eval-mode BatchNorm (running statistics, never updated or exchanged) on the training workspace, every
+// activation the backward reads kept; per-layer trunk launches only
+int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int update_running, int phases, bool frozen,
+                 cudaStream_t st) {
   if (!e->ws) { set_error("generator_forward: not bound"); return -23; }
   if (training && !e->ws_training) { set_error("generator_forward: bound workspace is eval-sized"); return -24; }
+  if (training) e->last_frozen = frozen;
+  if (frozen) update_running = 0;
   const Layout& L = e->L;
   const PackOffsets& po = e->po;
   uint8_t* ws = e->ws;
@@ -1064,6 +1092,11 @@ int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int
     // eval: every BatchNorm's folded coefficients in one launch, two kernels ahead of the first conv that reads them
     RC(launch_bn_eval_coeffs_all(e->master, e->bn_buffers, ws + L.trunk_tab, 2 * e->n_res, kBnEps,
                                  reinterpret_cast<float*>(ws + L.bncoef), st));
+    e->launches += 1;
+  }
+  if (frozen && e->n_res > 0) {
+    RC(launch_bn_frozen_coeffs_all(e->master, e->bn_buffers, ws + L.frozen_tab, 2 * e->n_res, kBnEps,
+                                   reinterpret_cast<float*>(ws + L.bncoef), st));
     e->launches += 1;
   }
   // conv1: 9x9, 3->64, LeakyReLU(0.2)  (src/models.py:56-57,81)
@@ -1134,6 +1167,10 @@ int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int
   // training-mode BatchNorm (+ReLU / +skip) behind a conv whose epilogue left the per-CTA statistics in `partials`
   auto bn_train_apply = [&](int b, int k, const void* y, const void* skip, int relu, void* out) -> int {
     float* coef = reinterpret_cast<float*>(ws + L.bncoef) + size_t(2 * b + k) * 256;
+    if (frozen) {
+      e->launches += 1;
+      return launch_bn_apply(y, coef, coef + 64, skip, relu, out, P, st);
+    }
     if (e->fin_fused && !e->allreduce && !e->peer) {
       // single GPU: the finalize runs inside the apply pass (every CTA re-reduces the partial rows): one launch, not two
       snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.weight", b, k + 1);
@@ -1155,7 +1192,8 @@ int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int
   };
 
   const void* x = ws + L.out1;
-  const bool fused = training && use_trunk_fused(*e);
+  const bool fused = training && !frozen && use_trunk_fused(*e);
+  const bool stats = training && !frozen;       // batch statistics accumulated by the trunk convs' epilogues
   e->prof_layers = 1;
   if (fused && (phases & kPhaseTrunk)) RC(run_trunk(e, 0, update_running, st));
   for (int b = 0; b < e->n_res && !fused && layers_here; ++b) {
@@ -1169,10 +1207,10 @@ int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int
       continue;
     }
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv1.bias", b);
-    RC(conv3x3(x, po.rb_f[0][b], e->master + poff(*e, nm), nullptr, ws + L.y1[b], training != 0));
+    RC(conv3x3(x, po.rb_f[0][b], e->master + poff(*e, nm), nullptr, ws + L.y1[b], stats));
     RC(bn_train_apply(b, 0, ws + L.y1[b], nullptr, 1, ws + L.z1[b]));
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv2.bias", b);
-    RC(conv3x3(ws + L.z1[b], po.rb_f[1][b], e->master + poff(*e, nm), nullptr, ws + L.y2[b], training != 0));
+    RC(conv3x3(ws + L.z1[b], po.rb_f[1][b], e->master + poff(*e, nm), nullptr, ws + L.y2[b], stats));
     RC(bn_train_apply(b, 1, ws + L.y2[b], x, 0, ws + L.out[b]));
     x = ws + L.out[b];
   }
@@ -1208,15 +1246,32 @@ int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int
   }
   return 0;
 }
+}  // namespace
 
-// ------------------------------------------------------------------ backward
-int generator_backward(GeneratorEngine* g, const float* dsr, cudaStream_t st) {
-  return generator_backward_phases(g, dsr, kPhaseAll, st);
+int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int training, int update_running, int phases,
+                             cudaStream_t st) {
+  return forward_impl(static_cast<EngineImpl*>(g), lr, sr, training, update_running, phases, false, st);
 }
 
-int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, cudaStream_t st) {
+int generator_forward_frozen(GeneratorEngine* g, const float* lr, float* sr, cudaStream_t st) {
   EngineImpl* e = static_cast<EngineImpl*>(g);
+  if (lr == nullptr || sr == nullptr) { set_error("generator_forward_frozen: null image pointer"); return -22; }
+  if (!e->ws || !e->ws_training) { set_error("generator_forward_frozen: needs a training-sized bound workspace"); return -25; }
+  return forward_impl(e, lr, sr, 1, 0, kPhaseAll, true, st);
+}
+
+// ------------------------------------------------------------------ backward
+namespace {
+// param_grads == false: only the data-gradient chain runs (no gradient memset, weight gradients, bias sums or BatchNorm
+// parameter gradients; the flat gradient buffer is not touched).  dlr != null: conv1's data gradient, fp32 NCHW.
+int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads, float* dlr, cudaStream_t st) {
   if (!e->ws || !e->ws_training) { set_error("generator_backward: needs a training-sized bound workspace"); return -25; }
+  const bool frozen = e->last_frozen;
+  if (frozen && phases != kPhaseAll) {
+    set_error("generator_backward_phases: the last forward used running BatchNorm statistics; split execution needs a training forward");
+    return -31;
+  }
+  const bool pg = param_grads;
   const Layout& L = e->L;
   const PackOffsets& po = e->po;
   uint8_t* ws = e->ws;
@@ -1230,7 +1285,13 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
   char nm[96];
 
   const bool pre = (phases & kPhasePre) != 0, mid = (phases & kPhaseTrunk) != 0, post = (phases & kPhasePost) != 0;
-  if (pre && cudaMemsetAsync(e->grads, 0, size_t(e->param_elems) * 4, st) != cudaSuccess) { set_error("memset grads failed"); return -26; }
+  if (dlr != nullptr) {
+    // conv1's data-gradient filter, gathered from the fp32 master only when an input gradient is requested (the conv that
+    // reads it runs at the end of this pass, far behind this launch)
+    RC(launch_pack_bf16(e->master, e->d_conv1_dgrad_idx, ws + L.c1d, kConv1DgradElems, st));
+    e->launches += 1;
+  }
+  if (pre && pg && cudaMemsetAsync(e->grads, 0, size_t(e->param_elems) * 4, st) != cudaSuccess) { set_error("memset grads failed"); return -26; }
 
   auto wgrad = [&](InView xv, int in_H, int in_W, bool pairs, int gh, int gw, const void* dy_base, int n_blocks,
                    bool dy_ps, const int* idx, const std::string& wname) -> int {
@@ -1312,10 +1373,11 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
   if (pre) {
   // ---- conv3 (9x9, 64->3): unfold d(SR) once; it feeds the bias sum, wgrad and dgrad
   RC(launch_unfold9(dsr, N, Hs, Ws, 1.f, ws + L.Ud, st));
-  RC(launch_nchw_chan_sum(dsr, N, 3, int64_t(Hs) * Ws, reinterpret_cast<double*>(ws + L.loss_scratch),
-                          e->grads + poff(*e, "conv3.bias"), 1.f, st));
-  e->launches += 3;
-  {
+  e->launches += 1;
+  if (pg) {
+    RC(launch_nchw_chan_sum(dsr, N, 3, int64_t(Hs) * Ws, reinterpret_cast<double*>(ws + L.loss_scratch),
+                            e->grads + poff(*e, "conv3.bias"), 1.f, st));
+    e->launches += 2;
     InView uv = plain_view(ws + L.Ud, Hs + 1, Ws);
     RC(wgrad(uv, Hs + 1, Ws, true, Hs, Ws, conv3_in, 1, false, e->d_wg_idx_conv3, "conv3.weight"));
   }
@@ -1334,18 +1396,20 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
   for (int j = S - 1; j >= 0; --j) {
     const int Hj = H << j, Wj = W << j;
     const void* in_j = j > 0 ? ws + L.up[j - 1] : ws + L.trunk;
-    snprintf(nm, sizeof(nm), "upsample.%d.bias", 3 * j);
-    RC(launch_ps_bias_grad(ws + L.dup[j], N, Hj * 2, Wj * 2, reinterpret_cast<float*>(ws + L.ps_scratch),
-                           e->grads + poff(*e, nm), st));
-    e->launches += 2;
-    snprintf(nm, sizeof(nm), "upsample.%d.weight", 3 * j);
-    RC(wgrad(plain_view(in_j, Hj, Wj), Hj, Wj, false, Hj, Wj, ws + L.dup[j], 4, true, e->d_wg_idx_up, nm));
+    if (pg) {
+      snprintf(nm, sizeof(nm), "upsample.%d.bias", 3 * j);
+      RC(launch_ps_bias_grad(ws + L.dup[j], N, Hj * 2, Wj * 2, reinterpret_cast<float*>(ws + L.ps_scratch),
+                             e->grads + poff(*e, nm), st));
+      e->launches += 2;
+      snprintf(nm, sizeof(nm), "upsample.%d.weight", 3 * j);
+      RC(wgrad(plain_view(in_j, Hj, Wj), Hj, Wj, false, Hj, Wj, ws + L.dup[j], 4, true, e->d_wg_idx_up, nm));
+    }
     RC(dgrad3x3(ws + L.dup[j], Hj, Wj, true, po.up_d[j], nullptr, j > 0 ? in_j : nullptr, j > 0 ? ws + L.dup[j - 1] : d_trunk, nullptr));
   }
   }
   // ---- conv2 (trunk = conv2(x_last) + out1)
   const void* x_last = e->n_res > 0 ? ws + L.out[e->n_res - 1] : ws + L.out1;
-  if (pre) RC(bias_grad(d_trunk, P, "conv2.bias"));
+  if (pre && pg) RC(bias_grad(d_trunk, P, "conv2.bias"));
   // The 2*n_res + 1 trunk weight gradients run as ONE batched launch at the end of backward (wgrad3_batched_kernel):
   // x of layer l = 2*block + conv sits at out1 + l * 2 * slot (out[b-1] | z1[b] are two slots apart, conv2 reads out[last]),
   // dy of layer l at dyall + l * slot.  SRG_WGRAD_BATCHED=0 (or a non-uniform layout) keeps one launch per layer.
@@ -1362,20 +1426,20 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     probe.N = N; probe.H = H; probe.W = W; probe.n_layers = 2 * e->n_res + 1;
     if (wgrad3_batched_partials_floats(probe) > L.wgb_floats) batched = false;
   }
-  if (!batched && pre) RC(wgrad(plain_view(x_last, H, W), H, W, false, H, W, d_trunk, 1, false, e->d_wg_idx_c3x3, "conv2.weight"));
+  if (!batched && pre && pg) RC(wgrad(plain_view(x_last, H, W), H, W, false, H, W, d_trunk, 1, false, e->d_wg_idx_c3x3, "conv2.weight"));
   const bool keep = e->keep_grads;
   void* dout = keep ? ws + L.kd_last : ws + L.g[0];
   void* dother = ws + L.g[1];
   void* dmid = ws + L.g[2];
   // the whole dgrad chain of the trunk (conv2, then every block's BatchNorm / ReLU / conv backward) in one launch
-  const bool fused = batched && use_trunk_fused(*e);
+  const bool fused = batched && !frozen && use_trunk_fused(*e);
   const bool layers_here = !fused && phases == kPhaseAll;
   if (phases != kPhaseAll && !fused && !(batched && use_trunk_grouped(*e))) {
     set_error("generator_backward_phases: split execution needs the fused or the grouped per-layer trunk path");
     return -31;
   }
   if (fused) {
-    if (mid) RC(run_trunk(e, 1, 0, st));
+    if (mid) RC(run_trunk(e, 1, 0, st, pg));
     dout = ws + L.g[0] + L.slot * size_t(e->trunk_dout_idx);
   } else if (!layers_here) {
     // split execution on the per-layer path: generators_trunk() ran (or will run) the dgrad chain as grouped launches
@@ -1393,11 +1457,31 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     const int64_t bo = poff(*e, nm);
     // sum dz and sum dz*y: either accumulated by the dgrad kernel that produced dz (fuse_bwd_stats) or by one pass here
     int rows = bwd_stats_rows;
+    if (frozen) {
+      // running statistics: no cross-rank exchange, dy = gamma * inv * dz, and the preceding conv's bias gets A * sum(dz)
+      if (!e->fuse_bwd_stats) {
+        RC(launch_chan_reduce(dz, y, P, partials, st));
+        rows = reduce_blocks(P);
+        e->launches += 1;
+      }
+      ReduceFinalize f; memset(&f, 0, sizeof(f));
+      f.mode = RF_BN_BWD_FROZEN; f.count = double(P); f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
+      if (pg) {
+        snprintf(nm, sizeof(nm), "residual_blocks.%d.conv%d.bias", b, k + 1);
+        f.dgamma = e->grads + go; f.dbeta = e->grads + bo; f.dbias = e->grads + poff(*e, nm);
+      }
+      f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
+      RC(launch_partials_finalize(partials, rows, f, st));
+      e->launches += 2;
+      return launch_bn_bwd_apply(dz, y, bwd, bwd + 64, bwd + 128, dy, P, st);
+    }
+    float* dgamma = pg ? e->grads + go : nullptr;
+    float* dbeta = pg ? e->grads + bo : nullptr;
     if (!e->fuse_bwd_stats && !e->allreduce && !e->peer && e->reduce_final) {
       // single GPU: the reduction's last block finalizes (atomic ticket): no finalize launch on the backward chain
       ReduceFinalize f; memset(&f, 0, sizeof(f));
       f.mode = RF_BN_BWD; f.count = double(P); f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
-      f.dgamma = e->grads + go; f.dbeta = e->grads + bo; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
+      f.dgamma = dgamma; f.dbeta = dbeta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
       RC(launch_chan_reduce_final(dz, y, P, partials, reinterpret_cast<unsigned int*>(ws + L.ticket), f, st));
       e->launches += 2;
       return launch_bn_bwd_apply(dz, y, bwd, bwd + 64, bwd + 128, dy, P, st);
@@ -1410,7 +1494,7 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     if (!e->allreduce || e->peer) {
       ReduceFinalize f; memset(&f, 0, sizeof(f));
       f.mode = RF_BN_BWD; f.count = double(P) * e->world; f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
-      f.dgamma = e->grads + go; f.dbeta = e->grads + bo; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
+      f.dgamma = dgamma; f.dbeta = dbeta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
       if (!e->peer && e->fin_fused) {
         e->launches += 1;
         return launch_bn_bwd_apply_fin(dz, y, partials, rows, f, dy, P, st);
@@ -1421,7 +1505,7 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     } else {
       RC(launch_partials_sums(partials, rows, sums, st));
       RC(e->allreduce(e->allreduce_ctx, sums, 128, st));
-      RC(launch_bn_bwd_finalize(sums, double(P) * e->world, e->master + go, coef + 128, coef + 192, e->grads + go, e->grads + bo,
+      RC(launch_bn_bwd_finalize(sums, double(P) * e->world, e->master + go, coef + 128, coef + 192, dgamma, dbeta,
                                 bwd, bwd + 64, bwd + 128, 1.f / float(e->world), st));
       e->launches += 4;
     }
@@ -1436,12 +1520,12 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     // out = bn2(y2) + x
     RC(bn_backward(b, 1, dout, ws + L.y2[b], d_y2));
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv2.weight", b);
-    if (!batched) RC(wgrad(plain_view(ws + L.z1[b], H, W), H, W, false, H, W, d_y2, 1, false, e->d_wg_idx_c3x3, nm));
+    if (!batched && pg) RC(wgrad(plain_view(ws + L.z1[b], H, W), H, W, false, H, W, d_y2, 1, false, e->d_wg_idx_c3x3, nm));
     RC(dgrad3x3(d_y2, H, W, false, po.rb_d[1][b], nullptr, ws + L.z1[b], d_p1, ws + L.y1[b]));   // ReLU backward via mask
     // z1 = relu(bn1(y1))
     RC(bn_backward(b, 0, d_p1, ws + L.y1[b], d_y1));
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv1.weight", b);
-    if (!batched) RC(wgrad(plain_view(x_in, H, W), H, W, false, H, W, d_y1, 1, false, e->d_wg_idx_c3x3, nm));
+    if (!batched && pg) RC(wgrad(plain_view(x_in, H, W), H, W, false, H, W, d_y1, 1, false, e->d_wg_idx_c3x3, nm));
     RC(dgrad3x3(d_y1, H, W, false, po.rb_d[0][b], dout, nullptr, d_in, b > 0 ? ws + L.y2[b - 1] : nullptr));   // + skip gradient
     if (keep) { dout = d_in; } else { void* t = dout; dout = dother; dother = t; }
   }
@@ -1450,6 +1534,19 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
   if (keep) dmid = ws + L.kd_c1;
   RC(launch_lrelu_bwd_add2(dout, d_trunk, ws + L.out1, kSlope, dmid, P, st));
   e->launches += 1;
+  if (dlr != nullptr) {
+    // d(lr): 9x9 64 -> 3 conv of d(pre-LeakyReLU) with the flipped filter, through the fold9 path of conv3's forward
+    ConvGemmArgs a; memset(&a, 0, sizeof(a));
+    a.N = N; a.H = H; a.W = W; a.TH = 4; a.TW = 32;
+    a.n_strips = 1; a.n_taps = 9; a.strip_rows = 12; a.strip_dh = -4; a.strip_dw[0] = 0;
+    for (int r = 0; r < 9; ++r) a.tap_row[r] = r;
+    a.n_views = 1; a.views[0] = plain_view(dmid, H, W); a.in_H = H; a.in_W = W;
+    a.weights = reinterpret_cast<const uint16_t*>(ws + L.c1d); a.cout_total = 32; a.block_n = 32;
+    a.bias = nullptr; a.act = ACT_NONE; a.out = dlr; a.out_mode = OUT_FOLD9_NCHW;
+    RC(launch_conv_gemm(a, st));
+    e->launches += 1;
+  }
+  if (!pg) return 0;
   RC(bias_grad(dmid, P, "conv1.bias"));
   RC(wgrad(plain_view(ws + L.U1, H + 1, W), H + 1, W, true, H, W, dmid, 1, false, e->d_wg_idx_conv1, "conv1.weight"));
   if (batched) {
@@ -1464,6 +1561,23 @@ int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, 
     e->launches += 2;
   }
   return 0;
+}
+}  // namespace
+
+int generator_backward(GeneratorEngine* g, const float* dsr, cudaStream_t st) {
+  return generator_backward_phases(g, dsr, kPhaseAll, st);
+}
+
+int generator_backward_phases(GeneratorEngine* g, const float* dsr, int phases, cudaStream_t st) {
+  return backward_impl(static_cast<EngineImpl*>(g), dsr, phases, true, nullptr, st);
+}
+
+int generator_backward_ex(GeneratorEngine* g, const float* dsr, int param_grads, float* dlr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  if (dsr == nullptr) { set_error("generator_backward_ex: null d(sr)"); return -22; }
+  if (param_grads == 0 && dlr == nullptr) { set_error("generator_backward_ex: nothing to compute (param_grads == 0 and dlr == NULL)"); return -22; }
+  if (!e->ws || !e->ws_training) { set_error("generator_backward_ex: needs a training-sized bound workspace"); return -25; }
+  return backward_impl(e, dsr, kPhaseAll, param_grads != 0, dlr, st);
 }
 
 }  // namespace srg

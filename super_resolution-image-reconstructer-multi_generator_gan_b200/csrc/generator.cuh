@@ -88,6 +88,11 @@ int generator_pack(GeneratorEngine* g, cudaStream_t st);
 int generator_forward(GeneratorEngine* g, const float* lr_nchw, float* sr_nchw, int training, int update_running,
                       cudaStream_t st);
 int generator_backward(GeneratorEngine* g, const float* dsr_nchw, cudaStream_t st);
+// eval-mode (running-statistics) BatchNorm on a training-bound workspace, keeping what the backward needs
+int generator_forward_frozen(GeneratorEngine* g, const float* lr_nchw, float* sr_nchw, cudaStream_t st);
+// backward of the last forward (training or frozen); param_grads == 0: no parameter gradient is computed or written;
+// dlr_nchw (optional) receives d(loss)/d(lr), fp32 N x 3 x H x W
+int generator_backward_ex(GeneratorEngine* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, cudaStream_t st);
 // Split execution for the multi-generator step: PRE = everything before the residual trunk, TRUNK = the trunk itself,
 // POST = everything after it (forward: conv1 | blocks + conv2 | upsample + conv3; backward: conv3 + upsample stages |
 // trunk dgrad chain | conv1 gradients + the batched trunk weight gradients).  The TRUNK phases of several engines of equal

@@ -629,7 +629,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) trunk_kernel(const __grid_const
           s_coef[ch] = float(sc);
           s_coef[64 + ch] = float(-sc * inv * dg / p.count);
           s_coef[128 + ch] = float(-sc * db / p.count + sc * inv * mean * dg / p.count);
-          if (cta == 0) {
+          if (cta == 0 && pp.grads != nullptr) {     // null: input-gradient-only backward
             pp.grads[PL.gamma_off + ch] = float(dg) * p.param_grad_scale;
             pp.grads[PL.beta_off + ch] = float(db) * p.param_grad_scale;
           }

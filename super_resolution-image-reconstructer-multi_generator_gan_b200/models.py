@@ -3,8 +3,8 @@
 ``SRResNet`` keeps the reference's constructor signature, sub-module tree, registration order, default
 initialisation (so ``torch.manual_seed(s); SRResNet()`` yields the reference's weights) and ``state_dict`` keys
 (SURVEY Appendix A), but none of its arithmetic: ``forward`` / ``backward`` are single calls into the C ABI
-(``srg_generator_forward`` / ``srg_generator_backward``), which enqueue hand-written sm_100a kernels on the current
-CUDA stream.  There is no PyTorch / cuDNN / CPU fallback: the sub-modules below only *hold* parameters.
+(``srg_generator_forward`` or ``srg_generator_forward_frozen`` / ``srg_generator_backward_ex``), which enqueue
+hand-written sm_100a kernels on the current CUDA stream.  There is no PyTorch / cuDNN / CPU fallback: the sub-modules below only *hold* parameters.
 
 Parameter storage: every ``nn.Parameter`` is a view into ONE flat fp32 buffer laid out as the engine's parameter table
 (``srg_generator_param_info``); gradients come back as views of one flat buffer of the same layout, so the optimiser
@@ -126,6 +126,7 @@ class _GeneratorEngine:
         self.handle = c_void_p()
         check(L.srg_generator_create(byref(self.handle), N, H, W, n_res, n_up), "srg_generator_create")
         self.N, self.H, self.W, self.n_res, self.n_up, self.training = N, H, W, n_res, n_up, training
+        self.frozen = False        # training workspace driven by srg_generator_forward_frozen (eval-mode autograd)
         self.device = device
         self.busy = False          # a training forward whose backward has not run yet
         self.ws = None
@@ -201,16 +202,22 @@ class _GeneratorEngine:
 
 
 class _GeneratorFn(torch.autograd.Function):
-    """autograd node for one SRResNet pass: forward = srg_generator_forward, backward = srg_generator_backward."""
+    """autograd node for one SRResNet pass: forward = srg_generator_forward (train mode) or srg_generator_forward_frozen
+    (eval mode, running BatchNorm statistics), backward = srg_generator_backward_ex."""
 
     @staticmethod
     def forward(ctx, module, eng, lr_imgs, *params):
         L = _lib.lib()
         sr = torch.empty(eng.N, 3, eng.H << eng.n_up, eng.W << eng.n_up, dtype=torch.float32, device=lr_imgs.device)
-        check(L.srg_generator_forward(eng.handle, c_void_p(lr_imgs.data_ptr()), c_void_p(sr.data_ptr()),
-                                      1 if module.training else 0, 1 if module.training else 0, stream_ptr()),
-              "srg_generator_forward")
+        if eng.frozen:
+            check(L.srg_generator_forward_frozen(eng.handle, c_void_p(lr_imgs.data_ptr()), c_void_p(sr.data_ptr()),
+                                                 stream_ptr()), "srg_generator_forward_frozen")
+        else:
+            check(L.srg_generator_forward(eng.handle, c_void_p(lr_imgs.data_ptr()), c_void_p(sr.data_ptr()),
+                                          1 if module.training else 0, 1 if module.training else 0, stream_ptr()),
+                  "srg_generator_forward")
         ctx.module_ref = weakref.ref(module)
+        ctx.x_shape = tuple(lr_imgs.shape)
         ctx.eng = eng
         _release_on_death(ctx, eng)
         ctx.n_params = len(params)
@@ -228,13 +235,24 @@ class _GeneratorFn(torch.autograd.Function):
         dsr = dsr.contiguous()
         if dsr.dtype != torch.float32:
             dsr = dsr.float()
-        flat_g = module._grad_buffer_for_backward(eng)
-        check(L.srg_generator_set_grads(eng.handle, c_void_p(flat_g.data_ptr())))
-        check(L.srg_generator_backward(eng.handle, c_void_p(dsr.data_ptr()), stream_ptr()), "srg_generator_backward")
+        # data-parallel ranks take the same branch: their requires_grad flags are identical
+        want_dx = ctx.needs_input_grad[2]
+        want_pg = any(ctx.needs_input_grad[3:])
+        dlr = torch.empty(ctx.x_shape, dtype=torch.float32, device=dsr.device) if want_dx else None
+        flat_g = None
+        if want_pg:
+            flat_g = module._grad_buffer_for_backward(eng)
+            check(L.srg_generator_set_grads(eng.handle, c_void_p(flat_g.data_ptr())))
+        check(L.srg_generator_backward_ex(eng.handle, c_void_p(dsr.data_ptr()), 1 if want_pg else 0,
+                                          c_void_p(dlr.data_ptr()) if dlr is not None else None, stream_ptr()),
+              "srg_generator_backward_ex")
         _release_if(eng, ctx.busy_token)
+        if not want_pg:
+            # input gradient only: the flat gradient buffer, the gradient hook and .grad are left alone
+            return (None, None, dlr) + (None,) * ctx.n_params
         module._after_backward(flat_g)
         grads = tuple(flat_g[off:off + n].view(shape) for (_, off, n, shape) in module._ptable)
-        return (None, None, None) + grads
+        return (None, None, dlr) + grads
 
 
 class SRResNet(_FlatModule):
@@ -276,9 +294,11 @@ class SRResNet(_FlatModule):
         return probe.param_table(), probe.buffer_table(), probe.param_elems, probe.buffer_elems
 
     # ---- engines ---------------------------------------------------------------------------------------------------
-    def _engine(self, N: int, H: int, W: int, training: bool, device, need_grad: bool) -> _GeneratorEngine:
+    def _engine(self, N: int, H: int, W: int, training: bool, device, need_grad: bool,
+                frozen: bool = False) -> _GeneratorEngine:
         rt = self._rt
-        key = (N, H, W, training)
+        # frozen engines (eval-mode autograd) run on a training-sized workspace but in their own pool
+        key = (N, H, W, "frozen") if frozen else (N, H, W, training)
         pool = rt["engines"].setdefault(key, [])
         eng = None
         for e in pool:
@@ -286,7 +306,8 @@ class SRResNet(_FlatModule):
                 eng = e
                 break
         if eng is None:
-            eng = _GeneratorEngine(N, H, W, self.num_residuals, self.num_upsample_stages, training, device)
+            eng = _GeneratorEngine(N, H, W, self.num_residuals, self.num_upsample_stages, training or frozen, device)
+            eng.frozen = frozen
             if rt["sync_bn"]:
                 self._attach_sync_bn(eng)
             if getattr(self, "debug_keep_grads", False):
@@ -357,6 +378,28 @@ class SRResNet(_FlatModule):
 
     # ---- forward ---------------------------------------------------------------------------------------------------
     def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """N x 3 x H x W fp32 CUDA -> N x 3 x (H << s) x (W << s), s = ``num_upsample_stages``.
+
+        ====== ========= ================== ========================= =================================================
+        mode   grad mode ``x.requires_grad`` any param requires grad   behaviour
+        ====== ========= ================== ========================= =================================================
+        train  on        no                 any                       batch statistics; parameter gradients
+        train  on        yes                yes                       the same, plus ``x.grad``
+        train  on        yes                no                        input-only backward: ``x.grad``, no parameter
+                                                                      gradient is computed and the gradient hook is
+                                                                      not called
+        eval   off       any                any                       detached output, BatchNorm folded into the convs,
+                                                                      large batches streamed in chunks
+        eval   on        no                 any                       the same (detached)
+        eval   on        yes                any                       running BatchNorm statistics, never updated
+                                                                      ("frozen"), whole batch in one engine call:
+                                                                      ``x.grad`` plus the gradients of the parameters
+                                                                      that require grad
+        ====== ========= ================== ========================= =================================================
+
+        The frozen output equals the detached eval output up to bf16 rounding (DESIGN §4).  Double backward is not
+        supported.
+        """
         if not x.is_cuda:
             raise RuntimeError("SRResNet (libsrgan_b200) runs on a CUDA device only; there is no CPU path")
         if x.dim() != 4 or x.shape[1] != 3:
@@ -368,7 +411,9 @@ class SRResNet(_FlatModule):
         self._flatten(x.device)
         rt = self._rt
         need_grad = self.training and torch.is_grad_enabled()
-        if not self.training and N > 1:
+        # eval mode with an input that requires grad (a fixed generator inside a larger differentiable pipeline)
+        frozen = not self.training and torch.is_grad_enabled() and x.requires_grad
+        if not self.training and N > 1 and not frozen:
             # Evaluation (src/evaluation.py:48-50, BASELINE configs[3]): frames are independent in eval mode (running
             # BatchNorm statistics), so a batch whose activations would not fit the streaming budget is run in chunks
             # of whole frames through ONE smaller engine: peak memory is O(chunk), the arithmetic per frame (and hence
@@ -382,16 +427,16 @@ class SRResNet(_FlatModule):
                     j = min(N, i + chunk)
                     self._eval_into(x[i:j], sr[i:j], packed)   # whole frames of an NCHW batch are contiguous: no copy
                 return sr
-        eng = self._engine(N, H, W, self.training, x.device, need_grad)
-        if self.training and getattr(eng, "grad_flat", None) is None:
+        eng = self._engine(N, H, W, self.training, x.device, need_grad, frozen=frozen)
+        if eng.training and getattr(eng, "grad_flat", None) is None:
             eng.grad_flat = torch.empty_like(rt["flat"])
-        eng.bind(rt["flat"], eng.grad_flat if self.training else None, rt["flat_buf"])
+        eng.bind(rt["flat"], eng.grad_flat if eng.training else None, rt["flat_buf"])
         L = _lib.lib()
         check(L.srg_generator_pack(eng.handle, stream_ptr()), "srg_generator_pack")
         rt["last_engine"] = eng
         if self.training and rt["nbt"] is not None and self.num_residuals > 0:
             rt["nbt"] += 1
-        if need_grad:
+        if need_grad or frozen:
             _acquire(eng)
             return _GeneratorFn.apply(self, eng, x, *rt["plist"])
         # eval mode (running statistics) or no_grad: no autograd graph.  The reference keeps a graph through an
