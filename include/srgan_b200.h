@@ -79,6 +79,26 @@ int srg_generator_forward_frozen(srg_generator_t* g, const float* lr_nchw, float
  * call on a null engine or dsr_nchw, an unbound or eval-bound workspace, or param_grads == 0 with dlr_nchw == NULL. */
 int srg_generator_backward_ex(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream);
 
+/* Spatially tiled eval forward: upscale frames larger than the engine, window by window, bit-identical to the whole-frame
+ * eval forward.  srg_generator_tile_halo: the receptive radius in LR pixels (40 for 16 residual blocks and 2 upsample
+ * stages): an output pixel depends on the input pixels at most that far away (-1 on negative arguments).
+ * srg_generator_forward_tiles: the engine, created as (N, Hw, Ww) and bound to an EVAL workspace, runs n <= min(N,
+ * SRG_MAX_TILES) windows of Hw x Ww LR pixels, taken from any of the F frames (NCHW fp32, F x 3 x H x W), in one eval pass:
+ * window i is read from frames[tile.frame, :, y0 .. y0+Hw-1, x0 .. x0+Ww-1] (zero outside it, exactly as if it had been
+ * cropped into its own tensor), and only the output pixels of its crop (crop_y0 .. crop_y0+crop_h-1 etc., window-relative,
+ * times 2^n_up) are written, into sr_nchw (F x 3 x (H << n_up) x (W << n_up)) at their place in the frame.  A crop edge that
+ * is not a frame edge must lie at least srg_generator_tile_halo() pixels inside its window for the output to equal the
+ * whole-frame forward; window origins on even rows keep it bit-identical (conv3_il's even / odd row blocks accumulate the
+ * three row taps in different orders).  `tiles` is a HOST array, copied into the kernel parameters: no allocation, upload
+ * or synchronisation, so the call can be captured in a CUDA graph.  Every argument is checked before any CUDA call. */
+typedef struct {
+  int32_t frame, y0, x0, crop_y0, crop_x0, crop_h, crop_w; /* LR pixels; (y0, x0) = window origin in the frame, crop relative to the window */
+} srg_tile_t;
+#define SRG_MAX_TILES 64
+int srg_generator_tile_halo(int num_residuals, int num_upsample_stages);
+int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W, const srg_tile_t* tiles,
+                                int n, float* sr_nchw, void* stream);
+
 /* named intermediates inside the workspace (per-layer parity checks): dtype 0 = bf16 NHWC, dims = N,H,W,C */
 int srg_generator_num_tensors(const srg_generator_t* g);
 int srg_generator_tensor_info(const srg_generator_t* g, int i, char* name, int name_cap, int64_t* byte_offset,

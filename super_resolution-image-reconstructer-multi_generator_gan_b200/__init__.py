@@ -9,6 +9,8 @@ package without that library raises as soon as a kernel is needed -- there is no
 from . import _lib
 from ._lib import build, check, lib
 from .models import BatchNormParams, ConvParams, Discriminator, ResidualBlock, SRResNet
+from . import tiling
+from .tiling import plan_tiles, tile_halo
 from .loss import ReconstructionLoss, bce_loss, l1_loss, mse_loss, tanh_mean
 from .optim import Adam
 from .policy import (GAN, PIXEL, MultiGeneratorPolicy, PolicyConfig, decide, gan_probability, interpolate_models,
@@ -23,4 +25,4 @@ from .evaluation import (ImageEnhancer, calculate_psnr, calculate_ssim, image_me
 
 __all__ = ["joint_pixel_generator_steps", "SRResNet", "ResidualBlock", "Discriminator", "ReconstructionLoss", "tanh_mean", "Adam", "train_generator",
            "train_discriminator", "train_one_epoch", "compute_score", "image_metrics", "calculate_ssim", "DevicePrefetcher", "MultiGeneratorGAN", "GraphedGeneratorStep", "MultiGeneratorPolicy", "PolicyConfig",
-           "build", "lib", "parallel"]
+           "build", "lib", "parallel", "tiling", "plan_tiles", "tile_halo"]

@@ -134,6 +134,15 @@ int srg_generator_forward_frozen(srg_generator_t* g, const float* lr_nchw, float
   if (g == nullptr) { set_error("srg_generator_forward_frozen: null engine"); return -1; }
   return generator_forward_frozen(G(g), lr_nchw, sr_nchw, S(stream));
 }
+static_assert(sizeof(srg_tile_t) == sizeof(TileDesc) && SRG_MAX_TILES == kMaxTiles, "srg_tile_t mirrors srg::TileDesc");
+int srg_generator_tile_halo(int num_residuals, int num_upsample_stages) {
+  return generator_tile_halo(num_residuals, num_upsample_stages);
+}
+int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W, const srg_tile_t* tiles,
+                                int n, float* sr_nchw, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_forward_tiles: null engine"); return -1; }
+  return generator_forward_tiles(G(g), frames_nchw, F, H, W, reinterpret_cast<const TileDesc*>(tiles), n, sr_nchw, S(stream));
+}
 int srg_generator_backward_ex(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream) {
   if (g == nullptr) { set_error("srg_generator_backward_ex: null engine"); return -1; }
   return generator_backward_ex(G(g), dsr_nchw, param_grads, dlr_nchw, S(stream));

@@ -70,6 +70,13 @@ struct ConvKParams {
   long long* prof;  // optional per-CTA role timers (debug)
 };
 
+// the fold9 instance also carries the cropped-scatter table (the other instances keep their parameter size)
+struct ConvKParamsFold : ConvKParams {
+  FoldScatter scatter;
+};
+template <int BLOCK_N> struct KParamsOf { using type = ConvKParams; };
+template <> struct KParamsOf<32> { using type = ConvKParamsFold; };
+
 constexpr int kThreads = 320;       // warp 0 producer, warp 1 MMA, warps 2..9 epilogue
 constexpr int kEpiThreads = 256;
 constexpr int kFoldPad = 33;
@@ -83,7 +90,7 @@ __device__ __forceinline__ float apply_act(float x, float slope) {
 }
 
 template <int BLOCK_N, int NT>
-__global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_constant__ ConvKParams p) {
+__global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_constant__ typename KParamsOf<BLOCK_N>::type p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __builtin_assume(__isShared(smem));
@@ -305,7 +312,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
 #pragma unroll
         for (int j = 0; j < 32; ++j) fold_buf[m * kFoldPad + j] = __uint_as_float(v[j]);
         named_bar_sync(1, 128);
-        if (tw >= 4 && tw < p.TW - 4 && h < p.H && w >= 0 && w < p.W) {
+        const bool in_crop = p.scatter.n == 0 || (h >= p.scatter.t[n].h_lo && h < p.scatter.t[n].h_hi &&
+                                                  w >= p.scatter.t[n].w_lo && w < p.scatter.t[n].w_hi);
+        if (tw >= 4 && tw < p.TW - 4 && h < p.H && w >= 0 && w < p.W && in_crop) {
           float o0 = p.bias ? p.bias[0] : 0.f, o1 = p.bias ? p.bias[1] : 0.f, o2 = p.bias ? p.bias[2] : 0.f;
 #pragma unroll
           for (int s = 0; s < 9; ++s) {
@@ -315,8 +324,14 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
             o2 += row[2];
           }
           float* o = reinterpret_cast<float*>(p.out);
-          const size_t plane = size_t(p.H) * p.W;
-          const size_t base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
+          size_t plane, base;
+          if (p.scatter.n == 0) {
+            plane = size_t(p.H) * p.W;
+            base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
+          } else {
+            plane = size_t(p.scatter.plane);
+            base = size_t(p.scatter.t[n].base + int64_t(h) * p.scatter.pitch + w);
+          }
           o[base] = o0;
           o[base + plane] = o1;
           o[base + 2 * plane] = o2;
@@ -1035,8 +1050,9 @@ struct C9KParams {
   int tiles_h, tiles_w, tiles_total, n_ctas;
   int n_stages;
   const float* bias;         // [3] or null
-  float* out;                // fp32 [N,3,H,W]
+  float* out;                // fp32 [N,3,H,W], or full frames through `scatter`
   long long* prof;
+  FoldScatter scatter;       // n == 0: plain store
 };
 
 constexpr int kC9Threads = 64 + 256;            // warp 0 producer, warp 1 MMA, warps 2-5 / 6-9 epilogue groups
@@ -1185,7 +1201,9 @@ __global__ void __launch_bounds__(kC9Threads, 1) conv9_rows_kernel(const __grid_
         for (int c = 0; c < 32; ++c) fb[m * kFoldPad + c] = __uint_as_float(v[c]);
         named_bar_sync(1 + 2 * grp, 128);
         const int h = h0 + j;
-        if (m >= 4 && m < 124 && h < p.H && w < p.W) {
+        const bool in_crop = p.scatter.n == 0 || (h >= p.scatter.t[n].h_lo && h < p.scatter.t[n].h_hi &&
+                                                  w >= p.scatter.t[n].w_lo && w < p.scatter.t[n].w_hi);
+        if (m >= 4 && m < 124 && h < p.H && w < p.W && in_crop) {
           float o0 = b0, o1 = b1, o2 = b2;
 #pragma unroll
           for (int s = 0; s < 9; ++s) {
@@ -1194,10 +1212,18 @@ __global__ void __launch_bounds__(kC9Threads, 1) conv9_rows_kernel(const __grid_
             o1 += row[1];
             o2 += row[2];
           }
-          const size_t base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
-          p.out[base] = o0;
-          p.out[base + plane] = o1;
-          p.out[base + 2 * plane] = o2;
+          if (p.scatter.n == 0) {
+            const size_t base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
+            p.out[base] = o0;
+            p.out[base + plane] = o1;
+            p.out[base + 2 * plane] = o2;
+          } else {
+            const size_t pl = size_t(p.scatter.plane);
+            const size_t base = size_t(p.scatter.t[n].base + int64_t(h) * p.scatter.pitch + w);
+            p.out[base] = o0;
+            p.out[base + pl] = o1;
+            p.out[base + 2 * pl] = o2;
+          }
         }
         named_bar_sync(2 + 2 * grp, 128);
       }
@@ -1288,7 +1314,7 @@ static int num_sms() {
 }
 
 template <int BLOCK_N, int NT>
-static int launch_instance(const ConvKParams& p, dim3 grid, size_t smem_bytes, cudaStream_t stream) {
+static int launch_instance(const typename KParamsOf<BLOCK_N>::type& p, dim3 grid, size_t smem_bytes, cudaStream_t stream) {
   static DeviceOnce attr_set;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<BLOCK_N, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1546,6 +1572,7 @@ static int launch_conv9_rows(const ConvGemmArgs& a, cudaStream_t stream) {
   p.bias = a.bias;
   p.out = reinterpret_cast<float*>(a.out);
   p.prof = reinterpret_cast<long long*>(a.prof);
+  if (a.scatter != nullptr) p.scatter = *a.scatter;
   static DeviceOnce attr_set;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(conv9_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -1590,6 +1617,10 @@ int launch_conv_gemm_grouped(const ConvGemmArgs* as, int n, cudaStream_t stream)
 }
 
 int launch_conv_gemm(const ConvGemmArgs& a, cudaStream_t stream) {
+  if (a.scatter != nullptr && (a.out_mode != OUT_FOLD9_NCHW || a.scatter->n > kMaxTiles || a.scatter->n != a.N)) {
+    set_error("conv_gemm: a cropped scatter needs the fold9 output and one entry per item (at most %d)", kMaxTiles);
+    return -20;
+  }
   if (use_conv3_il(a)) return launch_conv3_il(&a, 1, stream);
   if (use_conv9_rows(a)) return launch_conv9_rows(a, stream);
   if (a.TH * a.TW != 128 || a.TW % 8 != 0) { set_error("conv_gemm: tile must be 128 pixels with TW%%8==0"); return -1; }
@@ -1716,7 +1747,11 @@ int launch_conv_gemm(const ConvGemmArgs& a, cudaStream_t stream) {
   const dim3 grid(p.ctas_per_block * p.n_blocks);
   if (fold) {
     if (a.n_taps != 9) { set_error("conv_gemm: fold9 needs 9 row taps"); return -14; }
-    return launch_instance<32, 9>(p, grid, smem_bytes, stream);
+    ConvKParamsFold pf;
+    memset(&pf, 0, sizeof(pf));
+    static_cast<ConvKParams&>(pf) = p;
+    if (a.scatter != nullptr) pf.scatter = *a.scatter;
+    return launch_instance<32, 9>(pf, grid, smem_bytes, stream);
   }
   switch (a.n_taps) {
     case 1: return launch_instance<64, 1>(p, grid, smem_bytes, stream);

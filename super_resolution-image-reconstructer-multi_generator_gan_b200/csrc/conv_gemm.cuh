@@ -20,6 +20,20 @@ enum ConvOutMode : int {
   OUT_NHWC_F32 = 3,      // fp32 [N,H,W,cout_total] (direct 128-bit stores; discriminator conv outputs)
 };
 
+// Cropped scatter of a fold9 (OUT_FOLD9_NCHW) launch over n <= kMaxTiles windows (srg_generator_forward_tiles): output
+// pixel (h, w) of item i is written only when h_lo <= h < h_hi and w_lo <= w < w_hi, to element base + h * pitch + w of
+// channel 0 (+ plane per channel) of the caller's full-size frames.  Passed by value in the kernel parameters.
+constexpr int kMaxTiles = 64;
+struct FoldTile {
+  int64_t base;            // element offset of the window origin in channel 0 of its frame
+  int h_lo, h_hi, w_lo, w_hi;
+};
+struct FoldScatter {
+  int n;                   // 0: plain NCHW store of the [N,3,H,W] output
+  int64_t plane, pitch;    // elements per output channel plane / row of the full frame
+  FoldTile t[kMaxTiles];
+};
+
 // One view of the (NHWC bf16) input that a K-chunk is loaded from. A plain tensor uses one view;
 // the pixel-unshuffled gradient of an up-conv uses four strided views of the HR tensor.
 struct InView {
@@ -68,6 +82,7 @@ struct ConvGemmArgs {
   const void* stats_y;       // optional with `stats`: bf16 tensor of the output's geometry; the second 64 columns then hold
                              // sum(out * stats_y) instead of sum(out^2) (BatchNorm backward: sum dz, sum dz*y)
   void* prof;                // optional debug timers: int64 [grid][3][6]
+  const FoldScatter* scatter;  // optional (OUT_FOLD9_NCHW only, host memory): cropped scatter into full frames at `out`
   // fold9: tile columns overlap; valid output columns per tile = TW-8
 };
 

@@ -903,11 +903,29 @@ int launch_ps_bias_grad(const void* g, int N, int H2, int W2, float* scratch, fl
 // ------------------------------------------------------------------------------------------------
 // unfold9: one thread per (pixel of the H+1 row grid, channel group of 8)
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) unfold9_kernel(const float* __restrict__ src, int N, int H, int W, float scale,
+// Where row hh (0 <= hh < H) of channel c of item n starts: a dense [N,3,H,W] batch, or a window of a larger frame
+// (launch_unfold9_windows).  Both kernels below read their source through one of these.
+struct PlainRows {
+  const float* src;
+  int64_t plane;
+  int W;
+  __device__ __forceinline__ const float* row(int n, int c, int hh) const {
+    return src + (int64_t(n) * 3 + c) * plane + int64_t(hh) * W;
+  }
+};
+struct WindowRows {
+  const float* src;
+  WindowGather g;
+  __device__ __forceinline__ const float* row(int n, int c, int hh) const {
+    return src + g.base[n] + c * g.plane + int64_t(hh) * g.pitch;
+  }
+};
+
+template <class Rows>
+__global__ void __launch_bounds__(256) unfold9_kernel(const __grid_constant__ Rows rows, int N, int H, int W, float scale,
                                                       uint4* __restrict__ dst) {
   // one thread per (n, h', w): gathers the 2 x 9 x 3 neighbourhood once and writes the pixel's 128-byte row
   const int64_t total = int64_t(N) * (H + 1) * W;
-  const int64_t plane = int64_t(H) * W;
   for (int64_t pix = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; pix < total; pix += int64_t(gridDim.x) * blockDim.x) {
     const int w = int(pix % W);
     const int64_t t = pix / W;
@@ -922,7 +940,7 @@ __global__ void __launch_bounds__(256) unfold9_kernel(const float* __restrict__ 
       const bool row_ok = hh >= 0 && hh < H;
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        const float* row = src + (int64_t(n) * 3 + c) * plane + int64_t(row_ok ? hh : 0) * W;
+        const float* row = rows.row(n, c, row_ok ? hh : 0);
 #pragma unroll
         for (int sft = 0; sft < 9; ++sft) {
           const int ww = w + sft - 4;
@@ -944,13 +962,13 @@ __global__ void __launch_bounds__(256) unfold9_kernel(const float* __restrict__ 
 // two source rows x three planes (+4 halo pixels each side) are read ONCE into shared memory with coalesced loads, every
 // thread assembles its pixel's 54 values from there, and the 16 KB of output go out as fully coalesced 16-byte vectors
 // (the per-thread form issues 54 global loads per pixel and writes 128-byte rows with a 128-byte lane stride).
-__global__ void __launch_bounds__(128) unfold9_tile_kernel(const float* __restrict__ src, int N, int H, int W, float scale,
+template <class Rows>
+__global__ void __launch_bounds__(128) unfold9_tile_kernel(const __grid_constant__ Rows rows, int N, int H, int W, float scale,
                                                            uint4* __restrict__ dst) {
   __shared__ float tile[6][136];             // [dr * 3 + c][4 + 128 + 4]
   __shared__ uint4 stage[128 * 8];
   const int segs = W / 128;
   const int64_t total = int64_t(N) * (H + 1) * segs;
-  const int64_t plane = int64_t(H) * W;
   const int tp = threadIdx.x;
   for (int64_t blk = blockIdx.x; blk < total; blk += gridDim.x) {
     const int seg = int(blk % segs);
@@ -962,7 +980,7 @@ __global__ void __launch_bounds__(128) unfold9_tile_kernel(const float* __restri
       const int r = i / 136, x = i - r * 136;
       const int dr = r / 3, c = r - dr * 3;
       const int hh = hp - 1 + dr, ww = w0 + x - 4;
-      tile[r][x] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? __ldg(src + (int64_t(n) * 3 + c) * plane + int64_t(hh) * W + ww) * scale : 0.f;
+      tile[r][x] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? __ldg(rows.row(n, c, hh) + ww) * scale : 0.f;
     }
     __syncthreads();
 #pragma unroll
@@ -988,17 +1006,29 @@ __global__ void __launch_bounds__(128) unfold9_tile_kernel(const float* __restri
     __syncthreads();
   }
 }
-int launch_unfold9(const float* src, int N, int H, int W, float scale, void* dst, cudaStream_t st) {
+template <class Rows>
+static int launch_unfold9_rows(const Rows& rows, int N, int H, int W, float scale, void* dst, cudaStream_t st) {
   const int64_t total = int64_t(N) * (H + 1) * W;
   if (W % 128 == 0) {
     int64_t blocks = int64_t(N) * (H + 1) * (W / 128);
     if (blocks > int64_t(sm_budget()) * 16) blocks = int64_t(sm_budget()) * 16;
-    unfold9_tile_kernel<<<int(blocks), 128, 0, st>>>(src, N, H, W, scale, reinterpret_cast<uint4*>(dst));
+    unfold9_tile_kernel<Rows><<<int(blocks), 128, 0, st>>>(rows, N, H, W, scale, reinterpret_cast<uint4*>(dst));
   } else {
-    unfold9_kernel<<<ew_blocks(total), 256, 0, st>>>(src, N, H, W, scale, reinterpret_cast<uint4*>(dst));
+    unfold9_kernel<Rows><<<ew_blocks(total), 256, 0, st>>>(rows, N, H, W, scale, reinterpret_cast<uint4*>(dst));
   }
   SRG_LAUNCH_CHECK("unfold9");
   return 0;
+}
+int launch_unfold9(const float* src, int N, int H, int W, float scale, void* dst, cudaStream_t st) {
+  const PlainRows rows{src, int64_t(H) * W, W};
+  return launch_unfold9_rows(rows, N, H, W, scale, dst, st);
+}
+int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st) {
+  if (wg.n < 1 || wg.n > kMaxWindows) { set_error("unfold9_windows: 1..%d windows", kMaxWindows); return -1; }
+  WindowRows rows;
+  rows.src = frames;
+  rows.g = wg;
+  return launch_unfold9_rows(rows, wg.n, H, W, 1.f, dst, st);
 }
 
 // ------------------------------------------------------------------------------------------------

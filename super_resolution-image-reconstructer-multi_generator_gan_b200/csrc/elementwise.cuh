@@ -97,6 +97,16 @@ int launch_ps_bias_grad(const void* g, int N, int H2, int W2, float* scratch, fl
 // dst bf16 [N][H+1][W][64]; channel (dr*27 + s*3 + c) of row h' holds src[n][c][h'-1+dr][w+s-4] (0 outside,
 // channels 54..63 = 0).  `scale` multiplies the values (used to keep tiny loss gradients in bf16 range).
 int launch_unfold9(const float* src, int N, int H, int W, float scale, void* dst, cudaStream_t st);
+// Window gather form: item i of the same [N][H+1][W][64] operand is the H x W window whose origin (channel 0) is element
+// base[i] of `frames` (NCHW fp32 frames of `plane` elements per channel and `pitch` per row), zero outside the window
+// exactly as if the window had been cropped into its own tensor.  Passed by value in the kernel parameters.
+constexpr int kMaxWindows = 64;
+struct WindowGather {
+  int n;
+  int64_t plane, pitch;
+  int64_t base[kMaxWindows];
+};
+int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st);
 
 // ---- parameters ------------------------------------------------------------------------------------
 // dst[i] = bf16(idx[i] >= 0 ? src[idx[i]] : 0)

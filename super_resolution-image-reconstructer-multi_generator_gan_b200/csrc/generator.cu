@@ -1065,10 +1065,20 @@ int generator_forward(GeneratorEngine* g, const float* lr, float* sr, int traini
 }
 
 namespace {
+// srg_generator_forward_tiles: n windows of larger frames in one eval pass (conv1's operand gathered from the frames,
+// conv3's output scattered into them, cropped)
+static_assert(kMaxWindows == kMaxTiles, "gather and scatter tables hold the same windows");
+struct TileCall {
+  const float* frames;
+  int n;
+  WindowGather gather;
+  FoldScatter scatter;
+};
+
 // frozen: eval-mode BatchNorm (running statistics, never updated or exchanged) on the training workspace, every
 // activation the backward reads kept; per-layer trunk launches only
 int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int update_running, int phases, bool frozen,
-                 cudaStream_t st) {
+                 cudaStream_t st, const TileCall* tc = nullptr) {
   if (!e->ws) { set_error("generator_forward: not bound"); return -23; }
   if (training && !e->ws_training) { set_error("generator_forward: bound workspace is eval-sized"); return -24; }
   if (training) e->last_frozen = frozen;
@@ -1078,7 +1088,7 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
   uint8_t* ws = e->ws;
   const uint16_t* packed = reinterpret_cast<const uint16_t*>(ws + L.packed);
   const float* pbias = reinterpret_cast<const float*>(ws + L.bias);
-  const int N = e->N, H = e->H, W = e->W;
+  const int N = tc ? tc->n : e->N, H = e->H, W = e->W;
   const int64_t P = int64_t(N) * H * W;
   char nm[96];
 
@@ -1101,7 +1111,8 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
   }
   // conv1: 9x9, 3->64, LeakyReLU(0.2)  (src/models.py:56-57,81)
   if (phases & kPhasePre) {
-  RC(launch_unfold9(lr, N, H, W, 1.f, ws + L.U1, st));
+  if (tc) RC(launch_unfold9_windows(tc->frames, tc->gather, H, W, ws + L.U1, st));
+  else RC(launch_unfold9(lr, N, H, W, 1.f, ws + L.U1, st));
   {
     ConvGemmArgs a; memset(&a, 0, sizeof(a));
     a.N = N; a.H = H; a.W = W; set_taps_pairs(a);
@@ -1241,12 +1252,68 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
     a.n_views = 1; a.views[0] = plain_view(in, Hs, Ws); a.in_H = Hs; a.in_W = Ws;
     a.weights = packed + po.conv3_f; a.cout_total = 32; a.block_n = 32;
     a.bias = e->master + poff(*e, "conv3.bias"); a.act = ACT_NONE; a.out = sr; a.out_mode = OUT_FOLD9_NCHW;
+    if (tc) a.scatter = &tc->scatter;
     RC(launch_conv_gemm(a, st));
     e->launches += 1;
   }
   return 0;
 }
 }  // namespace
+
+int generator_tile_halo(int n_res, int n_up) {
+  if (n_res < 0 || n_up < 0 || n_up > 8) { set_error("tile_halo: num_residuals >= 0 and 0 <= num_upsample_stages <= 8"); return -1; }
+  // rows of the input an output row at LR row 0 depends on, walked from conv3 (9x9 at 2^n_up) back to conv1
+  int lo = -4, hi = (1 << n_up) + 3;
+  for (int j = 0; j < n_up; ++j) {
+    lo = (lo >> 1) - 1;               // PixelShuffle (floor division), then the up-conv's 3x3 taps
+    hi = (hi >> 1) + 1;
+  }
+  const int r = lo < -hi ? -lo : hi;
+  return r + (2 * n_res + 1) + 4;      // the trunk's 3x3 convs (2 per block + conv2), conv1's 9x9
+}
+
+int generator_forward_tiles(GeneratorEngine* g, const float* frames, int F, int H, int W, const TileDesc* tiles, int n,
+                            float* sr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  if (frames == nullptr || tiles == nullptr || sr == nullptr) { set_error("srg_generator_forward_tiles: null pointer"); return -22; }
+  if (F < 1 || H < 1 || W < 1) { set_error("srg_generator_forward_tiles: F, H and W must be >= 1 (got %d, %d, %d)", F, H, W); return -26; }
+  const int n_max = e->N < kMaxTiles ? e->N : kMaxTiles;
+  if (n < 1 || n > n_max) { set_error("srg_generator_forward_tiles: tile count %d outside 1..%d (engine N and SRG_MAX_TILES)", n, n_max); return -27; }
+  for (int i = 0; i < n; ++i) {
+    const TileDesc& t = tiles[i];
+    if (t.frame < 0 || t.frame >= F) { set_error("srg_generator_forward_tiles: tile %d frame index %d outside 0..%d", i, t.frame, F - 1); return -28; }
+    if (t.y0 < 0 || t.x0 < 0 || int64_t(t.y0) + e->H > H || int64_t(t.x0) + e->W > W) {
+      set_error("srg_generator_forward_tiles: tile %d window (%d, %d) + %d x %d is not inside the %d x %d frame", i, t.y0, t.x0,
+                e->H, e->W, H, W);
+      return -29;
+    }
+    if (t.crop_h < 1 || t.crop_w < 1) { set_error("srg_generator_forward_tiles: tile %d crop is empty", i); return -30; }
+    if (t.crop_y0 < 0 || t.crop_x0 < 0 || int64_t(t.crop_y0) + t.crop_h > e->H || int64_t(t.crop_x0) + t.crop_w > e->W) {
+      set_error("srg_generator_forward_tiles: tile %d crop is not inside its window", i);
+      return -31;
+    }
+  }
+  if (!e->ws) { set_error("srg_generator_forward_tiles: no workspace bound"); return -23; }
+  if (e->ws_training) { set_error("srg_generator_forward_tiles: needs an eval-sized workspace (this one is bound for training)"); return -24; }
+
+  const int s = e->n_up;
+  const int64_t plane = int64_t(H) * W, Ws = int64_t(W) << s, plane_o = (int64_t(H) << s) * Ws;
+  TileCall tc;
+  memset(&tc, 0, sizeof(tc));
+  tc.frames = frames;
+  tc.n = n;
+  tc.gather.n = n; tc.gather.plane = plane; tc.gather.pitch = W;
+  tc.scatter.n = n; tc.scatter.plane = plane_o; tc.scatter.pitch = Ws;
+  for (int i = 0; i < n; ++i) {
+    const TileDesc& t = tiles[i];
+    tc.gather.base[i] = int64_t(t.frame) * 3 * plane + int64_t(t.y0) * W + t.x0;
+    FoldTile& o = tc.scatter.t[i];
+    o.base = int64_t(t.frame) * 3 * plane_o + (int64_t(t.y0) << s) * Ws + (int64_t(t.x0) << s);
+    o.h_lo = t.crop_y0 << s; o.h_hi = (t.crop_y0 + t.crop_h) << s;
+    o.w_lo = t.crop_x0 << s; o.w_hi = (t.crop_x0 + t.crop_w) << s;
+  }
+  return forward_impl(e, nullptr, sr, 0, 0, kPhaseAll, false, st, &tc);
+}
 
 int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int training, int update_running, int phases,
                              cudaStream_t st) {

@@ -93,6 +93,11 @@ int generator_forward_frozen(GeneratorEngine* g, const float* lr_nchw, float* sr
 // backward of the last forward (training or frozen); param_grads == 0: no parameter gradient is computed or written;
 // dlr_nchw (optional) receives d(loss)/d(lr), fp32 N x 3 x H x W
 int generator_backward_ex(GeneratorEngine* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, cudaStream_t st);
+// spatially tiled eval forward (srg_generator_forward_tiles): same layout as srg_tile_t, LR pixels
+struct TileDesc { int32_t frame, y0, x0, crop_y0, crop_x0, crop_h, crop_w; };
+int generator_tile_halo(int n_res, int n_up);
+int generator_forward_tiles(GeneratorEngine* g, const float* frames_nchw, int F, int H, int W, const TileDesc* tiles, int n,
+                            float* sr_nchw, cudaStream_t st);
 // Split execution for the multi-generator step: PRE = everything before the residual trunk, TRUNK = the trunk itself,
 // POST = everything after it (forward: conv1 | blocks + conv2 | upsample + conv3; backward: conv3 + upsample stages |
 // trunk dgrad chain | conv1 gradients + the batched trunk weight gradients).  The TRUNK phases of several engines of equal

@@ -22,7 +22,7 @@ from typing import Dict, List, Optional, Tuple
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, tiling
 from ._flat import _FlatModule
 from ._lib import check, stream_ptr
 
@@ -362,19 +362,51 @@ class SRResNet(_FlatModule):
     #: eval-mode activation budget in bytes: larger batches are streamed in chunks of frames (None: never chunk)
     stream_budget_bytes: Optional[int] = 6 << 30
 
-    def _stream_chunk(self, N: int, H: int, W: int, device) -> int:
-        """Frames per eval-mode engine call such that the engine workspace stays within ``stream_budget_bytes``."""
-        budget = self.stream_budget_bytes
-        if budget is None:
-            return N
+    #: eval-mode workspace budget in bytes for ONE frame: a frame whose whole-frame eval workspace is larger is upscaled
+    #: window by window (spatial tiles with a halo, ``tiling.plan_tiles``), bit-identical to the whole-frame forward,
+    #: with at most this much engine workspace (None: never tile)
+    tile_budget_bytes: Optional[int] = None
+
+    def _eval_ws_bytes(self, H: int, W: int, device) -> int:
+        """eval workspace of a one-frame H x W engine (a probe engine: creation needs no device memory)"""
         rt = self._rt
         key = ("ws1", H, W)
         if key not in rt:
             probe = _GeneratorEngine(1, H, W, self.num_residuals, self.num_upsample_stages, False, device)
             rt[key] = int(_lib.lib().srg_generator_workspace_bytes(probe.handle, 0))
             del probe
-        per_frame = max(rt[key], 1)
+        return rt[key]
+
+    def _stream_chunk(self, N: int, H: int, W: int, device) -> int:
+        """Frames per eval-mode engine call such that the engine workspace stays within ``stream_budget_bytes``."""
+        budget = self.stream_budget_bytes
+        if budget is None:
+            return N
+        per_frame = max(self._eval_ws_bytes(H, W, device), 1)
         return max(1, min(N, int(budget // per_frame)))
+
+    def _forward_tiled(self, x: torch.Tensor) -> torch.Tensor:
+        """eval-mode forward of frames too large for ``tile_budget_bytes``: the windows of all frames in order, as many per
+        ``srg_generator_forward_tiles`` call as the plan's ``tiles_per_call`` (usually 1: the planner picks the largest
+        window that fits), through ONE engine of that many windows."""
+        N, _, H, W = x.shape
+        rt = self._rt
+        budget = int(self.tile_budget_bytes)
+        key = ("tiles", N, H, W, budget)
+        if key not in rt:
+            halo = tiling.tile_halo(self.num_residuals, self.num_upsample_stages)
+            rt[key] = tiling.plan_tiles(N, H, W, halo, lambda h, w: self._eval_ws_bytes(h, w, x.device), budget)
+        win_h, win_w, per_call, tiles = rt[key]
+        s = self.num_upsample_stages
+        sr = torch.empty(N, 3, H << s, W << s, dtype=torch.float32, device=x.device)
+        n = min(per_call, len(tiles))
+        eng = self._engine(n, win_h, win_w, False, x.device, False)
+        eng.bind(rt["flat"], None, rt["flat_buf"])
+        check(_lib.lib().srg_generator_pack(eng.handle, stream_ptr()), "srg_generator_pack")
+        rt["last_engine"] = eng
+        for i in range(0, len(tiles), n):
+            tiling.forward_tiles(eng.handle, x, tiles[i:i + n], sr, stream_ptr())
+        return sr
 
     # ---- forward ---------------------------------------------------------------------------------------------------
     def forward(self, x: torch.Tensor) -> torch.Tensor:
@@ -390,6 +422,11 @@ class SRResNet(_FlatModule):
                                                                       not called
         eval   off       any                any                       detached output, BatchNorm folded into the convs,
                                                                       large batches streamed in chunks
+        eval   off       any                any                       with ``tile_budget_bytes`` set and a frame whose
+                                                                      eval workspace exceeds it: every frame upscaled
+                                                                      in spatial windows with a halo (the largest
+                                                                      window that fits, so usually one window per
+                                                                      engine call), bit-identical
         eval   on        no                 any                       the same (detached)
         eval   on        yes                any                       running BatchNorm statistics, never updated
                                                                       ("frozen"), whole batch in one engine call:
@@ -413,6 +450,9 @@ class SRResNet(_FlatModule):
         need_grad = self.training and torch.is_grad_enabled()
         # eval mode with an input that requires grad (a fixed generator inside a larger differentiable pipeline)
         frozen = not self.training and torch.is_grad_enabled() and x.requires_grad
+        if (not self.training and not frozen and self.tile_budget_bytes is not None
+                and self._eval_ws_bytes(H, W, x.device) > self.tile_budget_bytes):
+            return self._forward_tiled(x)
         if not self.training and N > 1 and not frozen:
             # Evaluation (src/evaluation.py:48-50, BASELINE configs[3]): frames are independent in eval mode (running
             # BatchNorm statistics), so a batch whose activations would not fit the streaming budget is run in chunks
