@@ -494,6 +494,10 @@ __global__ void __launch_bounds__(kTrThreads, 1) trunk_kernel(const __grid_const
         const int pslot = slot - 1;
         const int pj = pslot >= 0 ? pslot / K : 0, pg = pslot >= 0 ? pslot - pj * K : 0;
         const int pst2 = (interleave && pslot >= 0) ? s_layers[pj].st2_idx : -1;
+        // no pass-2 job of the previous slot to interleave (it had no BatchNorm: the last layer of a direction): the flags
+        // still pending would otherwise wait for this slot's own pass-1 jobs, whose MMAs may need them (K = 2: the last
+        // generator's last layer reads the tiles of the pass-2 job issued one slot earlier)
+        if (interleave && pst2 < 0) flush();
         for (int ti = 0; ti < n_my; ++ti) {
           if (pst2 >= 0) job(pg, pst2, ti, true);
           if (st1 >= 0) job(g, st1, ti, false);
