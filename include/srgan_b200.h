@@ -98,6 +98,25 @@ typedef struct {
 int srg_generator_tile_halo(int num_residuals, int num_upsample_stages);
 int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W, const srg_tile_t* tiles,
                                 int n, float* sr_nchw, void* stream);
+/* Eval-mode autograd over windows, for frames whose whole-frame frozen workspace is too large.  With running BatchNorm
+ * statistics every layer is local, so for windows whose crops partition the frames (crop edges at least
+ * srg_generator_tile_halo() inside the window, as for srg_generator_forward_tiles) the whole-frame gradients are sums of
+ * window-local ones: x.grad adds up every window's input gradient over its whole window, a parameter gradient adds up the
+ * windows' parameter gradients.
+ * srg_generator_forward_frozen_tiles: srg_generator_forward_frozen over n <= min(N, SRG_MAX_TILES) windows, read from the
+ * frames and written to sr_nchw (crops only) exactly as srg_generator_forward_tiles does, on an engine bound to a TRAINING
+ * workspace.  It keeps every activation the backward reads and remembers the windows and the frames' H and W.  sr_nchw may be NULL:
+ * the output conv is then skipped (a recompute for the backward).
+ * srg_generator_backward_tiles: the backward of the last forward, which must be a frozen-tiles forward.  dsr_nchw is
+ * F x 3 x (H << n_up) x (W << n_up); each window's backward sees it inside the window's crop and zero elsewhere.
+ * param_grads != 0: the bound `grads` receive the sum over these windows (overwritten, as srg_generator_backward_ex does).
+ * dlr_nchw (F x 3 x H x W, may be NULL) is ADDED to: every window's input gradient over its whole window, window by window
+ * in table order, deterministic without atomics (the caller zeroes it once before the first call).  Windows of one call
+ * may overlap.  param_grads == 0 with dlr_nchw == NULL fails.  Both check every argument before any CUDA call; tables
+ * travel in kernel parameters.  srg_generator_backward / _ex refuse to run after a frozen-tiles forward. */
+int srg_generator_forward_frozen_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W,
+                                       const srg_tile_t* tiles, int n, float* sr_nchw, void* stream);
+int srg_generator_backward_tiles(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream);
 
 /* named intermediates inside the workspace (per-layer parity checks): dtype 0 = bf16 NHWC, dims = N,H,W,C */
 int srg_generator_num_tensors(const srg_generator_t* g);

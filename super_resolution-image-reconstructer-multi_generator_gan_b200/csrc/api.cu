@@ -143,6 +143,16 @@ int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, in
   if (g == nullptr) { set_error("srg_generator_forward_tiles: null engine"); return -1; }
   return generator_forward_tiles(G(g), frames_nchw, F, H, W, reinterpret_cast<const TileDesc*>(tiles), n, sr_nchw, S(stream));
 }
+int srg_generator_forward_frozen_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W,
+                                       const srg_tile_t* tiles, int n, float* sr_nchw, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_forward_frozen_tiles: null engine"); return -1; }
+  return generator_forward_frozen_tiles(G(g), frames_nchw, F, H, W, reinterpret_cast<const TileDesc*>(tiles), n, sr_nchw,
+                                        S(stream));
+}
+int srg_generator_backward_tiles(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_backward_tiles: null engine"); return -1; }
+  return generator_backward_tiles(G(g), dsr_nchw, param_grads, dlr_nchw, S(stream));
+}
 int srg_generator_backward_ex(srg_generator_t* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, void* stream) {
   if (g == nullptr) { set_error("srg_generator_backward_ex: null engine"); return -1; }
   return generator_backward_ex(G(g), dsr_nchw, param_grads, dlr_nchw, S(stream));

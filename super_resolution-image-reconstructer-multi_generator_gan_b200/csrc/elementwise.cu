@@ -1032,6 +1032,67 @@ int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, i
 }
 
 // ------------------------------------------------------------------------------------------------
+// window gather / scatter-add of the frozen-tiles backward: one thread per (item, channel, row, column) of the window
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ int64_t window_elem(const WindowTable& t, int i, int c, int h, int w) {
+  return ((int64_t(t.frame[i]) * 3 + c) * t.fh + t.y0[i] + h) * t.fw + t.x0[i] + w;
+}
+
+__global__ void __launch_bounds__(256) crop_masked_gather_kernel(const float* __restrict__ frames,
+                                                                 const __grid_constant__ WindowTable t, int H, int W,
+                                                                 float* __restrict__ dst) {
+  const int64_t total = int64_t(t.n) * 3 * H * W;
+  for (int64_t e = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; e < total; e += int64_t(gridDim.x) * blockDim.x) {
+    const int w = int(e % W);
+    const int64_t r = e / W;
+    const int h = int(r % H);
+    const int ic = int(r / H);
+    const int i = ic / 3, c = ic - 3 * i;
+    const bool in = h >= t.h_lo[i] && h < t.h_hi[i] && w >= t.w_lo[i] && w < t.w_hi[i];
+    dst[e] = in ? __ldg(frames + window_elem(t, i, c, h, w)) : 0.f;
+  }
+}
+
+__global__ void __launch_bounds__(256) window_scatter_add_kernel(const float* __restrict__ src,
+                                                                 const __grid_constant__ WindowTable t, int H, int W,
+                                                                 float* __restrict__ frames) {
+  const int64_t total = int64_t(t.n) * 3 * H * W;
+  for (int64_t e = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; e < total; e += int64_t(gridDim.x) * blockDim.x) {
+    const int w = int(e % W);
+    const int64_t r = e / W;
+    const int h = int(r % H);
+    const int ic = int(r / H);
+    const int i = ic / 3, c = ic - 3 * i;
+    const int f = t.frame[i], y = t.y0[i] + h, x = t.x0[i] + w;
+    auto covers = [&](int j) {
+      return t.frame[j] == f && y >= t.y0[j] && y < t.y0[j] + H && x >= t.x0[j] && x < t.x0[j] + W;
+    };
+    // the first window that contains this frame element owns it; later ones are added by the owner, in order
+    bool owner = true;
+    for (int j = 0; j < i && owner; ++j) owner = !covers(j);
+    if (!owner) continue;
+    const int64_t o = window_elem(t, i, c, h, w);
+    float acc = frames[o] + src[e];
+    for (int j = i + 1; j < t.n; ++j)
+      if (covers(j)) acc += src[((int64_t(j) * 3 + c) * H + (y - t.y0[j])) * W + (x - t.x0[j])];
+    frames[o] = acc;
+  }
+}
+
+int launch_crop_masked_gather(const float* frames, const WindowTable& wt, int H, int W, float* dst, cudaStream_t st) {
+  if (wt.n < 1 || wt.n > kMaxWindows) { set_error("crop_masked_gather: 1..%d windows", kMaxWindows); return -1; }
+  crop_masked_gather_kernel<<<ew_blocks(int64_t(wt.n) * 3 * H * W), 256, 0, st>>>(frames, wt, H, W, dst);
+  SRG_LAUNCH_CHECK("crop_masked_gather");
+  return 0;
+}
+int launch_window_scatter_add(const float* src, const WindowTable& wt, int H, int W, float* frames, cudaStream_t st) {
+  if (wt.n < 1 || wt.n > kMaxWindows) { set_error("window_scatter_add: 1..%d windows", kMaxWindows); return -1; }
+  window_scatter_add_kernel<<<ew_blocks(int64_t(wt.n) * 3 * H * W), 256, 0, st>>>(src, wt, H, W, frames);
+  SRG_LAUNCH_CHECK("window_scatter_add");
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
 // parameters
 // ------------------------------------------------------------------------------------------------
 __global__ void pack_bf16_kernel(const float* __restrict__ src, const int* __restrict__ idx, __nv_bfloat16* __restrict__ dst,

@@ -107,6 +107,20 @@ struct WindowGather {
   int64_t base[kMaxWindows];
 };
 int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st);
+// Windows of F x 3 x fh x fw fp32 frames for the backward of the frozen-tiles forward (srg_generator_backward_tiles), in
+// the pixel units of the grid they index (HR for d(SR), LR for d(lr)).  Item i is the window of frame[i] at (y0[i], x0[i]);
+// its crop is rows [h_lo, h_hi) x columns [w_lo, w_hi), window-relative.  Passed by value in the kernel parameters.
+struct WindowTable {
+  int n;
+  int fh, fw;
+  int frame[kMaxWindows], y0[kMaxWindows], x0[kMaxWindows];
+  int h_lo[kMaxWindows], h_hi[kMaxWindows], w_lo[kMaxWindows], w_hi[kMaxWindows];
+};
+// Crop-masked gather: dst (n x 3 x H x W, H x W = the window) = the frames inside each item's crop, 0 elsewhere
+int launch_crop_masked_gather(const float* frames, const WindowTable& wt, int H, int W, float* dst, cudaStream_t st);
+// Ordered scatter-add: frames += src (n x 3 x H x W) over each item's whole window.  Where windows overlap, one thread adds
+// every item's value in table order, ((f + src[i1]) + src[i2]) + ..., so the result is deterministic without atomics.
+int launch_window_scatter_add(const float* src, const WindowTable& wt, int H, int W, float* frames, cudaStream_t st);
 
 // ---- parameters ------------------------------------------------------------------------------------
 // dst[i] = bf16(idx[i] >= 0 ? src[idx[i]] : 0)

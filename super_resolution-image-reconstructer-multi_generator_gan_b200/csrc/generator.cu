@@ -253,6 +253,10 @@ struct EngineImpl : GeneratorEngine {
   std::vector<int> h_pack_idx, h_bias_idx, h_wg_c3x3, h_wg_up, h_wg_conv1, h_wg_conv3, h_conv1_dgrad;
   int* d_conv1_dgrad_idx = nullptr;
   bool last_frozen = false;     // the last forward on the training workspace used running BatchNorm statistics
+  // srg_generator_forward_frozen_tiles: the windows and frame height / width of the last forward on the training workspace when
+  // it was a frozen-tiles forward (tile_n == 0 otherwise); srg_generator_backward_tiles runs their backward
+  int tile_n = 0, tile_H = 0, tile_W = 0;
+  TileDesc tile_tab[kMaxTiles];
   ~EngineImpl() override { cudaFree(d_conv1_dgrad_idx); }
   // fused trunk (trunk_fused.cu): set at bind when the workspace layout is uniformly strided and the geometry fits
   bool trunk_ok = false;
@@ -984,6 +988,7 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
   if (cudaMemset(e->ws + e->L.ticket, 0, 256) != cudaSuccess) { set_error("generator_bind: memset failed"); return -29; }
   e->trunk_ok = false;
   e->last_frozen = false;
+  e->tile_n = 0;
   if (e->n_res > 0) {
     // offsets of every BatchNorm's parameters / statistics / preceding conv bias: launch_bn_eval_coeffs_all (eval
     // workspace) or launch_bn_frozen_coeffs_all (training workspace)
@@ -1081,7 +1086,7 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
                  cudaStream_t st, const TileCall* tc = nullptr) {
   if (!e->ws) { set_error("generator_forward: not bound"); return -23; }
   if (training && !e->ws_training) { set_error("generator_forward: bound workspace is eval-sized"); return -24; }
-  if (training) e->last_frozen = frozen;
+  if (training) { e->last_frozen = frozen; e->tile_n = 0; }
   if (frozen) update_running = 0;
   const Layout& L = e->L;
   const PackOffsets& po = e->po;
@@ -1242,6 +1247,8 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
     e->launches += 1;
     in = ws + L.up[j];
   }
+  // a frozen-tiles forward without an output recomputes the activations for its backward, which does not read SR
+  if (tc && sr == nullptr) return 0;
   // conv3: 9x9, 64->3, no activation (src/models.py:78,86); fp32 NCHW output
   {
     const int Hs = H << e->n_up, Ws = W << e->n_up;
@@ -1272,47 +1279,67 @@ int generator_tile_halo(int n_res, int n_up) {
   return r + (2 * n_res + 1) + 4;      // the trunk's 3x3 convs (2 per block + conv2), conv1's 9x9
 }
 
-int generator_forward_tiles(GeneratorEngine* g, const float* frames, int F, int H, int W, const TileDesc* tiles, int n,
-                            float* sr, cudaStream_t st) {
-  EngineImpl* e = static_cast<EngineImpl*>(g);
-  if (frames == nullptr || tiles == nullptr || sr == nullptr) { set_error("srg_generator_forward_tiles: null pointer"); return -22; }
-  if (F < 1 || H < 1 || W < 1) { set_error("srg_generator_forward_tiles: F, H and W must be >= 1 (got %d, %d, %d)", F, H, W); return -26; }
+namespace {
+// argument checks shared by the eval and the frozen tiled forwards (no CUDA call) and the call's gather / scatter tables
+int make_tile_call(const EngineImpl* e, const char* who, const float* frames, int F, int H, int W, const TileDesc* tiles,
+                   int n, float* sr, bool sr_optional, TileCall* tc) {
+  if (frames == nullptr || tiles == nullptr || (sr == nullptr && !sr_optional)) { set_error("%s: null pointer", who); return -22; }
+  if (F < 1 || H < 1 || W < 1) { set_error("%s: F, H and W must be >= 1 (got %d, %d, %d)", who, F, H, W); return -26; }
   const int n_max = e->N < kMaxTiles ? e->N : kMaxTiles;
-  if (n < 1 || n > n_max) { set_error("srg_generator_forward_tiles: tile count %d outside 1..%d (engine N and SRG_MAX_TILES)", n, n_max); return -27; }
+  if (n < 1 || n > n_max) { set_error("%s: tile count %d outside 1..%d (engine N and SRG_MAX_TILES)", who, n, n_max); return -27; }
   for (int i = 0; i < n; ++i) {
     const TileDesc& t = tiles[i];
-    if (t.frame < 0 || t.frame >= F) { set_error("srg_generator_forward_tiles: tile %d frame index %d outside 0..%d", i, t.frame, F - 1); return -28; }
+    if (t.frame < 0 || t.frame >= F) { set_error("%s: tile %d frame index %d outside 0..%d", who, i, t.frame, F - 1); return -28; }
     if (t.y0 < 0 || t.x0 < 0 || int64_t(t.y0) + e->H > H || int64_t(t.x0) + e->W > W) {
-      set_error("srg_generator_forward_tiles: tile %d window (%d, %d) + %d x %d is not inside the %d x %d frame", i, t.y0, t.x0,
-                e->H, e->W, H, W);
+      set_error("%s: tile %d window (%d, %d) + %d x %d is not inside the %d x %d frame", who, i, t.y0, t.x0, e->H, e->W, H, W);
       return -29;
     }
-    if (t.crop_h < 1 || t.crop_w < 1) { set_error("srg_generator_forward_tiles: tile %d crop is empty", i); return -30; }
+    if (t.crop_h < 1 || t.crop_w < 1) { set_error("%s: tile %d crop is empty", who, i); return -30; }
     if (t.crop_y0 < 0 || t.crop_x0 < 0 || int64_t(t.crop_y0) + t.crop_h > e->H || int64_t(t.crop_x0) + t.crop_w > e->W) {
-      set_error("srg_generator_forward_tiles: tile %d crop is not inside its window", i);
+      set_error("%s: tile %d crop is not inside its window", who, i);
       return -31;
     }
   }
-  if (!e->ws) { set_error("srg_generator_forward_tiles: no workspace bound"); return -23; }
-  if (e->ws_training) { set_error("srg_generator_forward_tiles: needs an eval-sized workspace (this one is bound for training)"); return -24; }
-
   const int s = e->n_up;
   const int64_t plane = int64_t(H) * W, Ws = int64_t(W) << s, plane_o = (int64_t(H) << s) * Ws;
-  TileCall tc;
-  memset(&tc, 0, sizeof(tc));
-  tc.frames = frames;
-  tc.n = n;
-  tc.gather.n = n; tc.gather.plane = plane; tc.gather.pitch = W;
-  tc.scatter.n = n; tc.scatter.plane = plane_o; tc.scatter.pitch = Ws;
+  memset(tc, 0, sizeof(*tc));
+  tc->frames = frames;
+  tc->n = n;
+  tc->gather.n = n; tc->gather.plane = plane; tc->gather.pitch = W;
+  tc->scatter.n = n; tc->scatter.plane = plane_o; tc->scatter.pitch = Ws;
   for (int i = 0; i < n; ++i) {
     const TileDesc& t = tiles[i];
-    tc.gather.base[i] = int64_t(t.frame) * 3 * plane + int64_t(t.y0) * W + t.x0;
-    FoldTile& o = tc.scatter.t[i];
+    tc->gather.base[i] = int64_t(t.frame) * 3 * plane + int64_t(t.y0) * W + t.x0;
+    FoldTile& o = tc->scatter.t[i];
     o.base = int64_t(t.frame) * 3 * plane_o + (int64_t(t.y0) << s) * Ws + (int64_t(t.x0) << s);
     o.h_lo = t.crop_y0 << s; o.h_hi = (t.crop_y0 + t.crop_h) << s;
     o.w_lo = t.crop_x0 << s; o.w_hi = (t.crop_x0 + t.crop_w) << s;
   }
+  return 0;
+}
+}  // namespace
+
+int generator_forward_tiles(GeneratorEngine* g, const float* frames, int F, int H, int W, const TileDesc* tiles, int n,
+                            float* sr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  TileCall tc;
+  RC(make_tile_call(e, "srg_generator_forward_tiles", frames, F, H, W, tiles, n, sr, false, &tc));
+  if (!e->ws) { set_error("srg_generator_forward_tiles: no workspace bound"); return -23; }
+  if (e->ws_training) { set_error("srg_generator_forward_tiles: needs an eval-sized workspace (this one is bound for training)"); return -24; }
   return forward_impl(e, nullptr, sr, 0, 0, kPhaseAll, false, st, &tc);
+}
+
+int generator_forward_frozen_tiles(GeneratorEngine* g, const float* frames, int F, int H, int W, const TileDesc* tiles, int n,
+                                   float* sr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  TileCall tc;
+  RC(make_tile_call(e, "srg_generator_forward_frozen_tiles", frames, F, H, W, tiles, n, sr, true, &tc));
+  if (!e->ws) { set_error("srg_generator_forward_frozen_tiles: no workspace bound"); return -23; }
+  if (!e->ws_training) { set_error("srg_generator_forward_frozen_tiles: needs a training-sized workspace (this one is bound for eval)"); return -24; }
+  RC(forward_impl(e, nullptr, sr, 1, 0, kPhaseAll, true, st, &tc));
+  e->tile_n = n; e->tile_H = H; e->tile_W = W;
+  memcpy(e->tile_tab, tiles, sizeof(TileDesc) * size_t(n));
+  return 0;
 }
 
 int generator_forward_phases(GeneratorEngine* g, const float* lr, float* sr, int training, int update_running, int phases,
@@ -1331,8 +1358,13 @@ int generator_forward_frozen(GeneratorEngine* g, const float* lr, float* sr, cud
 namespace {
 // param_grads == false: only the data-gradient chain runs (no gradient memset, weight gradients, bias sums or BatchNorm
 // parameter gradients; the flat gradient buffer is not touched).  dlr != null: conv1's data gradient, fp32 NCHW.
-int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads, float* dlr, cudaStream_t st) {
+// n_win > 0: the backward of a frozen-tiles forward over its n_win windows (the first n_win items of the workspace)
+int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads, float* dlr, cudaStream_t st, int n_win = 0) {
   if (!e->ws || !e->ws_training) { set_error("generator_backward: needs a training-sized bound workspace"); return -25; }
+  if (e->tile_n > 0 && n_win == 0) {
+    set_error("generator_backward: the last forward was srg_generator_forward_frozen_tiles; its backward is srg_generator_backward_tiles");
+    return -32;
+  }
   const bool frozen = e->last_frozen;
   if (frozen && phases != kPhaseAll) {
     set_error("generator_backward_phases: the last forward used running BatchNorm statistics; split execution needs a training forward");
@@ -1343,7 +1375,7 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
   const PackOffsets& po = e->po;
   uint8_t* ws = e->ws;
   const uint16_t* packed = reinterpret_cast<const uint16_t*>(ws + L.packed);
-  const int N = e->N, H = e->H, W = e->W, S = e->n_up;
+  const int N = n_win > 0 ? n_win : e->N, H = e->H, W = e->W, S = e->n_up;
   const int64_t P = int64_t(N) * H * W;
   const int Hs = H << S, Ws = W << S;
   float* partials = reinterpret_cast<float*>(ws + L.partials);
@@ -1645,6 +1677,46 @@ int generator_backward_ex(GeneratorEngine* g, const float* dsr, int param_grads,
   if (param_grads == 0 && dlr == nullptr) { set_error("generator_backward_ex: nothing to compute (param_grads == 0 and dlr == NULL)"); return -22; }
   if (!e->ws || !e->ws_training) { set_error("generator_backward_ex: needs a training-sized bound workspace"); return -25; }
   return backward_impl(e, dsr, kPhaseAll, param_grads != 0, dlr, st);
+}
+
+// Staging buffers of srg_generator_backward_tiles, in workspace regions that are dead while they are live:
+//  - the window-shaped, crop-masked d(SR) (n x 3 x Hs x Ws fp32, 12 B per HR pixel) sits in dup[S-1] (128 B per HR
+//    pixel), or in g[3] = d(trunk) (one 128 B-per-pixel slot) when S = 0.  backward_impl reads it only in its first two
+//    launches (unfold9 into Ud, the conv3.bias sum); the first write to dup[S-1] / g[3] is conv3's data gradient, which
+//    reads Ud.  debug_keep_grads changes neither buffer (its kd_* buffers are separate; g[3] stays the conv2 slot).
+//  - conv1's window-shaped data gradient (n x 3 x H x W fp32) goes to Ud (128 B per HR pixel), which only conv3's
+//    bias sum, weight gradient and data gradient read, all of them enqueued before conv1's data gradient.
+int generator_backward_tiles(GeneratorEngine* g, const float* dsr, int param_grads, float* dlr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  if (dsr == nullptr) { set_error("srg_generator_backward_tiles: null d(sr)"); return -22; }
+  if (param_grads == 0 && dlr == nullptr) { set_error("srg_generator_backward_tiles: nothing to compute (param_grads == 0 and dlr == NULL)"); return -22; }
+  if (!e->ws || !e->ws_training) { set_error("srg_generator_backward_tiles: needs a training-sized bound workspace"); return -25; }
+  if (e->tile_n < 1) { set_error("srg_generator_backward_tiles: no preceding srg_generator_forward_frozen_tiles"); return -32; }
+  const int S = e->n_up, n = e->tile_n;
+  WindowTable hr, lr;
+  memset(&hr, 0, sizeof(hr));
+  hr.n = n; hr.fh = e->tile_H << S; hr.fw = e->tile_W << S;
+  for (int i = 0; i < n; ++i) {
+    const TileDesc& t = e->tile_tab[i];
+    hr.frame[i] = t.frame; hr.y0[i] = t.y0 << S; hr.x0[i] = t.x0 << S;
+    hr.h_lo[i] = t.crop_y0 << S; hr.h_hi[i] = (t.crop_y0 + t.crop_h) << S;
+    hr.w_lo[i] = t.crop_x0 << S; hr.w_hi[i] = (t.crop_x0 + t.crop_w) << S;
+  }
+  lr = hr;
+  lr.fh = e->tile_H; lr.fw = e->tile_W;
+  for (int i = 0; i < n; ++i) {
+    const TileDesc& t = e->tile_tab[i];
+    lr.y0[i] = t.y0; lr.x0[i] = t.x0;
+    lr.h_lo[i] = t.crop_y0; lr.h_hi[i] = t.crop_y0 + t.crop_h; lr.w_lo[i] = t.crop_x0; lr.w_hi[i] = t.crop_x0 + t.crop_w;
+  }
+  float* dsr_win = reinterpret_cast<float*>(e->ws + (S > 0 ? e->L.dup[S - 1] : e->L.g[3]));
+  float* dlr_win = reinterpret_cast<float*>(e->ws + e->L.Ud);
+  RC(launch_crop_masked_gather(dsr, hr, e->H << S, e->W << S, dsr_win, st));
+  e->launches += 1;
+  RC(backward_impl(e, dsr_win, kPhaseAll, param_grads != 0, dlr ? dlr_win : nullptr, st, n));
+  if (dlr == nullptr) return 0;
+  e->launches += 1;
+  return launch_window_scatter_add(dlr_win, lr, e->H, e->W, dlr, st);
 }
 
 }  // namespace srg

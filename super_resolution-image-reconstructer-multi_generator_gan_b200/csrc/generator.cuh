@@ -98,6 +98,11 @@ struct TileDesc { int32_t frame, y0, x0, crop_y0, crop_x0, crop_h, crop_w; };
 int generator_tile_halo(int n_res, int n_up);
 int generator_forward_tiles(GeneratorEngine* g, const float* frames_nchw, int F, int H, int W, const TileDesc* tiles, int n,
                             float* sr_nchw, cudaStream_t st);
+// eval-mode autograd over windows (srg_generator_forward_frozen_tiles / srg_generator_backward_tiles): the frozen forward of
+// n windows on a training workspace (sr_nchw may be NULL: activations only), then the backward of those windows
+int generator_forward_frozen_tiles(GeneratorEngine* g, const float* frames_nchw, int F, int H, int W, const TileDesc* tiles,
+                                   int n, float* sr_nchw, cudaStream_t st);
+int generator_backward_tiles(GeneratorEngine* g, const float* dsr_nchw, int param_grads, float* dlr_nchw, cudaStream_t st);
 // Split execution for the multi-generator step: PRE = everything before the residual trunk, TRUNK = the trunk itself,
 // POST = everything after it (forward: conv1 | blocks + conv2 | upsample + conv3; backward: conv3 + upsample stages |
 // trunk dgrad chain | conv1 gradients + the batched trunk weight gradients).  The TRUNK phases of several engines of equal

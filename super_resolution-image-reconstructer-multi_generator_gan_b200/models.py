@@ -255,6 +255,66 @@ class _GeneratorFn(torch.autograd.Function):
         return (None, None, dlr) + grads
 
 
+class _FrozenTilesFn(torch.autograd.Function):
+    """autograd node of an eval-mode forward under ``SRResNet.grad_budget_bytes``: the frozen forward of every window
+    (``srg_generator_forward_frozen_tiles``), call by call through one engine of ``n`` windows.  The engine keeps only the
+    last call's activations, so the backward recomputes each call's windows before running their backward
+    (``srg_generator_backward_tiles``).  Each backward recomputes its own windows, so the engine is not reserved between
+    forward and backward and any number of such graphs can be alive at once."""
+
+    @staticmethod
+    def forward(ctx, module, plan, x, *params):
+        win_h, win_w, n, tiles = plan
+        s = module.num_upsample_stages
+        eng = module._frozen_tiles_engine(n, win_h, win_w, x.device)
+        sr = torch.empty(x.shape[0], 3, x.shape[2] << s, x.shape[3] << s, dtype=torch.float32, device=x.device)
+        for i in range(0, len(tiles), n):
+            tiling.forward_frozen_tiles(eng.handle, x, tiles[i:i + n], sr, stream_ptr())
+        ctx.save_for_backward(x)
+        ctx.module_ref = weakref.ref(module)
+        ctx.plan = plan
+        ctx.versions = module._state_versions()
+        ctx.n_params = len(params)
+        ctx.set_materialize_grads(False)
+        return sr
+
+    @staticmethod
+    def backward(ctx, dsr):
+        module = ctx.module_ref()
+        if dsr is None or module is None:
+            return (None,) * (3 + ctx.n_params)
+        (x,) = ctx.saved_tensors
+        if module._state_versions() != ctx.versions:
+            raise RuntimeError("SRResNet: a parameter or BatchNorm buffer was modified in place between the forward and the "
+                               "backward of an eval-mode forward under grad_budget_bytes (its backward recomputes the "
+                               "forward from the current values)")
+        dsr = dsr.contiguous()
+        if dsr.dtype != torch.float32:
+            dsr = dsr.float()
+        want_dx = ctx.needs_input_grad[2]
+        want_pg = any(ctx.needs_input_grad[3:])
+        win_h, win_w, n, tiles = ctx.plan
+        eng = module._frozen_tiles_engine(n, win_h, win_w, x.device)       # re-packs the weights
+        dlr = torch.zeros(x.shape, dtype=torch.float32, device=x.device) if want_dx else None
+        total = module._grad_buffer_for_backward(eng) if want_pg else None
+        part = torch.empty_like(total) if want_pg and len(tiles) > n else None
+        L = _lib.lib()
+        for k, i in enumerate(range(0, len(tiles), n)):
+            tiling.forward_frozen_tiles(eng.handle, x, tiles[i:i + n], None, stream_ptr())
+            if want_pg:
+                # the first call writes the running total, later ones a second buffer that is added to it
+                check(L.srg_generator_set_grads(eng.handle, c_void_p((total if k == 0 else part).data_ptr())))
+            tiling.backward_tiles(eng.handle, dsr, want_pg, dlr, stream_ptr())
+            if want_pg and k > 0:
+                total.add_(part)
+        if not want_pg:
+            # input gradient only: the flat gradient buffer, the gradient hook and .grad are left alone
+            return (None, None, dlr) + (None,) * ctx.n_params
+        module._after_backward(total)
+        grads = tuple(total[off:off + m].view(shape) for (_, off, m, shape) in module._ptable)
+        return (None, None, dlr) + grads
+
+
 class SRResNet(_FlatModule):
     """Drop-in for the reference's SRResNet (src/models.py:44-87).
 
@@ -385,6 +445,55 @@ class SRResNet(_FlatModule):
         per_frame = max(self._eval_ws_bytes(H, W, device), 1)
         return max(1, min(N, int(budget // per_frame)))
 
+    #: eval-mode autograd workspace budget in bytes: an eval forward whose input requires grad, and whose whole-batch
+    #: frozen (training-layout) workspace is larger, runs in halo-padded windows (``tiling.plan_tiles``; a frame that fits
+    #: is one window) through one engine of at most this much workspace, and its backward recomputes the windows' forward
+    #: (None: the whole batch in one engine call)
+    grad_budget_bytes: Optional[int] = None
+
+    def _train_ws_bytes(self, N: int, H: int, W: int, device) -> int:
+        """training (frozen) workspace of an N x H x W engine, as ``_engine`` would create it (a host-only probe)"""
+        rt = self._rt
+        keep = bool(getattr(self, "debug_keep_grads", False))
+        key = ("ws_train", N, H, W, keep)
+        if key not in rt:
+            probe = _GeneratorEngine(N, H, W, self.num_residuals, self.num_upsample_stages, True, device)
+            if keep:
+                check(_lib.lib().srg_generator_set_keep_grads(probe.handle, 1))
+            rt[key] = int(_lib.lib().srg_generator_workspace_bytes(probe.handle, 1))
+            del probe
+        return rt[key]
+
+    def _state_versions(self) -> Tuple[int, ...]:
+        return tuple(p._version for p in self._rt["plist"]) + tuple(b._version for b in self.buffers())
+
+    def _frozen_tiles_engine(self, n: int, H: int, W: int, device) -> _GeneratorEngine:
+        """a frozen engine of n windows of H x W, bound and with freshly packed weights"""
+        rt = self._rt
+        eng = self._engine(n, H, W, False, device, False, frozen=True)
+        if getattr(eng, "grad_flat", None) is None:
+            eng.grad_flat = torch.empty_like(rt["flat"])
+        eng.bind(rt["flat"], eng.grad_flat, rt["flat_buf"])
+        check(_lib.lib().srg_generator_pack(eng.handle, stream_ptr()), "srg_generator_pack")
+        rt["last_engine"] = eng
+        return eng
+
+    def _frozen_tiles_plan(self, N: int, H: int, W: int, device) -> Tuple[int, int, int, list]:
+        """(window_h, window_w, windows per call, windows) for ``grad_budget_bytes``: the planner's windows, and as many
+        per call as an engine of that many windows fits the budget"""
+        rt = self._rt
+        budget = int(self.grad_budget_bytes)
+        key = ("frozen_tiles", N, H, W, budget, bool(getattr(self, "debug_keep_grads", False)))
+        if key not in rt:
+            halo = tiling.tile_halo(self.num_residuals, self.num_upsample_stages)
+            win_h, win_w, per_call, tiles = tiling.plan_tiles(N, H, W, halo,
+                                                              lambda h, w: self._train_ws_bytes(1, h, w, device), budget)
+            n = min(per_call, len(tiles))
+            while n > 1 and self._train_ws_bytes(n, win_h, win_w, device) > budget:
+                n -= 1
+            rt[key] = (win_h, win_w, n, tiles)
+        return rt[key]
+
     def _forward_tiled(self, x: torch.Tensor) -> torch.Tensor:
         """eval-mode forward of frames too large for ``tile_budget_bytes``: the windows of all frames in order, as many per
         ``srg_generator_forward_tiles`` call as the plan's ``tiles_per_call`` (usually 1: the planner picks the largest
@@ -432,6 +541,13 @@ class SRResNet(_FlatModule):
                                                                       ("frozen"), whole batch in one engine call:
                                                                       ``x.grad`` plus the gradients of the parameters
                                                                       that require grad
+        eval   on        yes                any                       with ``grad_budget_bytes`` set and a whole-batch
+                                                                      frozen workspace above it: the same gradients,
+                                                                      summed over halo-padded windows (a frame that
+                                                                      fits is one window) run through one engine within
+                                                                      the budget; the backward recomputes each call's
+                                                                      windows; equal to the whole-batch path up to
+                                                                      fp32 summation order and bf16 rounding
         ====== ========= ================== ========================= =================================================
 
         The frozen output equals the detached eval output up to bf16 rounding (DESIGN §4).  Double backward is not
@@ -450,6 +566,9 @@ class SRResNet(_FlatModule):
         need_grad = self.training and torch.is_grad_enabled()
         # eval mode with an input that requires grad (a fixed generator inside a larger differentiable pipeline)
         frozen = not self.training and torch.is_grad_enabled() and x.requires_grad
+        if (frozen and self.grad_budget_bytes is not None
+                and self._train_ws_bytes(N, H, W, x.device) > self.grad_budget_bytes):
+            return _FrozenTilesFn.apply(self, self._frozen_tiles_plan(N, H, W, x.device), x, *rt["plist"])
         if (not self.training and not frozen and self.tile_budget_bytes is not None
                 and self._eval_ws_bytes(H, W, x.device) > self.tile_budget_bytes):
             return self._forward_tiled(x)

@@ -183,3 +183,22 @@ def forward_tiles(handle, frames, tiles: List[Tile], out, stream) -> None:
     _lib.check(_lib.lib().srg_generator_forward_tiles(handle, ctypes.c_void_p(frames.data_ptr()), F, H, W, arr, len(tiles),
                                                       ctypes.c_void_p(out.data_ptr()), stream),
                "srg_generator_forward_tiles")
+
+
+def forward_frozen_tiles(handle, frames, tiles: List[Tile], out, stream) -> None:
+    """One ``srg_generator_forward_frozen_tiles`` call: as ``forward_tiles`` on an engine bound to a training workspace,
+    keeping the activations for ``backward_tiles``.  ``out`` may be None (a recompute for the backward: no output)."""
+    arr = (SrgTile * len(tiles))(*[SrgTile(*t) for t in tiles])
+    F, _, H, W = frames.shape
+    _lib.check(_lib.lib().srg_generator_forward_frozen_tiles(
+        handle, ctypes.c_void_p(frames.data_ptr()), F, H, W, arr, len(tiles),
+        ctypes.c_void_p(out.data_ptr()) if out is not None else None, stream), "srg_generator_forward_frozen_tiles")
+
+
+def backward_tiles(handle, dsr, param_grads: bool, dlr, stream) -> None:
+    """One ``srg_generator_backward_tiles`` call for the windows of the last ``forward_frozen_tiles``: the bound flat
+    gradient buffer receives their parameter gradients (``param_grads``), ``dlr`` (None: not computed) their input
+    gradients, added in window order."""
+    _lib.check(_lib.lib().srg_generator_backward_tiles(
+        handle, ctypes.c_void_p(dsr.data_ptr()), 1 if param_grads else 0,
+        ctypes.c_void_p(dlr.data_ptr()) if dlr is not None else None, stream), "srg_generator_backward_tiles")
