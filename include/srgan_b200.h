@@ -98,6 +98,17 @@ typedef struct {
 int srg_generator_tile_halo(int num_residuals, int num_upsample_stages);
 int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W, const srg_tile_t* tiles,
                                 int n, float* sr_nchw, void* stream);
+/* 8-bit frame I/O of the eval forward, for frames as decoders produce them: uint8 RGB, channel-last.  Input byte v is read
+ * as __fdiv_rn(v, 255) (ToTensor's fp32 division), output value y is stored as rint(255 * clamp(y, 0, 1)) (fp32 multiply,
+ * round half to even; NaN stores 0), so the result equals (sr.clamp(0, 1) * 255).round().to(uint8) of the fp32 forward of
+ * ToTensor(frames), bit for bit, with no fp32 copy of the input and no fp32 SR tensor.  The workspace is unchanged.
+ * srg_generator_forward_u8: the eval forward (training = 0, no running-statistics update) of the engine's N frames,
+ * lr_nhwc N x H x W x 3 -> sr_nhwc N x (H << n_up) x (W << n_up) x 3.
+ * srg_generator_forward_tiles_u8: srg_generator_forward_tiles on F x H x W x 3 frames into F x (H << n_up) x (W << n_up)
+ * x 3, with the same windows, checks and graph-capture guarantee.  Both check every argument before any CUDA call. */
+int srg_generator_forward_u8(srg_generator_t* g, const uint8_t* lr_nhwc, uint8_t* sr_nhwc, void* stream);
+int srg_generator_forward_tiles_u8(srg_generator_t* g, const uint8_t* frames_nhwc, int F, int H, int W,
+                                   const srg_tile_t* tiles, int n, uint8_t* sr_nhwc, void* stream);
 /* Eval-mode autograd over windows, for frames whose whole-frame frozen workspace is too large.  With running BatchNorm
  * statistics every layer is local, so for windows whose crops partition the frames (crop edges at least
  * srg_generator_tile_halo() inside the window, as for srg_generator_forward_tiles) the whole-frame gradients are sums of

@@ -94,6 +94,9 @@ EXPORTS = {
     "srg_generator_forward_frozen_tiles": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p,
                                                    c_void_p]),
     "srg_generator_backward_tiles": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "srg_generator_forward_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    "srg_generator_forward_tiles_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p,
+                                               c_void_p]),
     "srg_generator_num_tensors": (c_int, [c_void_p]),
     "srg_generator_tensor_info": (c_int, [c_void_p, c_int, c_char_p, c_int, POINTER(c_int64), POINTER(c_int),
                                           POINTER(c_int)]),

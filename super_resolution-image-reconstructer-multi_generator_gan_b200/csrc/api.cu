@@ -143,6 +143,16 @@ int srg_generator_forward_tiles(srg_generator_t* g, const float* frames_nchw, in
   if (g == nullptr) { set_error("srg_generator_forward_tiles: null engine"); return -1; }
   return generator_forward_tiles(G(g), frames_nchw, F, H, W, reinterpret_cast<const TileDesc*>(tiles), n, sr_nchw, S(stream));
 }
+int srg_generator_forward_u8(srg_generator_t* g, const uint8_t* lr_nhwc, uint8_t* sr_nhwc, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_forward_u8: null engine"); return -1; }
+  return generator_forward_u8(G(g), lr_nhwc, sr_nhwc, S(stream));
+}
+int srg_generator_forward_tiles_u8(srg_generator_t* g, const uint8_t* frames_nhwc, int F, int H, int W,
+                                   const srg_tile_t* tiles, int n, uint8_t* sr_nhwc, void* stream) {
+  if (g == nullptr) { set_error("srg_generator_forward_tiles_u8: null engine"); return -1; }
+  return generator_forward_tiles_u8(G(g), frames_nhwc, F, H, W, reinterpret_cast<const TileDesc*>(tiles), n, sr_nhwc,
+                                    S(stream));
+}
 int srg_generator_forward_frozen_tiles(srg_generator_t* g, const float* frames_nchw, int F, int H, int W,
                                        const srg_tile_t* tiles, int n, float* sr_nchw, void* stream) {
   if (g == nullptr) { set_error("srg_generator_forward_frozen_tiles: null engine"); return -1; }

@@ -63,14 +63,14 @@ struct ConvKParams {
   int act;
   float slope;
   int aux_mode;  // 0 none, 1 add (residual), 2 mask (zero where aux <= 0)
-  void* out;     // fold9 only (fp32 NCHW)
+  void* out;     // fold9 only (through the FoldScatter of ConvKParamsFold)
   int out_mode;
   float* stats;  // per-CTA channel sums / sums of squares (BatchNorm statistics fused into the epilogue)
   const uint32_t* stats_y;  // optional second factor (bf16 pairs) for the product sums
   long long* prof;  // optional per-CTA role timers (debug)
 };
 
-// the fold9 instance also carries the cropped-scatter table (the other instances keep their parameter size)
+// the fold9 instance also carries its store table (the other instances keep their parameter size)
 struct ConvKParamsFold : ConvKParams {
   FoldScatter scatter;
 };
@@ -87,6 +87,37 @@ __device__ __forceinline__ float apply_act(float x, float slope) {
   if (ACT == ACT_RELU) return fmaxf(x, 0.f);
   if (ACT == ACT_LRELU) return x > 0.f ? x : x * slope;
   return x;
+}
+
+// one output pixel of a fold9 epilogue through its FoldScatter.  The 8-bit store is torch's
+// (sr.clamp(0, 1) * 255).round().to(uint8): fp32 multiply, round half to even; NaN stores 0 (fmaxf returns 0)
+__device__ __forceinline__ uint8_t quantise_u8(float y) {
+  return uint8_t(rintf(__fmul_rn(fminf(fmaxf(y, 0.f), 1.f), 255.f)));
+}
+__device__ __forceinline__ void fold9_store(const FoldScatter& s, void* out, int n, int h, int w, float o0, float o1,
+                                            float o2) {
+  const int64_t base = (s.n == 0 ? int64_t(n) * s.item : s.t[n].base) + int64_t(h) * s.pitch + int64_t(w) * s.px;
+  if (s.u8) {
+    uint8_t* o = reinterpret_cast<uint8_t*>(out) + base;
+    o[0] = quantise_u8(o0);
+    o[s.plane] = quantise_u8(o1);
+    o[2 * s.plane] = quantise_u8(o2);
+  } else {
+    float* o = reinterpret_cast<float*>(out) + base;
+    o[0] = o0;
+    o[s.plane] = o1;
+    o[2 * s.plane] = o2;
+  }
+}
+// the plain fp32 NCHW store of an H x W launch that brings no FoldScatter
+static FoldScatter fold9_nchw(int H, int W) {
+  FoldScatter s;
+  memset(&s, 0, sizeof(s));
+  s.plane = int64_t(H) * W;
+  s.item = 3 * s.plane;
+  s.pitch = W;
+  s.px = 1;
+  return s;
 }
 
 template <int BLOCK_N, int NT>
@@ -323,18 +354,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
             o1 += row[1];
             o2 += row[2];
           }
-          float* o = reinterpret_cast<float*>(p.out);
-          size_t plane, base;
-          if (p.scatter.n == 0) {
-            plane = size_t(p.H) * p.W;
-            base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
-          } else {
-            plane = size_t(p.scatter.plane);
-            base = size_t(p.scatter.t[n].base + int64_t(h) * p.scatter.pitch + w);
-          }
-          o[base] = o0;
-          o[base + plane] = o1;
-          o[base + 2 * plane] = o2;
+          fold9_store(p.scatter, p.out, n, h, w, o0, o1, o2);
         }
         named_bar_sync(2, 128);
       } else {
@@ -1050,9 +1070,9 @@ struct C9KParams {
   int tiles_h, tiles_w, tiles_total, n_ctas;
   int n_stages;
   const float* bias;         // [3] or null
-  float* out;                // fp32 [N,3,H,W], or full frames through `scatter`
+  void* out;                 // through `scatter`
   long long* prof;
-  FoldScatter scatter;       // n == 0: plain store
+  FoldScatter scatter;
 };
 
 constexpr int kC9Threads = 64 + 256;            // warp 0 producer, warp 1 MMA, warps 2-5 / 6-9 epilogue groups
@@ -1176,7 +1196,6 @@ __global__ void __launch_bounds__(kC9Threads, 1) conv9_rows_kernel(const __grid_
     const int m = q * 32 + lane;               // pixel within the 128-wide tile
     float* fb = fold_buf + grp * 128 * kFoldPad;
     const float b0 = p.bias ? p.bias[0] : 0.f, b1 = p.bias ? p.bias[1] : 0.f, b2 = p.bias ? p.bias[2] : 0.f;
-    const size_t plane = size_t(p.H) * p.W;
     int acc = 0;
     uint32_t acc_phase = 0;
     for (int tile = blockIdx.x; tile < p.tiles_total; tile += p.n_ctas) {
@@ -1212,18 +1231,7 @@ __global__ void __launch_bounds__(kC9Threads, 1) conv9_rows_kernel(const __grid_
             o1 += row[1];
             o2 += row[2];
           }
-          if (p.scatter.n == 0) {
-            const size_t base = (size_t(n) * 3) * plane + size_t(h) * p.W + w;
-            p.out[base] = o0;
-            p.out[base + plane] = o1;
-            p.out[base + 2 * plane] = o2;
-          } else {
-            const size_t pl = size_t(p.scatter.plane);
-            const size_t base = size_t(p.scatter.t[n].base + int64_t(h) * p.scatter.pitch + w);
-            p.out[base] = o0;
-            p.out[base + pl] = o1;
-            p.out[base + 2 * pl] = o2;
-          }
+          fold9_store(p.scatter, p.out, n, h, w, o0, o1, o2);
         }
         named_bar_sync(2 + 2 * grp, 128);
       }
@@ -1570,9 +1578,9 @@ static int launch_conv9_rows(const ConvGemmArgs& a, cudaStream_t stream) {
     if (rc) return rc;
   }
   p.bias = a.bias;
-  p.out = reinterpret_cast<float*>(a.out);
+  p.out = a.out;
   p.prof = reinterpret_cast<long long*>(a.prof);
-  if (a.scatter != nullptr) p.scatter = *a.scatter;
+  p.scatter = a.scatter != nullptr ? *a.scatter : fold9_nchw(a.H, a.W);
   static DeviceOnce attr_set;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(conv9_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -1617,8 +1625,9 @@ int launch_conv_gemm_grouped(const ConvGemmArgs* as, int n, cudaStream_t stream)
 }
 
 int launch_conv_gemm(const ConvGemmArgs& a, cudaStream_t stream) {
-  if (a.scatter != nullptr && (a.out_mode != OUT_FOLD9_NCHW || a.scatter->n > kMaxTiles || a.scatter->n != a.N)) {
-    set_error("conv_gemm: a cropped scatter needs the fold9 output and one entry per item (at most %d)", kMaxTiles);
+  if (a.scatter != nullptr && (a.out_mode != OUT_FOLD9_NCHW || a.scatter->n > kMaxTiles ||
+                              (a.scatter->n != 0 && a.scatter->n != a.N))) {
+    set_error("conv_gemm: a fold9 store table needs the fold9 output and none or one entry per item (at most %d)", kMaxTiles);
     return -20;
   }
   if (use_conv3_il(a)) return launch_conv3_il(&a, 1, stream);
@@ -1750,7 +1759,7 @@ int launch_conv_gemm(const ConvGemmArgs& a, cudaStream_t stream) {
     ConvKParamsFold pf;
     memset(&pf, 0, sizeof(pf));
     static_cast<ConvKParams&>(pf) = p;
-    if (a.scatter != nullptr) pf.scatter = *a.scatter;
+    pf.scatter = a.scatter != nullptr ? *a.scatter : fold9_nchw(a.H, a.W);
     return launch_instance<32, 9>(pf, grid, smem_bytes, stream);
   }
   switch (a.n_taps) {

@@ -20,17 +20,21 @@ enum ConvOutMode : int {
   OUT_NHWC_F32 = 3,      // fp32 [N,H,W,cout_total] (direct 128-bit stores; discriminator conv outputs)
 };
 
-// Cropped scatter of a fold9 (OUT_FOLD9_NCHW) launch over n <= kMaxTiles windows (srg_generator_forward_tiles): output
-// pixel (h, w) of item i is written only when h_lo <= h < h_hi and w_lo <= w < w_hi, to element base + h * pitch + w of
-// channel 0 (+ plane per channel) of the caller's full-size frames.  Passed by value in the kernel parameters.
+// Store of a fold9 (OUT_FOLD9_NCHW) launch: channel c of output pixel (h, w) of item i goes to element
+// base_i + c * plane + h * pitch + w * px of `out`, with base_i = i * item (n == 0: whole frames) or t[i].base (a cropped
+// scatter over n <= kMaxTiles windows, srg_generator_forward_tiles, which writes only h_lo <= h < h_hi, w_lo <= w < w_hi).
+// fp32 NCHW: (plane, pitch, px) = (H x W, W, 1); uint8 NHWC (u8 = 1, quantised, srg_generator_forward_u8): (1, 3W, 3), in
+// the units of the full frames.  A launch without one stores fp32 NCHW of its own geometry.  Passed by value in the
+// kernel parameters; offsets are 64-bit.
 constexpr int kMaxTiles = 64;
 struct FoldTile {
   int64_t base;            // element offset of the window origin in channel 0 of its frame
   int h_lo, h_hi, w_lo, w_hi;
 };
 struct FoldScatter {
-  int n;                   // 0: plain NCHW store of the [N,3,H,W] output
-  int64_t plane, pitch;    // elements per output channel plane / row of the full frame
+  int n;                   // 0: whole-frame store of the launch's N items
+  int u8;                  // 1: uint8, y -> rint(255 * clamp(y, 0, 1)) (NaN -> 0); 0: fp32
+  int64_t item, plane, pitch, px;  // element strides: item (n == 0), channel, row, pixel
   FoldTile t[kMaxTiles];
 };
 
@@ -82,7 +86,7 @@ struct ConvGemmArgs {
   const void* stats_y;       // optional with `stats`: bf16 tensor of the output's geometry; the second 64 columns then hold
                              // sum(out * stats_y) instead of sum(out^2) (BatchNorm backward: sum dz, sum dz*y)
   void* prof;                // optional debug timers: int64 [grid][3][6]
-  const FoldScatter* scatter;  // optional (OUT_FOLD9_NCHW only, host memory): cropped scatter into full frames at `out`
+  const FoldScatter* scatter;  // optional (OUT_FOLD9_NCHW only, host memory): the store layout (default fp32 NCHW)
   // fold9: tile columns overlap; valid output columns per tile = TW-8
 };
 

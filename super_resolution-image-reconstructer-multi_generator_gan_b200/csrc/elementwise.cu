@@ -903,8 +903,9 @@ int launch_ps_bias_grad(const void* g, int N, int H2, int W2, float* scratch, fl
 // ------------------------------------------------------------------------------------------------
 // unfold9: one thread per (pixel of the H+1 row grid, channel group of 8)
 // ------------------------------------------------------------------------------------------------
-// Where row hh (0 <= hh < H) of channel c of item n starts: a dense [N,3,H,W] batch, or a window of a larger frame
-// (launch_unfold9_windows).  Both kernels below read their source through one of these.
+// Where row hh (0 <= hh < H) of channel c of item n starts (row) and the value of its column ww (at): a dense [N,3,H,W]
+// fp32 batch or a window of larger fp32 frames (launch_unfold9_windows), or the same two forms of 8-bit NHWC frames
+// (launch_unfold9_u8 / launch_unfold9_windows_u8).  Both kernels below read their source through one of these.
 struct PlainRows {
   const float* src;
   int64_t plane;
@@ -912,6 +913,7 @@ struct PlainRows {
   __device__ __forceinline__ const float* row(int n, int c, int hh) const {
     return src + (int64_t(n) * 3 + c) * plane + int64_t(hh) * W;
   }
+  __device__ __forceinline__ float at(const float* r, int ww) const { return __ldg(r + ww); }
 };
 struct WindowRows {
   const float* src;
@@ -919,6 +921,26 @@ struct WindowRows {
   __device__ __forceinline__ const float* row(int n, int c, int hh) const {
     return src + g.base[n] + c * g.plane + int64_t(hh) * g.pitch;
   }
+  __device__ __forceinline__ float at(const float* r, int ww) const { return __ldg(r + ww); }
+};
+// 8-bit pixels are 3 bytes (no alignment); a byte v becomes v / 255 with the same fp32 division as ToTensor
+// (resample.cu), so conv1's bf16 operand, and every later bit, equals the fp32 path's for to_tensor(frames)
+__device__ __forceinline__ float u8_to_unit(const uint8_t* p) { return __fdiv_rn(float(__ldg(p)), 255.f); }
+struct PlainRowsU8 {
+  const uint8_t* src;       // [N][H][W][3]
+  int H, W;
+  __device__ __forceinline__ const uint8_t* row(int n, int c, int hh) const {
+    return src + ((int64_t(n) * H + hh) * W) * 3 + c;
+  }
+  __device__ __forceinline__ float at(const uint8_t* r, int ww) const { return u8_to_unit(r + 3 * ww); }
+};
+struct WindowRowsU8 {
+  const uint8_t* src;
+  WindowGather g;           // byte offsets: plane = 1 (channel stride), pitch = 3 x frame width
+  __device__ __forceinline__ const uint8_t* row(int n, int c, int hh) const {
+    return src + g.base[n] + c * g.plane + int64_t(hh) * g.pitch;
+  }
+  __device__ __forceinline__ float at(const uint8_t* r, int ww) const { return u8_to_unit(r + 3 * ww); }
 };
 
 template <class Rows>
@@ -940,11 +962,11 @@ __global__ void __launch_bounds__(256) unfold9_kernel(const __grid_constant__ Ro
       const bool row_ok = hh >= 0 && hh < H;
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        const float* row = rows.row(n, c, row_ok ? hh : 0);
+        const auto* row = rows.row(n, c, row_ok ? hh : 0);
 #pragma unroll
         for (int sft = 0; sft < 9; ++sft) {
           const int ww = w + sft - 4;
-          f[dr * 27 + sft * 3 + c] = (row_ok && ww >= 0 && ww < W) ? __ldg(row + ww) * scale : 0.f;
+          f[dr * 27 + sft * 3 + c] = (row_ok && ww >= 0 && ww < W) ? rows.at(row, ww) * scale : 0.f;
         }
       }
     }
@@ -980,7 +1002,7 @@ __global__ void __launch_bounds__(128) unfold9_tile_kernel(const __grid_constant
       const int r = i / 136, x = i - r * 136;
       const int dr = r / 3, c = r - dr * 3;
       const int hh = hp - 1 + dr, ww = w0 + x - 4;
-      tile[r][x] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? __ldg(rows.row(n, c, hh) + ww) * scale : 0.f;
+      tile[r][x] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? rows.at(rows.row(n, c, hh), ww) * scale : 0.f;
     }
     __syncthreads();
 #pragma unroll
@@ -1026,6 +1048,17 @@ int launch_unfold9(const float* src, int N, int H, int W, float scale, void* dst
 int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st) {
   if (wg.n < 1 || wg.n > kMaxWindows) { set_error("unfold9_windows: 1..%d windows", kMaxWindows); return -1; }
   WindowRows rows;
+  rows.src = frames;
+  rows.g = wg;
+  return launch_unfold9_rows(rows, wg.n, H, W, 1.f, dst, st);
+}
+int launch_unfold9_u8(const uint8_t* src, int N, int H, int W, void* dst, cudaStream_t st) {
+  const PlainRowsU8 rows{src, H, W};
+  return launch_unfold9_rows(rows, N, H, W, 1.f, dst, st);
+}
+int launch_unfold9_windows_u8(const uint8_t* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st) {
+  if (wg.n < 1 || wg.n > kMaxWindows) { set_error("unfold9_windows_u8: 1..%d windows", kMaxWindows); return -1; }
+  WindowRowsU8 rows;
   rows.src = frames;
   rows.g = wg;
   return launch_unfold9_rows(rows, wg.n, H, W, 1.f, dst, st);

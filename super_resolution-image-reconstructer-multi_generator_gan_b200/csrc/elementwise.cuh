@@ -107,6 +107,11 @@ struct WindowGather {
   int64_t base[kMaxWindows];
 };
 int launch_unfold9_windows(const float* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st);
+// 8-bit forms (srg_generator_forward_u8 / _tiles_u8): the same operand from uint8 NHWC frames, each byte v read as
+// __fdiv_rn(v, 255) like ToTensor.  Dense: src [N][H][W][3].  Windows: base / plane / pitch of `wg` in bytes (plane = 1,
+// pitch = 3 x frame width); any width, pixels need no alignment.
+int launch_unfold9_u8(const uint8_t* src, int N, int H, int W, void* dst, cudaStream_t st);
+int launch_unfold9_windows_u8(const uint8_t* frames, const WindowGather& wg, int H, int W, void* dst, cudaStream_t st);
 // Windows of F x 3 x fh x fw fp32 frames for the backward of the frozen-tiles forward (srg_generator_backward_tiles), in
 // the pixel units of the grid they index (HR for d(SR), LR for d(lr)).  Item i is the window of frame[i] at (y0[i], x0[i]);
 // its crop is rows [h_lo, h_hi) x columns [w_lo, w_hi), window-relative.  Passed by value in the kernel parameters.

@@ -1071,10 +1071,12 @@ int generator_forward(GeneratorEngine* g, const float* lr, float* sr, int traini
 
 namespace {
 // srg_generator_forward_tiles: n windows of larger frames in one eval pass (conv1's operand gathered from the frames,
-// conv3's output scattered into them, cropped)
+// conv3's output scattered into them, cropped).  u8: the frames, in and out, are uint8 NHWC (srg_generator_forward_u8,
+// whose dense batch of the engine's N frames has gather.n == 0 and scatter.n == 0, and _tiles_u8)
 static_assert(kMaxWindows == kMaxTiles, "gather and scatter tables hold the same windows");
 struct TileCall {
-  const float* frames;
+  const void* frames;
+  bool u8;
   int n;
   WindowGather gather;
   FoldScatter scatter;
@@ -1082,7 +1084,7 @@ struct TileCall {
 
 // frozen: eval-mode BatchNorm (running statistics, never updated or exchanged) on the training workspace, every
 // activation the backward reads kept; per-layer trunk launches only
-int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int update_running, int phases, bool frozen,
+int forward_impl(EngineImpl* e, const float* lr, void* sr, int training, int update_running, int phases, bool frozen,
                  cudaStream_t st, const TileCall* tc = nullptr) {
   if (!e->ws) { set_error("generator_forward: not bound"); return -23; }
   if (training && !e->ws_training) { set_error("generator_forward: bound workspace is eval-sized"); return -24; }
@@ -1116,7 +1118,9 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
   }
   // conv1: 9x9, 3->64, LeakyReLU(0.2)  (src/models.py:56-57,81)
   if (phases & kPhasePre) {
-  if (tc) RC(launch_unfold9_windows(tc->frames, tc->gather, H, W, ws + L.U1, st));
+  if (tc && tc->u8 && tc->gather.n == 0) RC(launch_unfold9_u8(static_cast<const uint8_t*>(tc->frames), N, H, W, ws + L.U1, st));
+  else if (tc && tc->u8) RC(launch_unfold9_windows_u8(static_cast<const uint8_t*>(tc->frames), tc->gather, H, W, ws + L.U1, st));
+  else if (tc) RC(launch_unfold9_windows(static_cast<const float*>(tc->frames), tc->gather, H, W, ws + L.U1, st));
   else RC(launch_unfold9(lr, N, H, W, 1.f, ws + L.U1, st));
   {
     ConvGemmArgs a; memset(&a, 0, sizeof(a));
@@ -1249,7 +1253,7 @@ int forward_impl(EngineImpl* e, const float* lr, float* sr, int training, int up
   }
   // a frozen-tiles forward without an output recomputes the activations for its backward, which does not read SR
   if (tc && sr == nullptr) return 0;
-  // conv3: 9x9, 64->3, no activation (src/models.py:78,86); fp32 NCHW output
+  // conv3: 9x9, 64->3, no activation (src/models.py:78,86); fp32 NCHW output, or uint8 NHWC through tc->scatter
   {
     const int Hs = H << e->n_up, Ws = W << e->n_up;
     ConvGemmArgs a; memset(&a, 0, sizeof(a));
@@ -1280,10 +1284,13 @@ int generator_tile_halo(int n_res, int n_up) {
 }
 
 namespace {
-// argument checks shared by the eval and the frozen tiled forwards (no CUDA call) and the call's gather / scatter tables
-int make_tile_call(const EngineImpl* e, const char* who, const float* frames, int F, int H, int W, const TileDesc* tiles,
-                   int n, float* sr, bool sr_optional, TileCall* tc) {
-  if (frames == nullptr || tiles == nullptr || (sr == nullptr && !sr_optional)) { set_error("%s: null pointer", who); return -22; }
+// argument checks shared by the eval and the frozen tiled forwards (no CUDA call) and the call's gather / scatter tables.
+// Frames are fp32 NCHW, or uint8 NHWC (u8): element strides per frame, channel, row and pixel.
+int make_tile_call(const EngineImpl* e, const char* who, const void* frames, bool u8, int F, int H, int W,
+                   const TileDesc* tiles, int n, void* sr, bool sr_optional, TileCall* tc) {
+  if (frames == nullptr) { set_error("%s: null pointer (frames)", who); return -22; }
+  if (tiles == nullptr) { set_error("%s: null pointer (tiles)", who); return -22; }
+  if (sr == nullptr && !sr_optional) { set_error("%s: null pointer (output)", who); return -22; }
   if (F < 1 || H < 1 || W < 1) { set_error("%s: F, H and W must be >= 1 (got %d, %d, %d)", who, F, H, W); return -26; }
   const int n_max = e->N < kMaxTiles ? e->N : kMaxTiles;
   if (n < 1 || n > n_max) { set_error("%s: tile count %d outside 1..%d (engine N and SRG_MAX_TILES)", who, n, n_max); return -27; }
@@ -1304,14 +1311,17 @@ int make_tile_call(const EngineImpl* e, const char* who, const float* frames, in
   const int64_t plane = int64_t(H) * W, Ws = int64_t(W) << s, plane_o = (int64_t(H) << s) * Ws;
   memset(tc, 0, sizeof(*tc));
   tc->frames = frames;
+  tc->u8 = u8;
   tc->n = n;
-  tc->gather.n = n; tc->gather.plane = plane; tc->gather.pitch = W;
-  tc->scatter.n = n; tc->scatter.plane = plane_o; tc->scatter.pitch = Ws;
+  const int64_t px = u8 ? 3 : 1;
+  tc->gather.n = n; tc->gather.plane = u8 ? 1 : plane; tc->gather.pitch = px * W;
+  tc->scatter.n = n; tc->scatter.u8 = u8; tc->scatter.plane = u8 ? 1 : plane_o; tc->scatter.pitch = px * Ws;
+  tc->scatter.px = px;
   for (int i = 0; i < n; ++i) {
     const TileDesc& t = tiles[i];
-    tc->gather.base[i] = int64_t(t.frame) * 3 * plane + int64_t(t.y0) * W + t.x0;
+    tc->gather.base[i] = int64_t(t.frame) * 3 * plane + (int64_t(t.y0) * W + t.x0) * px;
     FoldTile& o = tc->scatter.t[i];
-    o.base = int64_t(t.frame) * 3 * plane_o + (int64_t(t.y0) << s) * Ws + (int64_t(t.x0) << s);
+    o.base = int64_t(t.frame) * 3 * plane_o + ((int64_t(t.y0) << s) * Ws + (int64_t(t.x0) << s)) * px;
     o.h_lo = t.crop_y0 << s; o.h_hi = (t.crop_y0 + t.crop_h) << s;
     o.w_lo = t.crop_x0 << s; o.w_hi = (t.crop_x0 + t.crop_w) << s;
   }
@@ -1323,9 +1333,35 @@ int generator_forward_tiles(GeneratorEngine* g, const float* frames, int F, int 
                             float* sr, cudaStream_t st) {
   EngineImpl* e = static_cast<EngineImpl*>(g);
   TileCall tc;
-  RC(make_tile_call(e, "srg_generator_forward_tiles", frames, F, H, W, tiles, n, sr, false, &tc));
+  RC(make_tile_call(e, "srg_generator_forward_tiles", frames, false, F, H, W, tiles, n, sr, false, &tc));
   if (!e->ws) { set_error("srg_generator_forward_tiles: no workspace bound"); return -23; }
   if (e->ws_training) { set_error("srg_generator_forward_tiles: needs an eval-sized workspace (this one is bound for training)"); return -24; }
+  return forward_impl(e, nullptr, sr, 0, 0, kPhaseAll, false, st, &tc);
+}
+
+int generator_forward_tiles_u8(GeneratorEngine* g, const uint8_t* frames, int F, int H, int W, const TileDesc* tiles, int n,
+                               uint8_t* sr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  TileCall tc;
+  RC(make_tile_call(e, "srg_generator_forward_tiles_u8", frames, true, F, H, W, tiles, n, sr, false, &tc));
+  if (!e->ws) { set_error("srg_generator_forward_tiles_u8: no workspace bound"); return -23; }
+  if (e->ws_training) { set_error("srg_generator_forward_tiles_u8: needs an eval-sized workspace (this one is bound for training)"); return -24; }
+  return forward_impl(e, nullptr, sr, 0, 0, kPhaseAll, false, st, &tc);
+}
+
+int generator_forward_u8(GeneratorEngine* g, const uint8_t* lr, uint8_t* sr, cudaStream_t st) {
+  EngineImpl* e = static_cast<EngineImpl*>(g);
+  if (lr == nullptr) { set_error("srg_generator_forward_u8: null pointer (input frames)"); return -22; }
+  if (sr == nullptr) { set_error("srg_generator_forward_u8: null pointer (output)"); return -22; }
+  if (!e->ws) { set_error("srg_generator_forward_u8: no workspace bound"); return -23; }
+  TileCall tc;
+  memset(&tc, 0, sizeof(tc));
+  tc.frames = lr;
+  tc.u8 = true;
+  tc.n = e->N;
+  const int64_t Ws = int64_t(e->W) << e->n_up, Hs = int64_t(e->H) << e->n_up;
+  tc.scatter.u8 = 1;
+  tc.scatter.item = 3 * Hs * Ws; tc.scatter.plane = 1; tc.scatter.pitch = 3 * Ws; tc.scatter.px = 3;
   return forward_impl(e, nullptr, sr, 0, 0, kPhaseAll, false, st, &tc);
 }
 
@@ -1333,7 +1369,7 @@ int generator_forward_frozen_tiles(GeneratorEngine* g, const float* frames, int 
                                    float* sr, cudaStream_t st) {
   EngineImpl* e = static_cast<EngineImpl*>(g);
   TileCall tc;
-  RC(make_tile_call(e, "srg_generator_forward_frozen_tiles", frames, F, H, W, tiles, n, sr, true, &tc));
+  RC(make_tile_call(e, "srg_generator_forward_frozen_tiles", frames, false, F, H, W, tiles, n, sr, true, &tc));
   if (!e->ws) { set_error("srg_generator_forward_frozen_tiles: no workspace bound"); return -23; }
   if (!e->ws_training) { set_error("srg_generator_forward_frozen_tiles: needs a training-sized workspace (this one is bound for eval)"); return -24; }
   RC(forward_impl(e, nullptr, sr, 1, 0, kPhaseAll, true, st, &tc));

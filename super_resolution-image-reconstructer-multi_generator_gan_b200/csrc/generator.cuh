@@ -98,6 +98,10 @@ struct TileDesc { int32_t frame, y0, x0, crop_y0, crop_x0, crop_h, crop_w; };
 int generator_tile_halo(int n_res, int n_up);
 int generator_forward_tiles(GeneratorEngine* g, const float* frames_nchw, int F, int H, int W, const TileDesc* tiles, int n,
                             float* sr_nchw, cudaStream_t st);
+// 8-bit frame I/O of the eval forward (srg_generator_forward_u8 / _tiles_u8): uint8 NHWC in, quantised uint8 NHWC out
+int generator_forward_u8(GeneratorEngine* g, const uint8_t* lr_nhwc, uint8_t* sr_nhwc, cudaStream_t st);
+int generator_forward_tiles_u8(GeneratorEngine* g, const uint8_t* frames_nhwc, int F, int H, int W, const TileDesc* tiles,
+                               int n, uint8_t* sr_nhwc, cudaStream_t st);
 // eval-mode autograd over windows (srg_generator_forward_frozen_tiles / srg_generator_backward_tiles): the frozen forward of
 // n windows on a training workspace (sr_nchw may be NULL: activations only), then the backward of those windows
 int generator_forward_frozen_tiles(GeneratorEngine* g, const float* frames_nchw, int F, int H, int W, const TileDesc* tiles,

@@ -320,7 +320,7 @@ class SRResNet(_FlatModule):
 
     conv 9x9 (3->64) + LeakyReLU(0.2) -> ``num_residuals`` x [conv3x3, BN, ReLU, conv3x3, BN, +skip] -> conv3x3 ->
     + global skip -> ``int(upscale_factor // 2)`` x [conv3x3 (64->256), PixelShuffle(2), ReLU] -> conv 9x9 (64->3).
-    Input / output: NCHW fp32 CUDA tensors.  The kernels are specialised for in_channels=3, num_features=64 (the
+    Input / output: NCHW fp32 CUDA tensors; ``upscale_u8`` takes and returns uint8 NHWC frames.  The kernels are specialised for in_channels=3, num_features=64 (the
     reference's only configuration); other widths raise.
     """
 
@@ -494,11 +494,12 @@ class SRResNet(_FlatModule):
             rt[key] = (win_h, win_w, n, tiles)
         return rt[key]
 
-    def _forward_tiled(self, x: torch.Tensor) -> torch.Tensor:
+    def _forward_tiled(self, x: torch.Tensor, u8: bool = False) -> torch.Tensor:
         """eval-mode forward of frames too large for ``tile_budget_bytes``: the windows of all frames in order, as many per
         ``srg_generator_forward_tiles`` call as the plan's ``tiles_per_call`` (usually 1: the planner picks the largest
-        window that fits), through ONE engine of that many windows."""
-        N, _, H, W = x.shape
+        window that fits), through ONE engine of that many windows.  ``u8``: uint8 N x H x W x 3 frames in and out
+        (``upscale_u8``, ``srg_generator_forward_tiles_u8``), with the same plan and engine."""
+        N, H, W = (x.shape[0], x.shape[1], x.shape[2]) if u8 else (x.shape[0], x.shape[2], x.shape[3])
         rt = self._rt
         budget = int(self.tile_budget_bytes)
         key = ("tiles", N, H, W, budget)
@@ -507,14 +508,18 @@ class SRResNet(_FlatModule):
             rt[key] = tiling.plan_tiles(N, H, W, halo, lambda h, w: self._eval_ws_bytes(h, w, x.device), budget)
         win_h, win_w, per_call, tiles = rt[key]
         s = self.num_upsample_stages
-        sr = torch.empty(N, 3, H << s, W << s, dtype=torch.float32, device=x.device)
+        if u8:
+            sr = torch.empty(N, H << s, W << s, 3, dtype=torch.uint8, device=x.device)
+        else:
+            sr = torch.empty(N, 3, H << s, W << s, dtype=torch.float32, device=x.device)
         n = min(per_call, len(tiles))
         eng = self._engine(n, win_h, win_w, False, x.device, False)
         eng.bind(rt["flat"], None, rt["flat_buf"])
         check(_lib.lib().srg_generator_pack(eng.handle, stream_ptr()), "srg_generator_pack")
         rt["last_engine"] = eng
+        call = tiling.forward_tiles_u8 if u8 else tiling.forward_tiles
         for i in range(0, len(tiles), n):
-            tiling.forward_tiles(eng.handle, x, tiles[i:i + n], sr, stream_ptr())
+            call(eng.handle, x, tiles[i:i + n], sr, stream_ptr())
         return sr
 
     # ---- forward ---------------------------------------------------------------------------------------------------
@@ -608,9 +613,11 @@ class SRResNet(_FlatModule):
         return sr
 
     def _eval_into(self, x: torch.Tensor, out: torch.Tensor, packed: set) -> None:
-        """eval-mode forward of a chunk of frames straight into ``out`` (a contiguous slice of the caller's batch)."""
+        """eval-mode forward of a chunk of frames straight into ``out`` (a contiguous slice of the caller's batch): fp32
+        NCHW, or uint8 NHWC in and out (``upscale_u8``, ``srg_generator_forward_u8``)."""
         assert x.is_contiguous() and out.is_contiguous()
-        n, _, H, W = x.shape
+        u8 = x.dtype == torch.uint8
+        n, H, W = (x.shape[0], x.shape[1], x.shape[2]) if u8 else (x.shape[0], x.shape[2], x.shape[3])
         rt = self._rt
         eng = self._engine(n, H, W, False, x.device, False)
         eng.bind(rt["flat"], None, rt["flat_buf"])
@@ -619,8 +626,46 @@ class SRResNet(_FlatModule):
             check(L.srg_generator_pack(eng.handle, stream_ptr()), "srg_generator_pack")
             packed.add(id(eng))
         rt["last_engine"] = eng
+        if u8:
+            check(L.srg_generator_forward_u8(eng.handle, c_void_p(x.data_ptr()), c_void_p(out.data_ptr()), stream_ptr()),
+                  "srg_generator_forward_u8")
+            return
         check(L.srg_generator_forward(eng.handle, c_void_p(x.data_ptr()), c_void_p(out.data_ptr()), 0, 0, stream_ptr()),
               "srg_generator_forward")
+
+    def upscale_u8(self, frames: torch.Tensor) -> torch.Tensor:
+        """8-bit frames in and out: uint8 N x H x W x 3 CUDA (decoded RGB, channel-last, as ``transformers`` takes
+        them) -> uint8 N x (H << s) x (W << s) x 3, s = ``num_upsample_stages``.
+
+        The result is, bit for bit, ``q(self(transformers.to_tensor(frames)))`` with
+        ``q(sr) = (sr.clamp(0, 1) * 255).round().to(torch.uint8).permute(0, 2, 3, 1)``: conv1 reads each byte v as
+        v / 255 with ToTensor's fp32 division, and conv3's epilogue stores round-half-even(255 * clamp(y, 0, 1)).  Neither
+        an fp32 copy of the input nor an fp32 SR tensor is made.  A NaN output stores 0 (torch's cast of NaN is
+        undefined).  Eval mode only.  Frames are routed like the detached eval forward: streamed in chunks under
+        ``stream_budget_bytes``, upscaled in windows under ``tile_budget_bytes``, through the same engines.  No autograd
+        graph is built.
+        """
+        if self.training:
+            raise RuntimeError("SRResNet.upscale_u8 runs the eval forward only: call .eval() first")
+        if frames.dtype != torch.uint8:
+            raise RuntimeError(f"SRResNet.upscale_u8 takes uint8 frames, got {frames.dtype}")
+        if frames.dim() != 4 or frames.shape[3] != 3 or min(frames.shape) < 1:
+            raise RuntimeError(f"SRResNet.upscale_u8 expects an N x H x W x 3 batch, got {tuple(frames.shape)}")
+        if not frames.is_cuda:
+            raise RuntimeError("SRResNet.upscale_u8 (libsrgan_b200) takes a CUDA tensor; there is no CPU path")
+        frames = frames.contiguous()
+        N, H, W, _ = frames.shape
+        self._flatten(frames.device)
+        if self.tile_budget_bytes is not None and self._eval_ws_bytes(H, W, frames.device) > self.tile_budget_bytes:
+            return self._forward_tiled(frames, u8=True)
+        s = self.num_upsample_stages
+        sr = torch.empty(N, H << s, W << s, 3, dtype=torch.uint8, device=frames.device)
+        chunk = self._stream_chunk(N, H, W, frames.device) if N > 1 else N
+        packed = set()
+        for i in range(0, N, chunk):
+            j = min(N, i + chunk)
+            self._eval_into(frames[i:j], sr[i:j], packed)
+        return sr
 
 
 # ----------------------------------------------------------------------------------------------------------------

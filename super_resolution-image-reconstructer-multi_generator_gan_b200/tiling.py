@@ -185,6 +185,16 @@ def forward_tiles(handle, frames, tiles: List[Tile], out, stream) -> None:
                "srg_generator_forward_tiles")
 
 
+def forward_tiles_u8(handle, frames, tiles: List[Tile], out, stream) -> None:
+    """One ``srg_generator_forward_tiles_u8`` call: as ``forward_tiles`` on uint8 frames F x H x W x 3 into a uint8
+    ``out`` F x (H << s) x (W << s) x 3 (contiguous CUDA tensors), quantised as ``SRResNet.upscale_u8`` documents."""
+    arr = (SrgTile * len(tiles))(*[SrgTile(*t) for t in tiles])
+    F, H, W, _ = frames.shape
+    _lib.check(_lib.lib().srg_generator_forward_tiles_u8(handle, ctypes.c_void_p(frames.data_ptr()), F, H, W, arr,
+                                                         len(tiles), ctypes.c_void_p(out.data_ptr()), stream),
+               "srg_generator_forward_tiles_u8")
+
+
 def forward_frozen_tiles(handle, frames, tiles: List[Tile], out, stream) -> None:
     """One ``srg_generator_forward_frozen_tiles`` call: as ``forward_tiles`` on an engine bound to a training workspace,
     keeping the activations for ``backward_tiles``.  ``out`` may be None (a recompute for the backward: no output)."""
