@@ -124,8 +124,23 @@ __global__ void __launch_bounds__(256) d_fold0_kernel(const __nv_bfloat16* __res
 }
 
 // ------------------------------------------------------------------------------------------------ pool + statistics
+// Pooled value of window (0, 0) (y = &Y[n][0][0][c]), same scan as the pool in d_stats_kernel.  Out of line: inlined,
+// it changes how the compiler schedules the pool loop's loads, and that loop runs a third slower.
+__device__ __noinline__ float d_pool_first(const float* __restrict__ y, int Wo, int C) {
+  float best = y[0];
+#pragma unroll
+  for (int k = 1; k < 9; ++k) {
+    const float v = y[(int64_t(k / 3) * Wo + (k % 3)) * C];
+    if (v > best) best = v;
+  }
+  return best;
+}
 // One block = one chunk of pooled pixels of one image.  Threads: channel-fastest.  partials[n][chunk][2][C].
-template <int MODE>  // 0: max-pool Y -> P, idx ; sums p, p^2.   1: backward: g = dz * act'(xhat) ; sums g, g*xhat
+// MODE 0 sums p - k and (p - k)^2 with k = p[n][0][0][c], one element of the map: a one-pass variance of shifted
+// values keeps its rounding error proportional to the spread of p instead of to mean^2, which matters when an
+// InstanceNorm map is nearly constant or has 2-4 elements (var << mean^2, at or below eps).  The shift must be an
+// element of the map: the conv output at pixel (0, 0), for one, can sit far from a 3-element map's values.
+template <int MODE>  // 0: max-pool Y -> P, idx ; sums p - k, (p - k)^2.   1: backward: g = dz * act'(xhat) ; sums g, g*xhat
 __global__ void __launch_bounds__(256) d_stats_kernel(const float* __restrict__ Y, int Ho, int Wo, int Hp, int Wp, int C,
                                                       float* __restrict__ P, uint8_t* __restrict__ idx,
                                                       const float* __restrict__ stats, const void* __restrict__ dz_src,
@@ -142,7 +157,8 @@ __global__ void __launch_bounds__(256) d_stats_kernel(const float* __restrict__ 
   for (int cbase = 0; cbase < C; cbase += 256) {
     const int c = cbase + cl;
     float s1 = 0.f, s2 = 0.f;
-    float mean = 0.f, inv = 0.f;
+    float mean = 0.f, inv = 0.f, shift = 0.f;
+    if (MODE == 0) shift = d_pool_first(Y + int64_t(n) * Ho * Wo * C + c, Wo, C);
     if (MODE == 1) { mean = stats[(int64_t(n) * C + c) * 2]; inv = stats[(int64_t(n) * C + c) * 2 + 1]; }
     for (int pp = p0 + lane; pp < p1; pp += lanes) {
       const int hp = pp / Wp, wp = pp - hp * Wp;
@@ -159,8 +175,9 @@ __global__ void __launch_bounds__(256) d_stats_kernel(const float* __restrict__ 
         }
         P[po] = best;
         idx[po] = uint8_t(bi);
-        s1 += best;
-        s2 += best * best;
+        const float q = best - shift;
+        s1 += q;
+        s2 += q * q;
       } else {
         const float xhat = (P[po] - mean) * inv;
         float dz, d;
@@ -196,13 +213,15 @@ __global__ void __launch_bounds__(256) d_stats_kernel(const float* __restrict__ 
     __syncthreads();
   }
 }
-// stats[n][c] = (mean, inv_std)  (MODE 0)   or   (sum g / cnt, sum g*xhat / cnt)  (MODE 1)
+// stats[n][c] = (mean, inv_std)  (MODE 0, P = pooled map holding the shift k at pixel 0)
+//           or  (sum g / cnt, sum g*xhat / cnt)  (MODE 1, P unused)
 template <int MODE>
 __global__ void d_finalize_kernel(const float* __restrict__ partials, int chunks, int C, int NC, double count,
-                                  float* __restrict__ stats) {
+                                  const float* __restrict__ P, int64_t npix, float* __restrict__ stats) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= NC) return;
   const int n = i / C, c = i - n * C;
+  const float shift = MODE == 0 ? __ldg(P + int64_t(n) * npix * C + c) : 0.f;   // issued ahead of the partial sums
   double a = 0.0, b = 0.0;
   for (int k = 0; k < chunks; ++k) {
     const float* src = partials + ((int64_t(n) * chunks + k) * 2) * C;
@@ -210,9 +229,10 @@ __global__ void d_finalize_kernel(const float* __restrict__ partials, int chunks
     b += double(src[C + c]);
   }
   if (MODE == 0) {
-    const double mean = a / count;
-    double var = b / count - mean * mean;
+    const double m = a / count;                 // mean of p - k
+    double var = b / count - m * m;
     if (var < 0.0) var = 0.0;
+    const double mean = double(shift) + m;
     stats[2 * i] = float(mean);
     stats[2 * i + 1] = float(1.0 / sqrt(var + double(kEps)));
   } else {
@@ -664,7 +684,9 @@ int discriminator_forward(DiscriminatorEngine* d, const float* x, float* out, in
                                                        nullptr, 0, 0, 0, nullptr, chunks, partials);
     D_LAUNCH_CHECK("d_pool_stats");
     d_finalize_kernel<0><<<(N * s.Cout + 127) / 128, 128, 0, st>>>(partials, chunks, s.Cout, N * s.Cout,
-                                                                   double(s.Hp) * s.Wp, stats);
+                                                                   double(s.Hp) * s.Wp,
+                                                                   reinterpret_cast<const float*>(ws + L.P[l]),
+                                                                   int64_t(s.Hp) * s.Wp, stats);
     D_LAUNCH_CHECK("d_in_finalize");
     if (l < 3) {
       const DiscStage& nx = e->st[l + 1];
@@ -712,7 +734,7 @@ int discriminator_backward(DiscriminatorEngine* d, const float* dout, int param_
                                                        l == 3 ? 0 : 1, Hs2, Ws2, G, chunks, partials);
     D_LAUNCH_CHECK("d_in_bwd_stats");
     d_finalize_kernel<1><<<(N * s.Cout + 127) / 128, 128, 0, st>>>(partials, chunks, s.Cout, N * s.Cout,
-                                                                   double(s.Hp) * s.Wp, stats2);
+                                                                   double(s.Hp) * s.Wp, nullptr, 0, stats2);
     D_LAUNCH_CHECK("d_in_bwd_finalize");
     // ---- InstanceNorm + MaxPool backward -> d(conv output), bf16
     {
