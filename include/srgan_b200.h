@@ -138,10 +138,10 @@ int srg_generator_tensor_info(const srg_generator_t* g, int i, char* name, int n
 int srg_generator_set_keep_grads(srg_generator_t* g, int keep);
 long long srg_generator_launch_count(const srg_generator_t* g); /* kernels enqueued so far by this engine */
 long long srg_total_launches(void);                             /* kernels enqueued so far by the whole library */
-/* parity-test / A-B aid: which convolution kernels later launches use.  0 = default (conv3_il for plain 3x3 / 64-channel
- * launches, conv9_rows for conv3; honours SRG_CONV_IL), 1 = the generic strip kernel for everything, 2 = conv3_il with one
- * 8-pixel strip per column shift, 3 = conv3_il with one 10-pixel strip.  Returns the previous value.  Affects kernels
- * enqueued afterwards (a captured CUDA graph keeps what it was captured with). */
+/* parity-test aid: which convolution kernels later launches use.  0 = default (conv3_il for plain 3x3 / 64-channel
+ * launches, conv9_rows for conv3), 1 = the generic strip kernel for everything (the reference the specialised kernels are
+ * tested against).  Returns the previous value; any other value returns a negative code (srg_last_error) and leaves the
+ * setting unchanged.  Affects kernels enqueued afterwards (a captured CUDA graph keeps what it was captured with). */
 int srg_set_conv_variant(int variant);
 /* host-only: the work split of the batched trunk weight-gradient kernel for `layers` same-shape [N,H,W,64] layers
  * (no device work, usable without a GPU): CTA c owns flattened (layer, tile) indices [c * per_cta, (c + 1) * per_cta),
@@ -161,7 +161,7 @@ int srg_generator_profile_read(srg_generator_t* g, double* ms_sum, long long* co
  * (src/models.py:10-25 ResidualBlock x 16, :66 conv2) with their training-mode BatchNorm steps in ONE cooperative launch.
  * srg_set_trunk_fused(mode): 0 = one launch per layer, 1 = the fused kernel wherever it applies, 2 = automatic (default:
  * fused when a layer has at most one 32x8-pixel tile per SM, i.e. launch-latency-bound sizes; measured in
- * profiles/r02_notes.md).  SRG_TRUNK_FUSED=0/1 sets the initial mode.  Returns the previous mode.  srg_generator_trunk_layers: trunk conv layers covered by
+ * profiles/r02_notes.md).  Returns the previous mode.  srg_generator_trunk_layers: trunk conv layers covered by
  * the engine's last profiled launch (1 = per-layer launches).  srg_generator_trunk_error: non-zero if a bounded in-kernel
  * wait of the fused kernel ever gave up (bit 0 cross-CTA flag / barrier, bit 1 mbarrier, bit 2 peer GPU); synchronises. */
 int srg_set_trunk_fused(int on);
@@ -177,7 +177,7 @@ int srg_set_trunk_fused(int on);
  * streams that join `stream` again before the call returns; capturable).  srg_generator_trunk_layers reports 33 / n / 1 for
  * the fused / grouped / per-layer form of the last profiled launch.  Engines must be bound for training; split execution
  * needs the fused trunk kernel or the grouped path (batched trunk weight gradients, single GPU or the peer-memory
- * SyncBatchNorm transport, SRG_TRUNK_GROUPED != 0) -- otherwise these return an error and the caller uses the whole-pass
+ * SyncBatchNorm transport) -- otherwise these return an error and the caller uses the whole-pass
  * entry points. */
 int srg_generator_forward_phases(srg_generator_t* g, const float* lr_nchw, float* sr_nchw, int training, int update_running,
                                  int phases, void* stream);

@@ -11,7 +11,7 @@
 //
 // Three kernels live in this file, all behind launch_conv_gemm():
 //   conv_gemm_kernel<BLOCK_N, NT>  the generic strip kernel described above (one N = 64 / 32 MMA per tap and K-step);
-//   conv3_il_kernel<WIDE>          plain 3x3 / 64-input-channel launches: row-interleaved accumulator blocks so that two
+//   conv3_il_kernel                plain 3x3 / 64-input-channel launches: row-interleaved accumulator blocks so that two
 //                                  taps share one N = 128 MMA (the ~64-cycle floor of an M128 MMA makes that free);
 //   conv9_rows_kernel              the 9x9 / 3-output-channel conv3: one image row per MMA feeding up to 8 output rows.
 #include "conv_gemm.cuh"
@@ -66,7 +66,6 @@ struct ConvKParams {
   void* out;     // fold9 only (through the FoldScatter of ConvKParamsFold)
   int out_mode;
   float* stats;  // per-CTA channel sums / sums of squares (BatchNorm statistics fused into the epilogue)
-  const uint32_t* stats_y;  // optional second factor (bf16 pairs) for the product sums
   long long* prof;  // optional per-CTA role timers (debug)
 };
 
@@ -296,36 +295,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
     int acc = 0, ob = 0, ab = 0;
     uint32_t acc_phase = 0, aux_phase = 0;
     float st_s0 = 0.f, st_s1 = 0.f, st_q0 = 0.f, st_q1 = 0.f;   // BatchNorm statistics of this thread's channel pair
-    uint32_t yv_next[16];
-    auto load_stats_y = [&](int t, uint32_t (&dst)[16]) {
-      if (t >= p.tiles_total) return;
-      const int n_ = t / tiles_per_img;
-      const int rem_ = t - n_ * tiles_per_img;
-      const int h0_ = (rem_ / p.tiles_w) * p.TH;
-      const int w0_ = (rem_ % p.tiles_w) * p.tile_step_w + p.tile_w_org;
-      const int c2 = etid & 31, part = etid >> 5;
-#pragma unroll
-      for (int rr = 0; rr < 16; ++rr) {
-        const int mm = part * 16 + rr;
-        const int th = mm >> 3;                      // statistics are only offered for 8-pixel-wide tiles
-        const int hh = h0_ + th, ww = w0_ + (mm & 7);
-        dst[rr] = (hh < p.H && ww < p.W) ? __ldg(p.stats_y + ((size_t(n_) * p.H + hh) * p.W + ww) * 32 + c2) : 0u;
-      }
-    };
-    if (!kFold && p.stats_y != nullptr) load_stats_y(tile0, yv_next);
     for (int tile = tile0; tile < p.tiles_total; tile += p.ctas_per_block) {
       const int n = tile / tiles_per_img;
       const int rem = tile - n * tiles_per_img;
       const int h0 = (rem / p.tiles_w) * p.TH;
       const int w0 = (rem % p.tiles_w) * p.tile_step_w + p.tile_w_org;
-      uint32_t yv[16];
-      if (!kFold && p.stats_y != nullptr) {
-        // second factor of the product statistics, software-pipelined one tile ahead: this tile's values were loaded
-        // during the previous iteration, the next tile's loads are issued now and land while this tile is processed
-#pragma unroll
-        for (int rr = 0; rr < 16; ++rr) yv[rr] = yv_next[rr];
-        load_stats_y(tile + p.ctas_per_block, yv_next);
-      }
       { long long t0_ = clock64(); mbar_wait(&tfull[acc], acc_phase); prof_acc[3] += clock64() - t0_; }
       tc_fence_after();
       const uint32_t t_addr = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(acc * BLOCK_N + hf * 32);
@@ -452,10 +426,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
             if (h0 + th < p.H && w0 + (mm & 7) < p.W) {
               const uint32_t v = *reinterpret_cast<const uint32_t*>(sp + mm * 128 + ((((c2 >> 2)) ^ (mm & 7)) << 4) + (c2 & 3) * 4);
               const float a0 = bf16_lo(v), a1 = bf16_hi(v);
-              float b0 = a0, b1 = a1;
-              if (p.stats_y != nullptr) { b0 = bf16_lo(yv[r]); b1 = bf16_hi(yv[r]); }
               st_s0 += a0; st_s1 += a1;
-              st_q0 = fmaf(a0, b0, st_q0); st_q1 = fmaf(a1, b1, st_q1);
+              st_q0 = fmaf(a0, a0, st_q0); st_q1 = fmaf(a1, a1, st_q1);
             }
           }
         }
@@ -534,22 +506,20 @@ struct IlKParams {
   int aux_mode;              // 0 none, 1 add (residual), 2 mask (zero where aux <= 0)
   int out_mode;
   float* stats[kIlMaxGroups];            // per-CTA channel sums / sums of squares (row = the CTA's index inside its group)
-  const uint32_t* stats_y[kIlMaxGroups]; // optional second factor (bf16 pairs, the output's geometry): sum(out * stats_y) replaces sum(out^2)
   uint64_t pol_out, pol_aux, pol_in; // L2 eviction priorities of the output store / the residual-mask tile loads / the operand strips
-  int opt;                   // SRG_IL_OPT bits: 1 = first tile column shift by column shift (filter streams in under the MMAs),
-                             // 2 = leave without waiting for the last store's global writes (only for its shared-memory reads)
+  int ramp;                  // 1: the first tile runs column shift by column shift (the filter streams in under the MMAs)
   long long* prof;
 };
 
 constexpr int kIlThreads = 64 + 512;            // warp 0 producer, warp 1 MMA, warps 2-9 block E, warps 10-17 block O
-constexpr uint32_t kIlHalfStrip = 17 * 8 * 128; // 17 rows x 8 pixels x 64 bf16
 constexpr uint32_t kIlWBytes = 9 * 64 * 128;    // resident filter: [kw 3][kh2 ; kh1 ; kh0][64 cout][64 cin]
-// WIDE: ONE 10-pixel-wide half strip (17 rows x 10 pixels, row pitch 1280 B) serves all three column shifts: the A
+// ONE 10-pixel-wide half strip (17 rows x 10 pixels, row pitch 1280 B) serves all three column shifts: the A
 // descriptor starts kw * 128 B into it with a stride (SBO) of 1280 B between 8-pixel row groups.  Measured on B200
 // (tools/conv_probe il_* cases): the UMMA 128B swizzle is a function of the ABSOLUTE shared-memory address bits, exactly
 // like the TMA write side, so a start address / group stride that is only 128-byte aligned reads the right data with
 // base_offset = 0 (setting base_offset = (addr >> 7) & 7 gives wrong results).  One third of the L2->SM operand traffic
-// and of the stage footprint of the three-strip form, so the same shared memory holds a 2x deeper prefetch.
+// and of the stage footprint of one 8-pixel half strip per column shift, so the same shared memory holds a 2x deeper
+// prefetch.
 constexpr uint32_t kIlWidePitch = 10 * 128;
 constexpr uint32_t kIlWideStage = 22 * 1024;    // 17 x 1280 = 21760 B, rounded up to the 1024-byte swizzle period
 
@@ -561,24 +531,11 @@ constexpr uint32_t kIlWideStage = 22 * 1024;    // 17 x 1280 = 21760 B, rounded 
 #define IL_PROF(...)
 #define IL_TIMED(slot, ...) { __VA_ARGS__ }
 #endif
-// SRG_IL_MAXREG (compile time): register cap of conv3_il.  576 threads x 96 registers leave 10 K of the SM's 64 K registers,
-// i.e. no 256-thread CTA of the BatchNorm passes (40-56 registers per thread) of another graph branch can be co-resident
-// with a convolution CTA; at 64 registers two of them fit.
-#ifndef SRG_IL_MAXREG
-#define SRG_IL_MAXREG 0
-#endif
-#if SRG_IL_MAXREG > 0
-#define IL_KERNEL_BOUNDS __maxnreg__(SRG_IL_MAXREG)
-#else
-#define IL_KERNEL_BOUNDS __launch_bounds__(kIlThreads, 1)
-#endif
-// YS: the statistics' second factor comes from a global tensor (p.stats_y, BatchNorm-backward product sums); a separate
-// instantiation so that its 16 prefetch registers do not push the common form over the 96-register budget.
 // GROUPED: CTA c works for group c % n_groups (a run-time index into the per-group tensor maps / pointers).  Measured on one
 // box: one body per group with a compile-time index (no spills, 3x the code) runs the grouped trunk launch in 38.5-40.9 us, the
 // run-time index (8 bytes of spills) in 33.2 us (profiles/r02_ab_grouped.log), so the run-time index stays.
-template <bool WIDE, bool YS, bool GROUPED = false>
-__global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKParams p) {
+template <bool GROUPED>
+__global__ void __launch_bounds__(kIlThreads, 1) conv3_il_kernel(const __grid_constant__ IlKParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __builtin_assume(__isShared(smem));      // the integer round-up hides the state space: keep LDS / STS instead of generic accesses
@@ -588,7 +545,7 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
 
   uint8_t* w_smem = smem;
   uint8_t* stages = w_smem + kIlWBytes;
-  constexpr uint32_t kStage = WIDE ? kIlWideStage : kIlHalfStrip;
+  constexpr uint32_t kStage = kIlWideStage;
   uint8_t* out_stage = stages + size_t(p.n_stages) * kStage;             // [block 2][16 KB]
   uint8_t* aux_stage = out_stage + 2 * kTileOutBytes;                     // [block 2][16 KB] (aux_mode != 0)
   uint8_t* tail = aux_stage + (p.aux_mode ? 2 * kTileOutBytes : 0);
@@ -614,7 +571,6 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
   const CUtensorMap* const aux_map = &p.aux_map[2 * grp];
   const CUtensorMap* const out_map = &p.out_map[GROUPED ? 2 * grp : 0];
   float* const stats = p.stats[grp];
-  const uint32_t* const stats_y = p.stats_y[grp];
   const int tiles_per_img = p.tiles_h * p.tiles_w;
 
   if (warp == 0 && lane == 0) {
@@ -655,10 +611,10 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
         for (int r = 0; r < 3; ++r)
           tma_load_2d(w_smem + size_t(s * 3 + (2 - r)) * 8192, w_map, &wfull[s], 0, (s * 3 + r) * p.cout_total + nblk * 64);
       };
-      // WIDE: only the first column shift's 24 KB go out ahead of the first tile's strips; the other two follow them.  All
+      // ramp: only the first column shift's 24 KB go out ahead of the first tile's strips; the other two follow them.  All
       // CTAs start together and fetch the same 72 KB, so the ramp is bound by L2 bandwidth (148 x 72 KB): the first tile's
       // MMAs run column shift by column shift (see the MMA warp) and start after 45 KB instead of 115 KB have arrived.
-      const bool ramp = WIDE && (p.opt & 1);
+      const bool ramp = p.ramp != 0;
       load_w(0);
       if (!ramp) { load_w(1); load_w(2); }
       pdl_wait();      // the activations (and aux tensor) come from the previous kernel; the weights above do not
@@ -670,38 +626,18 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
         const int rem = tile - n * tiles_per_img;
         const int hh = (rem / p.tiles_w) * 16;       // tile origin in parity-view rows (h0 / 2)
         const int w0 = (rem % p.tiles_w) * 8;
-        if constexpr (WIDE) {
 #pragma unroll
-          for (int par = 1; par >= 0; --par) {       // odd image rows h0-1+2j first, then even rows h0+2j (j = 0..16)
-            IL_TIMED(0, mbar_wait(&empty[stage], phase ^ 1);)
-            mbar_expect_tx(&full[stage], 17 * kIlWidePitch);
-            tma_load_4d_hint(stages + size_t(stage) * kStage, &in_map[par], &full[stage], 0, w0 + p.strip_dw[0], hh - par, n, p.pol_in);
-            if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
-          }
-          if (first) {
-            if (ramp) { load_w(1); load_w(2); }
-            if (p.aux_mode) {
-              // the first tile's residual / mask blocks go out here, behind everything the first MMAs wait for (the TMA
-              // engine fetches descriptors in order: an aux load issued first would hold the operands back)
-#pragma unroll
-              for (int b = 0; b < 2; ++b) {
-                mbar_expect_tx(&auxfull[b], kTileOutBytes);
-                tma_load_4d_hint(aux_stage + b * kTileOutBytes, &aux_map[b], &auxfull[b], nblk * 64, w0, hh, n, p.pol_aux);
-              }
-            }
-            first = false;
-          }
-        } else {
-          for (int s = 0; s < 3; ++s) {
-#pragma unroll
-            for (int par = 1; par >= 0; --par) {
-              IL_TIMED(0, mbar_wait(&empty[stage], phase ^ 1);)
-              mbar_expect_tx(&full[stage], kIlHalfStrip);
-              tma_load_4d(stages + size_t(stage) * kStage, &in_map[par], &full[stage], 0, w0 + p.strip_dw[s], hh - par, n);
-              if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
-            }
-          }
-          if (first && p.aux_mode) {
+        for (int par = 1; par >= 0; --par) {         // odd image rows h0-1+2j first, then even rows h0+2j (j = 0..16)
+          IL_TIMED(0, mbar_wait(&empty[stage], phase ^ 1);)
+          mbar_expect_tx(&full[stage], 17 * kIlWidePitch);
+          tma_load_4d_hint(stages + size_t(stage) * kStage, &in_map[par], &full[stage], 0, w0 + p.strip_dw[0], hh - par, n, p.pol_in);
+          if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
+        }
+        if (first) {
+          if (ramp) { load_w(1); load_w(2); }
+          if (p.aux_mode) {
+            // the first tile's residual / mask blocks go out here, behind everything the first MMAs wait for (the TMA
+            // engine fetches descriptors in order: an aux load issued first would hold the operands back)
 #pragma unroll
             for (int b = 0; b < 2; ++b) {
               mbar_expect_tx(&auxfull[b], kTileOutBytes);
@@ -719,7 +655,6 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
     constexpr uint32_t idesc64 = make_idesc_bf16(128, 64, 0, 0);
     constexpr uint32_t idesc128 = make_idesc_bf16(128, 128, 0, 0);
     const uint64_t desc_hi = (uint64_t(1024 >> 4) << 32) | (uint64_t(1) << 46) | (uint64_t(2) << 61);
-    const uint32_t stage0_lo = smem_u32(stages) >> 4;
     const uint32_t w_lo = smem_u32(w_smem) >> 4;
     int stage = 0;
     uint32_t phase = 0;
@@ -731,70 +666,69 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
       tc_fence_after();
       const uint32_t d_e = tmem_base + uint32_t(acc * 128);
       const uint32_t d_o = d_e + 64;
-      if constexpr (WIDE) {
-        // descriptor high part: SBO = 1280 B between 8-pixel row groups, base_offset 0 (see kIlWidePitch)
-        const uint64_t adesc_hi = (uint64_t(kIlWidePitch >> 4) << 32) | (uint64_t(1) << 46) | (uint64_t(2) << 61);
-        // the 16 MMAs of one (row parity, column shift) pair; a_base = the half strip's stage (1024-byte aligned)
-        auto issue = [&](int par, int s, uint32_t a_base, bool fresh) {
-          const uint32_t wb = w_lo + uint32_t(s) * (3 * 8192 >> 4);
-          // window starting at half-strip row 0 / row 1, column shift s pixels
-          const uint32_t st0 = a_base + uint32_t(s) * 128u, st1 = st0 + kIlWidePitch;
-          const uint64_t a0 = adesc_hi | uint64_t((st0 & 0x3FFFFu) >> 4);
-          const uint64_t a1 = adesc_hi | uint64_t((st1 & 0x3FFFFu) >> 4);
-          if (par == 1) {
-            const uint64_t b1 = desc_hi | uint64_t(wb);                         // rho = 1: E += kh2, O += kh1
+      // descriptor high part: SBO = 1280 B between 8-pixel row groups, base_offset 0 (see kIlWidePitch)
+      const uint64_t adesc_hi = (uint64_t(kIlWidePitch >> 4) << 32) | (uint64_t(1) << 46) | (uint64_t(2) << 61);
+      // the 16 MMAs of one (row parity, column shift) pair; a_base = the half strip's stage (1024-byte aligned)
+      auto issue = [&](int par, int s, uint32_t a_base, bool fresh) {
+        const uint32_t wb = w_lo + uint32_t(s) * (3 * 8192 >> 4);
+        // window starting at half-strip row 0 / row 1, column shift s pixels
+        const uint32_t st0 = a_base + uint32_t(s) * 128u, st1 = st0 + kIlWidePitch;
+        const uint64_t a0 = adesc_hi | uint64_t((st0 & 0x3FFFFu) >> 4);
+        const uint64_t a1 = adesc_hi | uint64_t((st1 & 0x3FFFFu) >> 4);
+        if (par == 1) {
+          const uint64_t b1 = desc_hi | uint64_t(wb);                         // rho = 1: E += kh2, O += kh1
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(d_e, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc128, (!fresh || k > 0) ? 1u : 0u);
-            const uint64_t b0 = desc_hi | uint64_t(wb + (2 * 8192 >> 4));       // rho = -1: E += kh0
+          for (int k = 0; k < 4; ++k)
+            umma_bf16(d_e, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc128, (!fresh || k > 0) ? 1u : 0u);
+          const uint64_t b0 = desc_hi | uint64_t(wb + (2 * 8192 >> 4));       // rho = -1: E += kh0
 #pragma unroll
-            for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc64, 1u);
-          } else {
-            const uint64_t b0 = desc_hi | uint64_t(wb + (8192 >> 4));           // rho = 0: E += kh1, O += kh0
-#pragma unroll
-            for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc128, 1u);
-            const uint64_t b1 = desc_hi | uint64_t(wb);                         // rho = 2: O += kh2
-#pragma unroll
-            for (int k = 0; k < 4; ++k) umma_bf16(d_o, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc64, 1u);
-          }
-        };
-        if (!w_ready && (p.opt & 1)) {
-          // first tile of a training launch: (kw0, odd) (kw0, even) | (kw1, odd) (kw2, odd) -> odd half strip released |
-          // (kw1, even) (kw2, even): the MMAs start once the first 24 KB of the filter and the first half strip have landed
-          // and the rest of the filter streams in underneath them.  Later tiles keep the strip-by-strip order (measured:
-          // the interleaved order costs 4 % in the steady state).  Eval-mode (exclusive) launches never take this path, so an
-          // output pixel's fp32 accumulation order does not depend on the tile slot that computes it and eval results stay
-          // bit-identical between batch layouts.
-          const int st1 = stage; const uint32_t ph1 = phase;
-          if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
-          const int st0 = stage; const uint32_t ph0 = phase;
-          if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
-          const uint32_t base1 = smem_u32(stages) + uint32_t(st1) * kStage, base0 = smem_u32(stages) + uint32_t(st0) * kStage;
-          mbar_wait(&wfull[0], 0);
-          IL_TIMED(2, mbar_wait(&full[st1], ph1);)
-          IL_PROF(prof_acc[0] = clock64() - t_start;)     // ramp: launch -> first MMA issue
-          tc_fence_after();
-          if (elect_one()) issue(1, 0, base1, true);
-          __syncwarp();
-          IL_TIMED(2, mbar_wait(&full[st0], ph0);)
-          tc_fence_after();
-          if (elect_one()) issue(0, 0, base0, false);
-          __syncwarp();
-          mbar_wait(&wfull[1], 0);
-          tc_fence_after();
-          if (elect_one()) issue(1, 1, base1, false);
-          __syncwarp();
-          mbar_wait(&wfull[2], 0);
-          tc_fence_after();
-          if (elect_one()) {
-            issue(1, 2, base1, false);
-            umma_commit(&empty[st1]);
-            issue(0, 1, base0, false);
-            issue(0, 2, base0, false);
-            umma_commit(&empty[st0]);
-          }
-          __syncwarp();
+          for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc64, 1u);
         } else {
+          const uint64_t b0 = desc_hi | uint64_t(wb + (8192 >> 4));           // rho = 0: E += kh1, O += kh0
+#pragma unroll
+          for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc128, 1u);
+          const uint64_t b1 = desc_hi | uint64_t(wb);                         // rho = 2: O += kh2
+#pragma unroll
+          for (int k = 0; k < 4; ++k) umma_bf16(d_o, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc64, 1u);
+        }
+      };
+      if (!w_ready && p.ramp) {
+        // first tile of a training launch: (kw0, odd) (kw0, even) | (kw1, odd) (kw2, odd) -> odd half strip released |
+        // (kw1, even) (kw2, even): the MMAs start once the first 24 KB of the filter and the first half strip have landed
+        // and the rest of the filter streams in underneath them.  Later tiles keep the strip-by-strip order (measured:
+        // the interleaved order costs 4 % in the steady state).  Eval-mode (exclusive) launches never take this path, so an
+        // output pixel's fp32 accumulation order does not depend on the tile slot that computes it and eval results stay
+        // bit-identical between batch layouts.
+        const int st1 = stage; const uint32_t ph1 = phase;
+        if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
+        const int st0 = stage; const uint32_t ph0 = phase;
+        if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
+        const uint32_t base1 = smem_u32(stages) + uint32_t(st1) * kStage, base0 = smem_u32(stages) + uint32_t(st0) * kStage;
+        mbar_wait(&wfull[0], 0);
+        IL_TIMED(2, mbar_wait(&full[st1], ph1);)
+        IL_PROF(prof_acc[0] = clock64() - t_start;)     // ramp: launch -> first MMA issue
+        tc_fence_after();
+        if (elect_one()) issue(1, 0, base1, true);
+        __syncwarp();
+        IL_TIMED(2, mbar_wait(&full[st0], ph0);)
+        tc_fence_after();
+        if (elect_one()) issue(0, 0, base0, false);
+        __syncwarp();
+        mbar_wait(&wfull[1], 0);
+        tc_fence_after();
+        if (elect_one()) issue(1, 1, base1, false);
+        __syncwarp();
+        mbar_wait(&wfull[2], 0);
+        tc_fence_after();
+        if (elect_one()) {
+          issue(1, 2, base1, false);
+          umma_commit(&empty[st1]);
+          issue(0, 1, base0, false);
+          issue(0, 2, base0, false);
+          umma_commit(&empty[st0]);
+        }
+        __syncwarp();
+      } else {
 #pragma unroll
         for (int par = 1; par >= 0; --par) {
           IL_TIMED(2, mbar_wait(&full[stage], phase);)
@@ -813,48 +747,6 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
           __syncwarp();
           if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
         }
-        }
-      } else {
-#pragma unroll 1
-      for (int s = 0; s < 3; ++s) {
-        if (!w_ready) mbar_wait(&wfull[s], 0);
-        const uint32_t wb = w_lo + uint32_t(s) * (3 * 8192 >> 4);     // [kh2 ; kh1 ; kh0] of this column shift
-#pragma unroll
-        for (int par = 1; par >= 0; --par) {
-          IL_TIMED(2, mbar_wait(&full[stage], phase);)
-          tc_fence_after();
-          const uint32_t a_lo = stage0_lo + uint32_t(stage) * (kIlHalfStrip >> 4);
-          if (elect_one()) {
-            if (par == 1) {
-              // odd rows: window rho = 1 (rows h0+1+2g = half-strip row g+1): E += kh2, O += kh1; first MMA of the tile
-              const uint64_t a1 = desc_hi | uint64_t(a_lo + (1024 >> 4));
-              const uint64_t b1 = desc_hi | uint64_t(wb);
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                umma_bf16(d_e, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc128, (s > 0 || k > 0) ? 1u : 0u);
-              // window rho = -1 (rows h0-1+2g = half-strip row g): E += kh0
-              const uint64_t a0 = desc_hi | uint64_t(a_lo);
-              const uint64_t b0 = desc_hi | uint64_t(wb + (2 * 8192 >> 4));
-#pragma unroll
-              for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc64, 1u);
-            } else {
-              // even rows: window rho = 0 (rows h0+2g = half-strip row g): E += kh1, O += kh0
-              const uint64_t a0 = desc_hi | uint64_t(a_lo);
-              const uint64_t b0 = desc_hi | uint64_t(wb + (8192 >> 4));
-#pragma unroll
-              for (int k = 0; k < 4; ++k) umma_bf16(d_e, a0 + uint64_t(2 * k), b0 + uint64_t(2 * k), idesc128, 1u);
-              // window rho = 2 (rows h0+2+2g = half-strip row g+1): O += kh2
-              const uint64_t a1 = desc_hi | uint64_t(a_lo + (1024 >> 4));
-              const uint64_t b1 = desc_hi | uint64_t(wb);
-#pragma unroll
-              for (int k = 0; k < 4; ++k) umma_bf16(d_o, a1 + uint64_t(2 * k), b1 + uint64_t(2 * k), idesc64, 1u);
-            }
-            umma_commit(&empty[stage]);
-          }
-          __syncwarp();
-          if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
-        }
-      }
       }
       w_ready = true;
       if (elect_one()) umma_commit(&tfull[acc]);
@@ -891,17 +783,6 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
       const int rem = tile - n * tiles_per_img;
       const int hh = (rem / p.tiles_w) * 16;
       const int w0 = (rem % p.tiles_w) * 8;
-      // second factor of the product statistics (BatchNorm backward: sum dz * y): the tensor is cold (written in the forward
-      // pass), so its lines are pulled into L2 here, a tile's worth of MMAs ahead of the loads below (no registers held)
-      if constexpr (YS) {
-        const int hr = 2 * (hh + rp) + blk;     // block row 8*rp + r = image row 2*(hh+rp)+blk, pixel w0+r
-        if (hr < p.H && (c4 & 3) == 0) {          // one prefetch per 32-byte sector
-          const uint2* yp = reinterpret_cast<const uint2*>(stats_y + ((size_t(n) * p.H + hr) * p.W + w0) * 32) + c4;
-#pragma unroll
-          for (int r = 0; r < 8; ++r)
-            if (w0 + r < p.W) asm volatile("prefetch.global.L2 [%0];" ::"l"(yp + r * 16));
-        }
-      }
       IL_TIMED(3, mbar_wait(&tfull[acc], acc_phase);) IL_PROF(prof_acc[0] = clock64() - t_start;)
       tc_fence_after();
       const uint32_t t_addr = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(acc * 128 + blk * 64 + hf * 32);
@@ -974,15 +855,6 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
       fence_proxy_async_smem();
       // a tile whose 16 rows x 8 pixels all lie inside the image needs no bounds tests in the statistics loop
       const bool full_tile = 2 * (hh + 15) + blk < p.H && w0 + 7 < p.W;
-      // 8 coalesced 8-byte loads per thread, issued before the barrier so that they land while the group synchronises and
-      // the store is handed to the TMA engine
-      uint2 yv[YS ? 8 : 1];
-      if constexpr (YS) {
-        const int hr = 2 * (hh + rp) + blk;
-        const uint2* yp = reinterpret_cast<const uint2*>(stats_y + ((size_t(n) * p.H + hr) * p.W + w0) * 32) + c4;
-#pragma unroll
-        for (int r = 0; r < 8; ++r) yv[r] = (hr < p.H && w0 + r < p.W) ? __ldg(yp + r * 16) : make_uint2(0u, 0u);
-      }
       named_bar_sync(bar_b, 256);
       if (gtid == 0) {
         const bool ps = p.out_mode == OUT_PIXEL_SHUFFLE;
@@ -1000,11 +872,9 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
           if (row_ok && (full_tile || w0 + r < p.W)) {
             const uint2 sv = *reinterpret_cast<const uint2*>(sp + r * 128 + ((cch ^ uint32_t(r)) << 4));
             const float a0 = bf16_lo(sv.x), a1 = bf16_hi(sv.x), a2 = bf16_lo(sv.y), a3 = bf16_hi(sv.y);
-            float b0 = a0, b1 = a1, b2 = a2, b3 = a3;
-            if constexpr (YS) { b0 = bf16_lo(yv[r].x); b1 = bf16_hi(yv[r].x); b2 = bf16_lo(yv[r].y); b3 = bf16_hi(yv[r].y); }
             st_s[0] += a0; st_s[1] += a1; st_s[2] += a2; st_s[3] += a3;
-            st_q[0] = fmaf(a0, b0, st_q[0]); st_q[1] = fmaf(a1, b1, st_q[1]);
-            st_q[2] = fmaf(a2, b2, st_q[2]); st_q[3] = fmaf(a3, b3, st_q[3]);
+            st_q[0] = fmaf(a0, a0, st_q[0]); st_q[1] = fmaf(a1, a1, st_q[1]);
+            st_q[2] = fmaf(a2, a2, st_q[2]); st_q[3] = fmaf(a3, a3, st_q[3]);
           }
         }
       }
@@ -1012,10 +882,7 @@ __global__ void IL_KERNEL_BOUNDS conv3_il_kernel(const __grid_constant__ IlKPara
       if (acc == 0) acc_phase ^= 1;
     }
     IL_PROF(prof_acc[1] = clock64() - t_start;)  // last tile's store handed to the TMA engine (+ statistics loop)
-    if (gtid == 0) {
-      // the shared-memory source must have been read before the CTA retires; the global writes complete with the grid
-      if (p.opt & 2) tma_store_wait_read<0>(); else tma_store_wait_all<0>();
-    }
+    if (gtid == 0) tma_store_wait_all<0>();
     IL_PROF(prof_acc[2] = clock64() - t_start;)
     if (stats != nullptr) {
       // lanes l and l+16 hold the same channels of different rows: fold them, then one row of partials per warp
@@ -1292,26 +1159,8 @@ int encode_map_bf16(CUtensorMap* map, const void* ptr, int rank, const uint64_t*
   return 0;
 }
 
-// Concurrency share: when K independent launch chains (the K generators' graph branches) run side by side, every
-// persistent kernel sizes its grid for 1/K of the SMs so that the chains really overlap instead of queueing for whole-GPU
-// grids (each kernel pays its launch ramp / pipeline fill / tail while the other chains keep the remaining SMs busy).
-static int g_sm_share = 0;
-void set_sm_share(int k) { g_sm_share = k < 1 ? 1 : k; }
-static int sm_share() {
-  if (g_sm_share == 0) {
-    const char* ev = getenv("SRG_SM_SHARE");
-    g_sm_share = ev ? atoi(ev) : 1;
-    if (g_sm_share < 1) g_sm_share = 1;
-  }
-  return g_sm_share;
-}
 static int g_num_sms = 0;
-static int num_sms();
 int sm_budget() {
-  int b = num_sms() / sm_share();
-  return b < 1 ? 1 : b;
-}
-static int num_sms() {
   if (g_num_sms == 0) {
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1337,36 +1186,21 @@ static int launch_instance(const typename KParamsOf<BLOCK_N>::type& p, dim3 grid
   return 0;
 }
 
-// conv3_il applies to the plain 3x3 / 64-input-channel launches (trunk fprop + dgrad, up-conv fprop); everything else
-// (multi-view inputs, 9x9 row pairs, fold9, fp32 outputs, product statistics) stays on the generic kernel.
-static bool conv3_il_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* ev = getenv("SRG_CONV_IL");
-    on = (ev != nullptr && ev[0] == '0') ? 0 : 1;
-  }
-  return on != 0;
-}
-// SRG_CONV_IL_WIDE=0: load one 8-pixel half strip per column shift instead of one 10-pixel strip for all three
-static bool conv3_il_wide_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* ev = getenv("SRG_CONV_IL_WIDE");
-    on = (ev != nullptr && ev[0] == '0') ? 0 : 1;
-  }
-  return on != 0;
-}
 static int g_variant_override = 0;
 int set_conv_variant(int variant) {
+  if (variant != 0 && variant != 1) { set_error("set_conv_variant: variant %d is not 0 (automatic) or 1 (generic)", variant); return -1; }
   const int old = g_variant_override;
-  g_variant_override = (variant >= 0 && variant <= 3) ? variant : 0;
+  g_variant_override = variant;
   return old;
 }
 static int effective_variant(const ConvGemmArgs& a) { return a.variant != 0 ? a.variant : g_variant_override; }
+// conv3_il applies to the plain 3x3 / 64-input-channel launches (trunk fprop + dgrad, up-conv fprop) whose three column
+// shifts are -1, 0, +1 (one 10-pixel strip starting at w0 - 1); everything else (multi-view inputs, 9x9 row pairs, fold9,
+// fp32 outputs) stays on the generic kernel.
 static bool use_conv3_il(const ConvGemmArgs& a) {
-  const int variant = effective_variant(a);
-  if (variant == 1 || (variant == 0 && !conv3_il_enabled())) return false;
+  if (effective_variant(a) == 1) return false;
   return a.TH == 16 && a.TW == 8 && a.block_n == 64 && a.n_strips == 3 && a.n_taps == 3 && a.strip_dh == -1 &&
+         a.strip_dw[0] == -1 && a.strip_dw[1] == 0 && a.strip_dw[2] == 1 &&
          a.strip_rows == 18 && a.tap_row[0] == 0 && a.tap_row[1] == 1 && a.tap_row[2] == 2 && a.n_views == 1 &&
          a.views[0].channels == 64 && a.in_H == a.H && a.in_W == a.W && a.H >= 2 &&
          (a.out_mode == OUT_NHWC || a.out_mode == OUT_PIXEL_SHUFFLE) &&
@@ -1393,7 +1227,7 @@ static int launch_conv3_il(const ConvGemmArgs* as, int n, cudaStream_t stream) {
     if (o.N != a.N || o.H != a.H || o.W != a.W || o.in_H != a.in_H || o.in_W != a.in_W || o.cout_total != 64 || a.cout_total != 64 ||
         o.out_mode != OUT_NHWC || a.out_mode != OUT_NHWC || o.act != a.act || o.slope != a.slope || o.exclusive != a.exclusive ||
         (o.residual != nullptr) != (a.residual != nullptr) || (o.mask_src != nullptr) != (a.mask_src != nullptr) ||
-        (o.stats != nullptr) != (a.stats != nullptr) || (o.stats_y != nullptr) != (a.stats_y != nullptr) ||
+        (o.stats != nullptr) != (a.stats != nullptr) ||
         o.views[0].stride_w != a.views[0].stride_w || o.views[0].stride_h != a.views[0].stride_h ||
         o.views[0].stride_n != a.views[0].stride_n || o.strip_dw[0] != a.strip_dw[0] || o.strip_dw[1] != a.strip_dw[1] ||
         o.strip_dw[2] != a.strip_dw[2] || effective_variant(o) != effective_variant(a) || a.prof != nullptr) {
@@ -1425,34 +1259,25 @@ static int launch_conv3_il(const ConvGemmArgs* as, int n, cudaStream_t stream) {
   p.aux_mode = a.residual ? 1 : (a.mask_src ? 2 : 0);
   const uint32_t fixed_bytes = kIlWBytes + 2 * kTileOutBytes + (has_aux ? 2 * kTileOutBytes : 0) + 768 +
                                (a.stats != nullptr ? 16 * 128 * 4 : 0);
-  // the wide form needs the three column shifts to be -1, 0, +1 (one 10-pixel strip starting at w0 - 1)
-  const int variant = effective_variant(a);
-  const bool wide = (variant == 3 || (variant == 0 && conv3_il_wide_enabled())) && a.strip_dw[0] == -1 && a.strip_dw[1] == 0 && a.strip_dw[2] == 1;
-  const uint32_t stage_bytes = wide ? kIlWideStage : kIlHalfStrip;
-  // Leave 44 KB of the SM's shared memory to CTAs of other graph branches (chan_reduce, finalize, loss passes need 8-18 KB):
-  // measured 11.27 -> 11.14 ms per cfg2 step; the shallower pipeline (3 / 2 stages) costs nothing (profiles/r01_notes.md).
-  static int reserve_kb = -1;
-  if (reserve_kb < 0) { const char* ev = getenv("SRG_IL_SMEM_RESERVE_KB"); reserve_kb = ev ? atoi(ev) : 44; }
-  // launches with a residual / mask tile keep everything (they would be down to two stages: the operand prefetch of the
-  // next tile could not start before half of the current tile's MMAs have retired; probe: 14.0 -> 12.8 us at cfg2)
-  static int aux_reserve = -1;
-  if (aux_reserve < 0) { const char* ev = getenv("SRG_IL_AUX_RESERVE"); aux_reserve = ev ? atoi(ev) : 0; }
-  const int reserve = a.exclusive ? 0 : ((has_aux && !aux_reserve) ? 0 : reserve_kb);
-  int stages = int((227 * 1024 - reserve * 1024 - 1024 - fixed_bytes) / stage_bytes);
-  static int stage_cap = -1;
-  if (stage_cap < 0) { const char* ev = getenv("SRG_IL_STAGE_CAP"); stage_cap = ev ? atoi(ev) : 8; }
-  if (!a.exclusive && stages > stage_cap) stages = stage_cap;
-  if (stages > 8) stages = 8;
+  // Training launches leave 44 KB of the SM's shared memory to CTAs of other graph branches (chan_reduce, finalize, loss
+  // passes need 8-18 KB): measured 11.27 -> 11.14 ms per cfg2 step; the shallower pipeline (3 / 2 stages) costs nothing
+  // (profiles/r01_notes.md).  Launches with a residual / mask tile keep everything (they would be down to two stages: the
+  // operand prefetch of the next tile could not start before half of the current tile's MMAs have retired; probe: 14.0 ->
+  // 12.8 us at cfg2), and so do inference (exclusive) launches.
+  constexpr int kIlSmemReserveKb = 44;
+  const int reserve_kb = (a.exclusive || has_aux) ? 0 : kIlSmemReserveKb;
+  int stages = int((227 * 1024 - reserve_kb * 1024 - 1024 - fixed_bytes) / kIlWideStage);
+  if (stages > 8) stages = 8;      // full[] / empty[] hold 8 barriers
   if (stages < 2) stages = 2;
   p.n_stages = stages;
-  const size_t smem_bytes = 1024 + fixed_bytes + size_t(stages) * stage_bytes;
+  const size_t smem_bytes = 1024 + fixed_bytes + size_t(stages) * kIlWideStage;
 
   for (int g = 0; g < n; ++g) {
     const ConvGemmArgs& ag = as[g];
     const InView& iv = ag.views[0];
     for (int par = 0; par < 2; ++par) {
       int rc = encode_parity_map(&p.in_map[2 * g + par], iv.ptr, 64, a.in_W, a.in_H, a.N, iv.stride_w, iv.stride_h, iv.stride_n, par, 17,
-                                 wide ? 10 : 8);
+                                 10);
       if (rc) return rc;
     }
     {
@@ -1491,45 +1316,29 @@ static int launch_conv3_il(const ConvGemmArgs* as, int n, cudaStream_t stream) {
     }
     p.bias[g] = ag.bias; p.scale[g] = ag.scale;
     p.stats[g] = ag.stats;
-    p.stats_y[g] = reinterpret_cast<const uint32_t*>(ag.stats_y);
   }
   p.act = a.act; p.slope = a.slope;
   p.out_mode = a.out_mode;
   // training launches (not exclusive): the output is read by the statistics / apply passes right behind this kernel (keep
-  // it in L2 ahead of streaming data); a mask / residual tile is dead after this read
-  const bool hints = !a.exclusive && l2_hints() >= 2;
-  p.pol_out = hints ? kL2EvictLast : kL2EvictNormal;
-  p.pol_aux = hints ? kL2EvictFirst : kL2EvictNormal;
-  // the operand tensor is not read again before the weight gradients at the end of backward (neighbouring tiles re-read
-  // their halo within microseconds, long before capacity pressure evicts it)
-  p.pol_in = (!a.exclusive && l2_hints() >= 3) ? kL2EvictFirst : kL2EvictNormal;
+  // it in L2 ahead of streaming data); a mask / residual tile is dead after this read.  The operand tensor is not read again
+  // before the weight gradients at the end of backward (neighbouring tiles re-read their halo within microseconds, long
+  // before capacity pressure evicts it)
+  p.pol_out = a.exclusive ? kL2EvictNormal : kL2EvictLast;
+  p.pol_aux = a.exclusive ? kL2EvictNormal : kL2EvictFirst;
+  p.pol_in = a.exclusive ? kL2EvictNormal : kL2EvictFirst;
   p.prof = reinterpret_cast<long long*>(a.prof);
-  static int il_opt = -1;
-  if (il_opt < 0) { const char* ev = getenv("SRG_IL_OPT"); il_opt = ev ? atoi(ev) : 1; }
-  p.opt = a.exclusive ? (il_opt & ~1) : il_opt;
+  p.ramp = a.exclusive ? 0 : 1;
   static DeviceOnce attr_set;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(conv3_il_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(conv3_il_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_il_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return int(e); }
     attr_set = true;
   }
   const dim3 grid(p.ctas_per_block * p.n_blocks * n);
-  const int pdl = a.exclusive ? 2 : (pdl_conv() ? 1 : 0);
-  const bool ys = a.stats != nullptr && a.stats_y != nullptr;
-  if (n > 1 && ys && !wide) { set_error("conv3_il: a grouped launch with a second statistics factor needs the wide form"); return -18; }
-  cudaError_t e = n > 1 ? (wide ? (ys ? launch_opt_pdl(pdl, conv3_il_kernel<true, true, true>, grid, dim3(kIlThreads), smem_bytes, stream, p)
-                                      : launch_opt_pdl(pdl, conv3_il_kernel<true, false, true>, grid, dim3(kIlThreads), smem_bytes, stream, p))
-                                : launch_opt_pdl(pdl, conv3_il_kernel<false, false, true>, grid, dim3(kIlThreads), smem_bytes, stream, p))
-                  : wide ? (ys ? launch_opt_pdl(pdl, conv3_il_kernel<true, true>, grid, dim3(kIlThreads), smem_bytes, stream, p)
-                             : launch_opt_pdl(pdl, conv3_il_kernel<true, false>, grid, dim3(kIlThreads), smem_bytes, stream, p))
-                       : (ys ? launch_opt_pdl(pdl, conv3_il_kernel<false, true>, grid, dim3(kIlThreads), smem_bytes, stream, p)
-                             : launch_opt_pdl(pdl, conv3_il_kernel<false, false>, grid, dim3(kIlThreads), smem_bytes, stream, p));
+  void (*const kernel)(IlKParams) = n > 1 ? conv3_il_kernel<true> : conv3_il_kernel<false>;
+  cudaError_t e = a.exclusive ? launch_pdl_exclusive(kernel, grid, dim3(kIlThreads), smem_bytes, stream, p)
+                              : launch_pdl(kernel, grid, dim3(kIlThreads), smem_bytes, stream, p);
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) { set_error("conv3_il launch: %s", cudaGetErrorString(e)); return int(e); }
   count_launch();
@@ -1541,7 +1350,6 @@ static int launch_conv3_il(const ConvGemmArgs* as, int n, cudaStream_t stream) {
 static bool use_conv9_rows(const ConvGemmArgs& a) {
   const int variant = effective_variant(a);
   if (variant == 1 || a.out_mode != OUT_FOLD9_NCHW) return false;
-  if (variant == 0 && !conv3_il_enabled()) return false;
   if (a.block_n != 32 || a.cout_total != 32 || a.n_strips != 1 || a.n_taps != 9 || a.strip_dh != -4 || a.strip_dw[0] != 0) return false;
   for (int r = 0; r < 9; ++r) if (a.tap_row[r] != r) return false;
   return a.n_views == 1 && a.views[0].channels == 64 && a.in_H == a.H && a.in_W == a.W && a.residual == nullptr &&
@@ -1747,10 +1555,9 @@ int launch_conv_gemm(const ConvGemmArgs& a, cudaStream_t stream) {
     p.aux_map = p.in_map[0];
   }
   p.bias = a.bias; p.scale = a.scale; p.act = a.act; p.slope = a.slope;
-  p.pol_in = (!a.exclusive && l2_hints() >= 4) ? kL2EvictFirst : kL2EvictNormal;
+  p.pol_in = kL2EvictNormal;
   p.out = a.out; p.out_mode = a.out_mode;
   p.stats = a.stats;
-  p.stats_y = reinterpret_cast<const uint32_t*>(a.stats_y);
   p.prof = reinterpret_cast<long long*>(a.prof);
 
   const dim3 grid(p.ctas_per_block * p.n_blocks);

@@ -78,13 +78,11 @@ struct ConvGemmArgs {
   int out_mode;
   int exclusive;             // 1: nothing else runs beside this launch (inference): conv3_il takes all shared memory for its
                              // pipeline instead of leaving 44 KB to co-resident CTAs of other graph branches
-  int variant;               // 0: pick the kernel automatically (row-interleaved conv3_il for plain 3x3 / 64-channel launches
-                             // unless SRG_CONV_IL=0), 1: force the generic strip kernel, 2: conv3_il with one 8-pixel half strip
-                             // per column shift, 3: conv3_il with one 10-pixel half strip for all three shifts (default form)
+  int variant;               // 0: pick the kernel automatically (row-interleaved conv3_il for plain 3x3 / 64-channel launches,
+                             // conv9_rows for the plain fold9 conv), 1: force the generic strip kernel (the reference the
+                             // specialised kernels are tested against)
   float* stats;              // optional (OUT_NHWC, cout 64): per-CTA column sums of the STORED bf16 tile values,
                              // float [conv_gemm_grid(a)][128] = {sum over valid pixels [64], sum of squares [64]}
-  const void* stats_y;       // optional with `stats`: bf16 tensor of the output's geometry; the second 64 columns then hold
-                             // sum(out * stats_y) instead of sum(out^2) (BatchNorm backward: sum dz, sum dz*y)
   void* prof;                // optional debug timers: int64 [grid][3][6]
   const FoldScatter* scatter;  // optional (OUT_FOLD9_NCHW only, host memory): the store layout (default fp32 NCHW)
   // fold9: tile columns overlap; valid output columns per tile = TW-8
@@ -155,12 +153,12 @@ __host__ __device__ inline C9Window c9_window(int ri) {
   return w;
 }
 
-// process-wide override of ConvGemmArgs::variant for launches that leave it 0 (parity tests, A/B runs); returns the old value
+// process-wide override of ConvGemmArgs::variant for launches that leave it 0 (parity tests): 0 or 1; returns the old
+// value, or a negative code (set_error) for any other value, leaving the override unchanged
 int set_conv_variant(int variant);
 
-// SMs a persistent kernel may size its grid for: device SM count / concurrency share (set_sm_share, SRG_SM_SHARE)
+// SMs a persistent kernel sizes its grid for: the device's SM count
 int sm_budget();
-void set_sm_share(int k);
 
 // total kernels launched by this library in this process (bench bookkeeping: "gpu_launches")
 void count_launch(int n = 1);

@@ -43,29 +43,19 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
 // ------------------------------------------------------------------------------------------------
 // per-channel reductions: thread = (pixel lane, channel group of 8)
 // ------------------------------------------------------------------------------------------------
-static int env_int(const char* name, int dflt) {
-  const char* ev = getenv(name);
-  return (ev != nullptr && ev[0] != '\0') ? atoi(ev) : dflt;
-}
-// developer knobs (read once): CTAs per SM of the elementwise / reduction passes.  Fewer CTAs leave HBM bandwidth to a
-// tensor-core kernel of another graph branch running beside them (profiles/r02_notes.md)
-static int red_per_sm() { static int v = -1; if (v < 0) v = env_int("SRG_RED_PER_SM", 2); return v < 1 ? 1 : v; }
-static int ew_per_sm() { static int v = -1; if (v < 0) v = env_int("SRG_EW_PER_SM", 4); return v < 1 ? 1 : v; }
-static int fin_per_sm() { static int v = -1; if (v < 0) v = env_int("SRG_FIN_PER_SM", 2); return v < 1 ? 1 : v; }
-// L2 eviction priorities (SRG_L2_HINTS: 0 none, 1 BatchNorm chain, 2 + conv outputs / aux tiles, 3 (default) + conv operands
-// and the block-input read, 4 + weight-gradient and generic-kernel operands).  Per trunk layer the three generators
-// stream ~450 MB through a 126 MB L2; without hints the tensors with a near reuse (the conv output the reduction and the
-// apply pass read next, the apply output the next conv reads) are evicted by data that is dead after its access.
-int l2_hints() { static int v = -1; if (v < 0) v = env_int("SRG_L2_HINTS", 3); return v; }
-static int red_threads() { static int v = -1; if (v < 0) v = env_int("SRG_RED_THREADS", 512) == 256 ? 256 : 512; return v; }
+// CTAs per SM of the reduction / elementwise passes.  Fewer CTAs leave HBM bandwidth to a tensor-core kernel of another
+// graph branch running beside them (profiles/r02_notes.md)
+constexpr int kRedPerSm = 2;
+constexpr int kEwPerSm = 4;
+constexpr int kRedThreads = 512;    // threads per chan_reduce_kernel block (see there)
 int reduce_blocks(int64_t pixels) {
   int64_t b = (pixels + 32 * 8 - 1) / (32 * 8);
   if (b < 1) b = 1;
-  const int cap = red_per_sm() * sm_budget() < kRedBlocksMax ? red_per_sm() * sm_budget() : kRedBlocksMax;
+  const int cap = kRedPerSm * sm_budget() < kRedBlocksMax ? kRedPerSm * sm_budget() : kRedBlocksMax;
   if (b > cap) {
     // every block the same number of 128-pixel rounds (4 pixels of a thread in flight per round): no block runs a tail of
     // single-pixel rounds after the others have finished (cfg2: 288 blocks x 4 rounds instead of 296 x 3 + up to 3 singles)
-    const int64_t per_round = red_threads() / 2;      // T / 8 pixels x 4 in flight
+    const int64_t per_round = kRedThreads / 2;      // T / 8 pixels x 4 in flight
     const int64_t rounds = (pixels + per_round - 1) / per_round;
     const int64_t per_block = (rounds + cap - 1) / cap;
     b = (rounds + per_block - 1) / per_block;
@@ -73,12 +63,13 @@ int reduce_blocks(int64_t pixels) {
   return int(b);
 }
 
-// T threads per block = T / 8 pixels per round-slot.  T = 512 (two blocks per SM) keeps 32 warps x 8 loads in flight per SM:
-// at cfg2 every block then runs 2 dependent rounds instead of 4 (the pass is bound by the latency of its rounds).
-template <bool TWO, int T>
-__global__ void __launch_bounds__(T) chan_reduce_kernel(const uint4* __restrict__ a, const uint4* __restrict__ b,
-                                                        int64_t pixels, float* __restrict__ partials, uint64_t pol) {
-  constexpr int PR = T / 8;       // pixels per round-slot
+// kRedThreads threads per block = kRedThreads / 8 pixels per round-slot.  512 threads (two blocks per SM) keep 32 warps x 8
+// loads in flight per SM: at cfg2 every block then runs 2 dependent rounds instead of 4 (the pass is bound by the latency of
+// its rounds).
+template <bool TWO>
+__global__ void __launch_bounds__(kRedThreads) chan_reduce_kernel(const uint4* __restrict__ a, const uint4* __restrict__ b,
+                                                                  int64_t pixels, float* __restrict__ partials, uint64_t pol) {
+  constexpr int PR = kRedThreads / 8;       // pixels per round-slot
   __shared__ float red[PR][129];
   pdl_trigger();
   pdl_wait();
@@ -134,8 +125,7 @@ __global__ void __launch_bounds__(T) chan_reduce_kernel(const uint4* __restrict_
   }
 }
 
-// ---- fused reduction + finalize: the last block to finish (atomic ticket) sums the block partials in a fixed order
-// and runs the per-channel finalize in the same launch (3 launches -> 1 when no cross-GPU all-reduce sits in between).
+// per-channel finalize of the fixed-order sums s1 = {sum a}, s2 = {sum a*a or sum a*b} (ReduceFinalize::mode)
 __device__ __forceinline__ void finalize_channels(const ReduceFinalize& f, int c, double s1, double s2) {
   if (f.mode == RF_BN_FWD) {
     const double mean = s1 / f.count;
@@ -177,108 +167,6 @@ __device__ __forceinline__ void finalize_channels(const ReduceFinalize& f, int c
   }
 }
 
-template <bool TWO, int T>
-__global__ void __launch_bounds__(T) chan_reduce_final_kernel(const uint4* __restrict__ a, const uint4* __restrict__ b,
-                                                                int64_t pixels, float* __restrict__ partials,
-                                                                unsigned int* __restrict__ ticket, const ReduceFinalize f,
-                                                                uint64_t pol) {
-  constexpr int PR = T / 8;       // pixels per round-slot (as chan_reduce_kernel)
-  constexpr int RL = T / 32;      // row lanes of the last block's fixed-order sum
-  __shared__ float red[PR][129];
-  __shared__ bool is_last;
-  static_assert(sizeof(float) * PR * 129 >= sizeof(double) * RL * 128, "the fp64 staging reuses the float rows");
-  pdl_trigger();
-  pdl_wait();
-  const int cg = threadIdx.x & 7;
-  const int lane_p = threadIdx.x >> 3;
-  float s1[8], s2[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) s1[e] = s2[e] = 0.f;
-  const int64_t stride = int64_t(gridDim.x) * PR;
-  int64_t p = int64_t(blockIdx.x) * PR + lane_p;
-  for (; p + 3 * stride < pixels; p += 4 * stride) {      // same loop (and per-thread accumulation order) as chan_reduce_kernel
-    uint4 ra[4], rb[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      ra[u] = ldg_hint_u4(a + (p + u * stride) * 8 + cg, pol);
-      if (TWO) rb[u] = ldg_hint_u4(b + (p + u * stride) * 8 + cg, pol);
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      float fa[8], fb[8];
-      unpack8(ra[u], fa);
-      if (TWO) unpack8(rb[u], fb);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        s1[e] += fa[e];
-        s2[e] += TWO ? fa[e] * fb[e] : fa[e] * fa[e];
-      }
-    }
-  }
-  for (; p < pixels; p += stride) {
-    float fa[8], fb[8];
-    unpack8(a[p * 8 + cg], fa);
-    if (TWO) unpack8(b[p * 8 + cg], fb);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      s1[e] += fa[e];
-      s2[e] += TWO ? fa[e] * fb[e] : fa[e] * fa[e];
-    }
-  }
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    red[lane_p][cg * 8 + e] = s1[e];
-    red[lane_p][64 + cg * 8 + e] = s2[e];
-  }
-  __syncthreads();
-  if (threadIdx.x < 128) {
-    float acc = 0.f;
-#pragma unroll 8
-    for (int l = 0; l < PR; ++l) acc += red[l][threadIdx.x];
-    partials[size_t(blockIdx.x) * 128 + threadIdx.x] = acc;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!is_last) return;
-  // the last block to finish: fixed-order fp64 sum of every block's row (RL row lanes x 32 column quads), then the finalize
-  __threadfence();
-  double* dred = reinterpret_cast<double*>(&red[0][0]);        // [RL][128] doubles over the dead float rows
-  const int c4 = threadIdx.x & 31, rl = threadIdx.x >> 5;
-  const float4* src = reinterpret_cast<const float4*>(partials) + c4;
-  const int rows = int(gridDim.x);
-  double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-  int r = rl;
-  for (; r + 4 * RL < rows; r += 5 * RL) {
-    const float4 v0 = __ldcg(src + size_t(r) * 32), v1 = __ldcg(src + size_t(r + RL) * 32), v2 = __ldcg(src + size_t(r + 2 * RL) * 32);
-    const float4 v3 = __ldcg(src + size_t(r + 3 * RL) * 32), v4 = __ldcg(src + size_t(r + 4 * RL) * 32);
-    a0 += double(v0.x); a1 += double(v0.y); a2 += double(v0.z); a3 += double(v0.w);
-    a0 += double(v1.x); a1 += double(v1.y); a2 += double(v1.z); a3 += double(v1.w);
-    a0 += double(v2.x); a1 += double(v2.y); a2 += double(v2.z); a3 += double(v2.w);
-    a0 += double(v3.x); a1 += double(v3.y); a2 += double(v3.z); a3 += double(v3.w);
-    a0 += double(v4.x); a1 += double(v4.y); a2 += double(v4.z); a3 += double(v4.w);
-  }
-  for (; r < rows; r += RL) {
-    const float4 v = __ldcg(src + size_t(r) * 32);
-    a0 += double(v.x); a1 += double(v.y); a2 += double(v.z); a3 += double(v.w);
-  }
-  __syncthreads();
-  dred[rl * 128 + c4 * 4 + 0] = a0; dred[rl * 128 + c4 * 4 + 1] = a1;
-  dred[rl * 128 + c4 * 4 + 2] = a2; dred[rl * 128 + c4 * 4 + 3] = a3;
-  __syncthreads();
-  double t = 0.0;
-  if (threadIdx.x < 128) {
-#pragma unroll
-    for (int i = 0; i < RL; ++i) t += dred[i * 128 + threadIdx.x];
-  }
-  __syncthreads();
-  if (threadIdx.x < 128) dred[threadIdx.x] = t;
-  __syncthreads();
-  if (threadIdx.x < 64) finalize_channels(f, threadIdx.x, dred[threadIdx.x], dred[64 + threadIdx.x]);
-  if (threadIdx.x == 0) *ticket = 0u;
-}
-
 // partials [rows][128] -> fixed-order column sums (8 row lanes x 128 columns, 4 independent accumulators per thread) ->
 // per-channel finalize, one 1024-thread block.
 __global__ void __launch_bounds__(1024) partials_finalize_kernel(const float* __restrict__ partials, int rows,
@@ -312,35 +200,14 @@ int launch_partials_sums(const float* partials, int rows, double* sums, cudaStre
   return 0;
 }
 
-int launch_chan_reduce_final(const void* a, const void* b, int64_t pixels, float* partials, unsigned int* ticket,
-                             const ReduceFinalize& f, cudaStream_t st) {
-  const int blocks = reduce_blocks(pixels);
-  const uint64_t pol = (b && l2_hints()) ? kL2EvictLast : kL2EvictNormal;
-  const uint4* aa = reinterpret_cast<const uint4*>(a);
-  const uint4* bb = reinterpret_cast<const uint4*>(b);
-  if (red_threads() == 512) {
-    if (b) launch_pdl(chan_reduce_final_kernel<true, 512>, dim3(blocks), dim3(512), 0, st, aa, bb, pixels, partials, ticket, f, pol);
-    else launch_pdl(chan_reduce_final_kernel<false, 512>, dim3(blocks), dim3(512), 0, st, aa, bb, pixels, partials, ticket, f, pol);
-  } else {
-    if (b) launch_pdl(chan_reduce_final_kernel<true, 256>, dim3(blocks), dim3(256), 0, st, aa, bb, pixels, partials, ticket, f, pol);
-    else launch_pdl(chan_reduce_final_kernel<false, 256>, dim3(blocks), dim3(256), 0, st, aa, bb, pixels, partials, ticket, f, pol);
-  }
-  SRG_LAUNCH_CHECK("chan_reduce_final");
-  return 0;
-}
-
 int launch_chan_reduce(const void* a, const void* b, int64_t pixels, float* partials, cudaStream_t st) {
   const int blocks = reduce_blocks(pixels);
-  const uint64_t pol = (b && l2_hints()) ? kL2EvictLast : kL2EvictNormal;
+  // BatchNorm backward (b = y): both tensors are read again by the apply pass right behind this one
+  const uint64_t pol = b ? kL2EvictLast : kL2EvictNormal;
   const uint4* aa = reinterpret_cast<const uint4*>(a);
   const uint4* bb = reinterpret_cast<const uint4*>(b);
-  if (red_threads() == 512) {
-    if (b) launch_pdl(chan_reduce_kernel<true, 512>, dim3(blocks), dim3(512), 0, st, aa, bb, pixels, partials, pol);
-    else launch_pdl(chan_reduce_kernel<false, 512>, dim3(blocks), dim3(512), 0, st, aa, bb, pixels, partials, pol);
-  } else {
-    if (b) launch_pdl(chan_reduce_kernel<true, 256>, dim3(blocks), dim3(256), 0, st, aa, bb, pixels, partials, pol);
-    else launch_pdl(chan_reduce_kernel<false, 256>, dim3(blocks), dim3(256), 0, st, aa, bb, pixels, partials, pol);
-  }
+  if (b) launch_pdl(chan_reduce_kernel<true>, dim3(blocks), dim3(kRedThreads), 0, st, aa, bb, pixels, partials, pol);
+  else launch_pdl(chan_reduce_kernel<false>, dim3(blocks), dim3(kRedThreads), 0, st, aa, bb, pixels, partials, pol);
   SRG_LAUNCH_CHECK("chan_reduce");
   return 0;
 }
@@ -457,8 +324,8 @@ template <bool RELU, bool SKIP>
 __global__ void __launch_bounds__(256) bn_apply_kernel(const uint4* __restrict__ y, const float* __restrict__ scale,
                                                        const float* __restrict__ shift, const uint4* __restrict__ skip,
                                                        uint4* __restrict__ out, int64_t n_vec, uint64_t pol_y, uint64_t pol_out,
-                                                       uint64_t pol_skip, int late) {
-  if (!late) pdl_trigger();
+                                                       uint64_t pol_skip) {
+  pdl_trigger();
   pdl_wait();
   const int cg = threadIdx.x & 7;  // blockDim is a multiple of 8 and the grid stride too
   float sc[8], sh[8];
@@ -497,18 +364,17 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const uint4* __restrict__
       }
     }
   }
-  if (late) pdl_trigger();
 }
 static int ew_blocks(int64_t n_vec) {
   int64_t b = (n_vec + 255) / 256;
-  if (b > sm_budget() * ew_per_sm()) b = sm_budget() * ew_per_sm();
+  if (b > sm_budget() * kEwPerSm) b = sm_budget() * kEwPerSm;
   if (b < 1) b = 1;
   return int(b);
 }
 // grid of a pass whose threads take U vectors per round: every block the same number of rounds (cfg2: 576 blocks x 2 or 4
 // full rounds instead of 592 blocks with a mostly-empty last round)
 static int ew_blocks_rounds(int64_t n_vec, int U) {
-  const int64_t cap = int64_t(sm_budget()) * ew_per_sm();
+  const int64_t cap = int64_t(sm_budget()) * kEwPerSm;
   const int64_t rounds = (n_vec + 256 * U - 1) / (256 * U);
   if (rounds <= cap) return int(rounds < 1 ? 1 : rounds);
   const int64_t per_block = (rounds + cap - 1) / cap;
@@ -521,13 +387,13 @@ int launch_bn_apply(const void* y, const float* scale, const float* shift, const
   const uint4* yy = reinterpret_cast<const uint4*>(y);
   const uint4* kk = reinterpret_cast<const uint4*>(skip);
   uint4* oo = reinterpret_cast<uint4*>(out);
-  // y is not read again before the backward pass (evict first); the output is the next convolution's operand (keep)
-  const uint64_t py = l2_hints() ? kL2EvictFirst : kL2EvictNormal, po = l2_hints() ? kL2EvictLast : kL2EvictNormal;
-  const uint64_t pk = l2_hints() >= 3 ? kL2EvictFirst : kL2EvictNormal;      // the block input: last read of the forward pass
-  if (relu && skip) launch_pdl(bn_apply_kernel<true, true>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk, pdl_ew_late());
-  else if (relu) launch_pdl(bn_apply_kernel<true, false>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk, pdl_ew_late());
-  else if (skip) launch_pdl(bn_apply_kernel<false, true>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk, pdl_ew_late());
-  else launch_pdl(bn_apply_kernel<false, false>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk, pdl_ew_late());
+  // y is not read again before the backward pass (evict first); the output is the next convolution's operand (keep); the
+  // block input (skip) is read for the last time in the forward pass
+  const uint64_t py = kL2EvictFirst, po = kL2EvictLast, pk = kL2EvictFirst;
+  if (relu && skip) launch_pdl(bn_apply_kernel<true, true>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk);
+  else if (relu) launch_pdl(bn_apply_kernel<true, false>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk);
+  else if (skip) launch_pdl(bn_apply_kernel<false, true>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk);
+  else launch_pdl(bn_apply_kernel<false, false>, dim3(blocks), dim3(256), 0, st, yy, scale, shift, kk, oo, n_vec, py, po, pk);
   SRG_LAUNCH_CHECK("bn_apply");
   return 0;
 }
@@ -564,8 +430,8 @@ int launch_bn_bwd_finalize(const double* sums, double count, const float* gamma,
 __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const uint4* __restrict__ dout, const uint4* __restrict__ y,
                                                            const float* __restrict__ cA, const float* __restrict__ cB,
                                                            const float* __restrict__ cC, uint4* __restrict__ dy,
-                                                           int64_t n_vec, uint64_t pol_in, uint64_t pol_out, int late) {
-  if (!late) pdl_trigger();
+                                                           int64_t n_vec, uint64_t pol_in, uint64_t pol_out) {
+  pdl_trigger();
   pdl_wait();
   const int cg = threadIdx.x & 7;
   float a[8], b[8], c[8];
@@ -596,7 +462,6 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const uint4* __restri
       stg_hint_u4(dy + i + stride, pack8(d), pol_out);
     }
   }
-  if (late) pdl_trigger();
 }
 int launch_bn_bwd_apply(const void* dout, const void* y, const float* coefA, const float* coefB, const float* coefC,
                         void* dy, int64_t pixels, cudaStream_t st) {
@@ -606,209 +471,9 @@ int launch_bn_bwd_apply(const void* dout, const void* y, const float* coefA, con
              // dz and y are (all but) dead after this pass.  Measured: keeping bn2's dz, which the block's conv1 dgrad reads
              // once more as the skip gradient, at high priority costs 0.15 ms per step, and discarding the dead bn1 dz lines
              // (discard.global.L2) buys nothing (profiles/r02_notes.md)
-             l2_hints() ? kL2EvictFirst : kL2EvictNormal,
-             l2_hints() ? kL2EvictLast : kL2EvictNormal,       // dy is the next dgrad's operand
-             pdl_ew_late());
+             kL2EvictFirst,
+             kL2EvictLast);      // dy is the next dgrad's operand
   SRG_LAUNCH_CHECK("bn_bwd_apply");
-  return 0;
-}
-
-// ---- BatchNorm apply / backward apply with the statistics finalize folded in ---------------------------------------
-// The separate one-block finalize launch between the producer of the [rows][128] partial sums and the apply pass is pure
-// latency on the per-generator dependency chain (measured in the replayed graph: ~5 us of execution + ~5 us of
-// dependent-launch gaps per BatchNorm layer and direction).  Here every CTA of the apply pass re-reduces the partial rows
-// itself (<= 296 x 512 B, L2-resident, fixed order => every CTA and every run gets bit-identical sums), computes the
-// per-channel coefficients into shared memory and goes straight on to the elementwise pass; CTA 0 also writes what
-// later kernels need (coefficients, saved mean / inv-std, running statistics, weight / bias gradients).
-constexpr int kFinThreads = 512;
-__device__ __forceinline__ void block_partial_sums(const float* __restrict__ partials, int rows, double (*red)[128],
-                                                   double* sums) {
-  // 512 threads = 16 row lanes x 32 column quads; row lane rl sums rows rl, rl+16, ... in order (fp64)
-  const int c4 = threadIdx.x & 31, rl = threadIdx.x >> 5;
-  double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-  const float4* src = reinterpret_cast<const float4*>(partials) + c4;
-  int r = rl;
-  for (; r + 48 < rows; r += 64) {
-    const float4 v0 = __ldcg(src + size_t(r) * 32), v1 = __ldcg(src + size_t(r + 16) * 32);
-    const float4 v2 = __ldcg(src + size_t(r + 32) * 32), v3 = __ldcg(src + size_t(r + 48) * 32);
-    a0 += double(v0.x); a1 += double(v0.y); a2 += double(v0.z); a3 += double(v0.w);
-    a0 += double(v1.x); a1 += double(v1.y); a2 += double(v1.z); a3 += double(v1.w);
-    a0 += double(v2.x); a1 += double(v2.y); a2 += double(v2.z); a3 += double(v2.w);
-    a0 += double(v3.x); a1 += double(v3.y); a2 += double(v3.z); a3 += double(v3.w);
-  }
-  for (; r < rows; r += 16) {
-    const float4 v = __ldcg(src + size_t(r) * 32);
-    a0 += double(v.x); a1 += double(v.y); a2 += double(v.z); a3 += double(v.w);
-  }
-  red[rl][c4 * 4 + 0] = a0; red[rl][c4 * 4 + 1] = a1; red[rl][c4 * 4 + 2] = a2; red[rl][c4 * 4 + 3] = a3;
-  __syncthreads();
-  if (threadIdx.x < 128) {
-    double t = 0.0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i) t += red[i][threadIdx.x];
-    sums[threadIdx.x] = t;
-  }
-  __syncthreads();
-}
-
-template <bool RELU, bool SKIP>
-__global__ void __launch_bounds__(kFinThreads) bn_apply_fin_kernel(const uint4* __restrict__ y, const float* __restrict__ partials,
-                                                                   int rows, const ReduceFinalize f,
-                                                                   const uint4* __restrict__ skip, uint4* __restrict__ out,
-                                                                   int64_t n_vec) {
-  __shared__ double red[16][128];
-  __shared__ double sums[128];
-  __shared__ float coef[2][64];
-  pdl_trigger();
-  pdl_wait();
-  block_partial_sums(partials, rows, red, sums);
-  if (threadIdx.x < 64) {
-    const int c = threadIdx.x;
-    const double mean = sums[c] / f.count;
-    double var = sums[64 + c] / f.count - mean * mean;
-    if (var < 0.0) var = 0.0;
-    const float inv = float(1.0 / sqrt(var + double(f.eps)));
-    const float sc = f.gamma[c] * inv;
-    const float sh = f.beta[c] - float(mean) * sc;
-    coef[0][c] = sc;
-    coef[1][c] = sh;
-    if (blockIdx.x == 0) {
-      f.out0[c] = sc; f.out1[c] = sh; f.out2[c] = float(mean); f.out3[c] = inv;
-      if (f.running_mean != nullptr) {
-        const double unbiased = f.count > 1.0 ? var * (f.count / (f.count - 1.0)) : var;
-        f.running_mean[c] = (1.f - f.momentum) * f.running_mean[c] + f.momentum * float(mean);
-        f.running_var[c] = (1.f - f.momentum) * f.running_var[c] + f.momentum * float(unbiased);
-      }
-    }
-  }
-  __syncthreads();
-  const int cg = threadIdx.x & 7;
-  float sc[8], sh[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) { sc[e] = coef[0][cg * 8 + e]; sh[e] = coef[1][cg * 8 + e]; }
-  const int64_t stride = int64_t(gridDim.x) * kFinThreads;
-  int64_t i = int64_t(blockIdx.x) * kFinThreads + threadIdx.x;
-  for (; i + 3 * stride < n_vec; i += 4 * stride) {
-    uint4 ry[4], rk[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      ry[u] = y[i + u * stride];
-      if (SKIP) rk[u] = skip[i + u * stride];
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      float v[8], k[8];
-      unpack8(ry[u], v);
-      if (SKIP) unpack8(rk[u], k);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        float o = fmaf(v[e], sc[e], sh[e]);
-        if (RELU) o = fmaxf(o, 0.f);
-        if (SKIP) o += k[e];
-        v[e] = o;
-      }
-      out[i + u * stride] = pack8(v);
-    }
-  }
-  for (; i < n_vec; i += stride) {
-    float v[8], k[8];
-    unpack8(y[i], v);
-    if (SKIP) unpack8(skip[i], k);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      float o = fmaf(v[e], sc[e], sh[e]);
-      if (RELU) o = fmaxf(o, 0.f);
-      if (SKIP) o += k[e];
-      v[e] = o;
-    }
-    out[i] = pack8(v);
-  }
-}
-static int fin_blocks(int64_t n_vec) {
-  int64_t b = (n_vec + kFinThreads - 1) / kFinThreads;
-  if (b > fin_per_sm() * sm_budget()) b = fin_per_sm() * sm_budget();
-  if (b < 1) b = 1;
-  return int(b);
-}
-int launch_bn_apply_fin(const void* y, const float* partials, int rows, const ReduceFinalize& f, const void* skip, int relu,
-                        void* out, int64_t pixels, cudaStream_t st) {
-  if (f.mode != RF_BN_FWD) { set_error("bn_apply_fin: needs an RF_BN_FWD finalize descriptor"); return -40; }
-  const int64_t n_vec = pixels * 8;
-  const dim3 grid(fin_blocks(n_vec)), block(kFinThreads);
-  const uint4* yy = reinterpret_cast<const uint4*>(y);
-  const uint4* kk = reinterpret_cast<const uint4*>(skip);
-  uint4* oo = reinterpret_cast<uint4*>(out);
-  if (relu && skip) launch_pdl(bn_apply_fin_kernel<true, true>, grid, block, 0, st, yy, partials, rows, f, kk, oo, n_vec);
-  else if (relu) launch_pdl(bn_apply_fin_kernel<true, false>, grid, block, 0, st, yy, partials, rows, f, kk, oo, n_vec);
-  else if (skip) launch_pdl(bn_apply_fin_kernel<false, true>, grid, block, 0, st, yy, partials, rows, f, kk, oo, n_vec);
-  else launch_pdl(bn_apply_fin_kernel<false, false>, grid, block, 0, st, yy, partials, rows, f, kk, oo, n_vec);
-  SRG_LAUNCH_CHECK("bn_apply_fin");
-  return 0;
-}
-
-__global__ void __launch_bounds__(kFinThreads) bn_bwd_apply_fin_kernel(const uint4* __restrict__ dout, const uint4* __restrict__ y,
-                                                                       const float* __restrict__ partials, int rows,
-                                                                       const ReduceFinalize f, uint4* __restrict__ dy,
-                                                                       int64_t n_vec) {
-  __shared__ double red[16][128];
-  __shared__ double sums[128];
-  __shared__ float coef[3][64];
-  pdl_trigger();
-  pdl_wait();
-  block_partial_sums(partials, rows, red, sums);
-  if (threadIdx.x < 64) {
-    const int c = threadIdx.x;
-    const double s1 = sums[c], s2 = sums[64 + c];
-    const double mean = f.save_mean[c], inv = f.save_inv[c];
-    const double dg = inv * (s2 - mean * s1);
-    const double db = s1;
-    const double sc = double(f.gamma[c]) * inv;
-    const float cA = float(sc), cB = float(-sc * inv * dg / f.count);
-    const float cC = float(-sc * db / f.count + sc * inv * mean * dg / f.count);
-    coef[0][c] = cA; coef[1][c] = cB; coef[2][c] = cC;
-    if (blockIdx.x == 0) {
-      if (f.dgamma) f.dgamma[c] = float(dg);
-      if (f.dbeta) f.dbeta[c] = float(db);
-      f.out0[c] = cA; f.out1[c] = cB; f.out2[c] = cC;
-    }
-  }
-  __syncthreads();
-  const int cg = threadIdx.x & 7;
-  float a[8], b[8], c[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) { a[e] = coef[0][cg * 8 + e]; b[e] = coef[1][cg * 8 + e]; c[e] = coef[2][cg * 8 + e]; }
-  const int64_t stride = int64_t(gridDim.x) * kFinThreads;
-  int64_t i = int64_t(blockIdx.x) * kFinThreads + threadIdx.x;
-  for (; i + 3 * stride < n_vec; i += 4 * stride) {
-    uint4 rd[4], ry[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) { rd[u] = dout[i + u * stride]; ry[u] = y[i + u * stride]; }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      float d[8], v[8];
-      unpack8(rd[u], d);
-      unpack8(ry[u], v);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) d[e] = fmaf(a[e], d[e], fmaf(b[e], v[e], c[e]));
-      dy[i + u * stride] = pack8(d);
-    }
-  }
-  for (; i < n_vec; i += stride) {
-    float d[8], v[8];
-    unpack8(dout[i], d);
-    unpack8(y[i], v);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) d[e] = fmaf(a[e], d[e], fmaf(b[e], v[e], c[e]));
-    dy[i] = pack8(d);
-  }
-}
-int launch_bn_bwd_apply_fin(const void* dout, const void* y, const float* partials, int rows, const ReduceFinalize& f, void* dy,
-                            int64_t pixels, cudaStream_t st) {
-  if (f.mode != RF_BN_BWD) { set_error("bn_bwd_apply_fin: needs an RF_BN_BWD finalize descriptor"); return -40; }
-  const int64_t n_vec = pixels * 8;
-  launch_pdl(bn_bwd_apply_fin_kernel, dim3(fin_blocks(n_vec)), dim3(kFinThreads), 0, st, reinterpret_cast<const uint4*>(dout),
-             reinterpret_cast<const uint4*>(y), partials, rows, f, reinterpret_cast<uint4*>(dy), n_vec);
-  SRG_LAUNCH_CHECK("bn_bwd_apply_fin");
   return 0;
 }
 

@@ -11,9 +11,8 @@ constexpr int kRedBlocksMax = 296;  // 2 x 148 SMs
 // ---- per-channel reductions over [P pixels][64 ch] bf16 ------------------------------------------
 // partials: float [blocks][128]  ([0,64) = sum a ; [64,128) = sum a*a (b == null) or sum a*b)
 int reduce_blocks(int64_t pixels);
-int l2_hints();   // SRG_L2_HINTS: 0 none, 1 BatchNorm chain, 2 + convolution stores
 int launch_chan_reduce(const void* a, const void* b, int64_t pixels, float* partials, cudaStream_t st);
-// Fused variant: reduction + fixed-order partial sum + per-channel finalize in ONE launch (last block done).
+// Per-channel finalize of the fixed-order partial sums (launch_partials_finalize).
 // RF_BN_BWD_FROZEN: backward of an eval-mode (running-statistics) BatchNorm; save_mean / save_inv hold running_mean and
 // 1 / sqrt(running_var + eps), the coefficients are A = gamma * inv, B = C = 0 and `dbias` (optional) receives the
 // gradient of the preceding conv's bias, A * sum(dz)
@@ -41,9 +40,6 @@ struct ReduceFinalize {
 int launch_partials_finalize(const float* partials, int rows, const ReduceFinalize& f, cudaStream_t st);
 // SyncBatchNorm path: only the fixed-order column sums (double[128]); the all-reduce and finalize follow.
 int launch_partials_sums(const float* partials, int rows, double* sums, cudaStream_t st);
-// `ticket` is a device counter that must be 0 before the first launch (the kernel resets it).
-int launch_chan_reduce_final(const void* a, const void* b, int64_t pixels, float* partials, unsigned int* ticket,
-                             const ReduceFinalize& f, cudaStream_t st);
 // sums[128] (double) = fixed-order sum of the block partials
 int launch_partials_to_sums(const float* partials, int blocks, double* sums, cudaStream_t st);
 
@@ -77,13 +73,6 @@ int launch_bn_bwd_finalize(const double* sums, double count, const float* gamma,
                            float* coefC, float param_grad_scale, cudaStream_t st);
 int launch_bn_bwd_apply(const void* dout, const void* y, const float* coefA, const float* coefB, const float* coefC,
                         void* dy, int64_t pixels, cudaStream_t st);
-// The same two passes with the statistics finalize folded in (training, single GPU): every CTA re-reduces the [rows][128]
-// partial sums (fixed order), derives the coefficients and applies them; CTA 0 also writes f.out0..3 (and the running
-// statistics / the BatchNorm weight and bias gradients).  One launch instead of two on the dependency chain.
-int launch_bn_apply_fin(const void* y, const float* partials, int rows, const ReduceFinalize& f, const void* skip, int relu,
-                        void* out, int64_t pixels, cudaStream_t st);
-int launch_bn_bwd_apply_fin(const void* dout, const void* y, const float* partials, int rows, const ReduceFinalize& f, void* dy,
-                            int64_t pixels, cudaStream_t st);
 // d(pre-activation) of LeakyReLU from two incoming gradients: dpre = (ga + gb) * (post > 0 ? 1 : slope)
 int launch_lrelu_bwd_add2(const void* ga, const void* gb, const void* post, float slope, void* dpre, int64_t pixels,
                           cudaStream_t st);

@@ -34,7 +34,7 @@ struct Carver {
 
 // ------------------------------------------------------------------ workspace layout
 struct Layout {
-  size_t packed, bias, bncoef, bwdcoef, partials, sums, ticket, wg_partials, ps_scratch, loss_scratch;
+  size_t packed, bias, bncoef, bwdcoef, partials, sums, trunk_err, wg_partials, ps_scratch, loss_scratch;
   size_t dyall = 0, slot = 0;             // per-layer output gradients of the trunk convs: slot l = 2*block + conv, last = conv2
   size_t wgb_partials = 0, wgb_floats = 0;  // partial sets of the batched trunk weight-gradient kernel
   size_t trunk_sync = 0, trunk_tab = 0;     // trunk_fused: flags / barrier words, the two TrunkLayer tables (fwd | bwd)
@@ -81,7 +81,7 @@ Layout make_layout(const GeneratorEngine& e, bool training) {
   L.bwdcoef = c.take(192 * 4);
   L.partials = c.take(size_t(kRedBlocksMax) * 128 * 4);
   L.sums = c.take(128 * 8);
-  L.ticket = c.take(256);
+  L.trunk_err = c.take(4);                 // the fused trunk kernel's error word (generator_trunk_error)
   L.trunk_sync = c.take(trunk_sync_bytes(e.N, e.H, e.W));
   L.trunk_tab = c.take(size_t(2) * (2 * e.n_res + 1) * sizeof(TrunkLayer));   // eval: 2*n_res int4 BatchNorm offset rows instead
   L.U1 = c.take(size_t(e.N) * (e.H + 1) * e.W * 128);
@@ -431,7 +431,7 @@ void fill_trunk_gen(EngineImpl* e, TrunkGen& t) {
   t.bncoef = reinterpret_cast<float*>(ws + L.bncoef);
   t.gpart = reinterpret_cast<float*>(ws + L.partials);
   t.sync = reinterpret_cast<unsigned int*>(ws + L.trunk_sync);
-  t.err = reinterpret_cast<unsigned int*>(ws + L.ticket + 128);
+  t.err = reinterpret_cast<unsigned int*>(ws + L.trunk_err);
   t.peer = e->peer;
 }
 
@@ -475,7 +475,8 @@ int run_trunk(EngineImpl* e, int bwd, int update_running, cudaStream_t st, bool 
 // tiles), and the BatchNorm passes between two layers run per generator on forked streams (they are HBM-bound and not
 // SM-exclusive, so the n chains overlap) and join again ahead of the next grouped launch.  Arithmetic per generator is the
 // per-layer path's (same kernels, same order).
-bool wgrad_layout_batched(const EngineImpl& e) {
+// N: the items of the pass (the engine's N, or the window count of a tiled backward)
+bool wgrad_layout_batched(const EngineImpl& e, int N) {
   const Layout& L = e.L;
   if (!e.wgrad_batched || e.n_res < 1) return false;
   for (int b = 0; b < e.n_res; ++b) {
@@ -484,26 +485,16 @@ bool wgrad_layout_batched(const EngineImpl& e) {
   }
   if (L.out[e.n_res - 1] != L.out1 + size_t(2 * e.n_res) * 2 * L.slot) return false;
   WgradBatchArgs probe; memset(&probe, 0, sizeof(probe));
-  probe.N = e.N; probe.H = e.H; probe.W = e.W; probe.n_layers = 2 * e.n_res + 1;
+  probe.N = N; probe.H = e.H; probe.W = e.W; probe.n_layers = 2 * e.n_res + 1;
+  // the partial-set workspace was sized for 148 SMs at create time: a device that splits the work differently keeps the
+  // per-layer launches instead of overrunning it
   return wgrad3_batched_partials_floats(probe) <= L.wgb_floats;
 }
 
 bool use_trunk_grouped(const EngineImpl& e) {
   if (!e.ws || !e.ws_training || e.n_res < 1) return false;
   if (e.allreduce != nullptr && e.peer == nullptr) return false;      // NCCL SyncBatchNorm transport: per-generator branches
-  if (e.fin_fused || e.reduce_final || e.fuse_bwd_stats) return false;
-  static const bool off = [] { const char* v = getenv("SRG_TRUNK_GROUPED"); return v != nullptr && v[0] == '0'; }();
-  if (off) return false;
-  return wgrad_layout_batched(e);
-}
-
-// SRG_GROUPED_OPT bits: 1 = the statistics finalize runs inside the apply / backward-apply pass (single GPU; the grouped launch
-// leaves 49 partial rows per generator instead of 148, so the re-reduction per CTA is cheap), 2 = the BatchNorm-backward sums
-// are accumulated by the grouped dgrad launch's epilogue instead of a separate reduction pass, 4 = the backward reduction's last
-// block finalizes the coefficients (single GPU)
-int grouped_opt() {
-  static const int v = [] { const char* e = getenv("SRG_GROUPED_OPT"); return e ? atoi(e) : 0; }();
-  return v;
+  return wgrad_layout_batched(e, e.N);
 }
 
 struct ForkJoin {
@@ -559,7 +550,7 @@ BnNames bn_offsets(const EngineImpl& e, int b, int k) {
 // one grouped 3x3 64 -> 64 launch: problem g reads in[g], writes out[g]
 int grouped_conv3x3(EngineImpl* const* es, int n, const void* const* in, const int64_t* w_off, const float* const* bias,
                     const void* const* residual, const void* const* mask, void* const* out, bool stats, int* stats_rows,
-                    cudaStream_t st, const void* const* stats_y = nullptr) {
+                    cudaStream_t st) {
   ConvGemmArgs as[kIlMaxGroups];
   for (int g = 0; g < n; ++g) {
     EngineImpl* e = es[g];
@@ -572,7 +563,6 @@ int grouped_conv3x3(EngineImpl* const* es, int n, const void* const* in, const i
     a.residual = residual ? residual[g] : nullptr; a.mask_src = mask ? mask[g] : nullptr;
     a.out = out[g]; a.out_mode = OUT_NHWC;
     if (stats) a.stats = reinterpret_cast<float*>(e->ws + e->L.partials);
-    if (stats && stats_y) a.stats_y = stats_y[g];
   }
   if (stats) *stats_rows = n > 1 ? conv_gemm_grouped_rows(as[0], n) : conv_gemm_grid(as[0]);
   es[0]->launches += 1;
@@ -621,11 +611,6 @@ int trunk_layers_forward_multi(EngineImpl* const* es, int n, int update_running,
       float* partials = reinterpret_cast<float*>(e->ws + L.partials);
       const void* y = e->ws + (k == 0 ? L.y1[b] : L.y2[b]);
       void* dst = e->ws + (k == 0 ? L.z1[b] : L.out[b]);
-      if (!e->peer && (grouped_opt() & 1)) {
-        RC(launch_bn_apply_fin(y, partials, rows, f, k == 0 ? nullptr : x[g], k == 0 ? 1 : 0, dst, P, sg));
-        e->launches += 1;
-        continue;
-      }
       if (e->peer) RC(launch_peer_finalize(e->peer, partials, rows, f, sg));
       else RC(launch_partials_finalize(partials, rows, f, sg));
       RC(launch_bn_apply(y, coef, coef + 64, k == 0 ? nullptr : x[g], k == 0 ? 1 : 0, dst, P, sg));
@@ -678,11 +663,7 @@ int trunk_layers_backward_multi(EngineImpl* const* es, int n, cudaStream_t st) {
     dother[g] = es[g]->ws + L.g[1];
     in[g] = es[g]->ws + L.g[3]; out[g] = dout[g]; woff[g] = es[g]->po.conv2_d;
   }
-  const bool epi_sums = (grouped_opt() & 2) != 0;
-  const void* sy[kIlMaxGroups];
-  int rows = 0;
-  for (int g = 0; g < n; ++g) sy[g] = es[g]->ws + es[g]->L.y2[R - 1];
-  RC(grouped_conv3x3(es, n, in, woff, nullptr, nullptr, nullptr, out, epi_sums, &rows, st, sy));
+  RC(grouped_conv3x3(es, n, in, woff, nullptr, nullptr, nullptr, out, false, nullptr, st));
   // BatchNorm backward of every generator (sums of dz and dz*y, coefficients, apply) on forked streams
   auto bn_bwd_stage = [&](int b, int k, void* const* dz, void* const* dy) -> int {
     RC(fj_fork(fj, n, st));
@@ -695,30 +676,12 @@ int trunk_layers_backward_multi(EngineImpl* const* es, int n, cudaStream_t st) {
       float* partials = reinterpret_cast<float*>(e->ws + L.partials);
       const BnNames o = bn_offsets(*e, b, k);
       const void* y = e->ws + (k == 0 ? L.y1[b] : L.y2[b]);
-      int r = rows;
-      if (!epi_sums && !e->peer && (grouped_opt() & 4)) {
-        // the reduction's last block finalizes (atomic ticket): no single-block finalize launch on the backward chain
-        ReduceFinalize f; memset(&f, 0, sizeof(f));
-        f.mode = RF_BN_BWD; f.count = double(P); f.gamma = e->master + o.gamma; f.save_mean = coef + 128; f.save_inv = coef + 192;
-        f.dgamma = e->grads + o.gamma; f.dbeta = e->grads + o.beta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
-        RC(launch_chan_reduce_final(dz[g], y, P, partials, reinterpret_cast<unsigned int*>(e->ws + L.ticket), f, sg));
-        RC(launch_bn_bwd_apply(dz[g], y, bwd, bwd + 64, bwd + 128, dy[g], P, sg));
-        e->launches += 2;
-        continue;
-      }
-      if (!epi_sums) {
-        RC(launch_chan_reduce(dz[g], y, P, partials, sg));
-        r = reduce_blocks(P);
-        e->launches += 1;
-      }
+      RC(launch_chan_reduce(dz[g], y, P, partials, sg));
+      const int r = reduce_blocks(P);
+      e->launches += 1;
       ReduceFinalize f; memset(&f, 0, sizeof(f));
       f.mode = RF_BN_BWD; f.count = double(P) * e->world; f.gamma = e->master + o.gamma; f.save_mean = coef + 128; f.save_inv = coef + 192;
       f.dgamma = e->grads + o.gamma; f.dbeta = e->grads + o.beta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
-      if (!e->peer && (grouped_opt() & 1)) {
-        RC(launch_bn_bwd_apply_fin(dz[g], y, partials, r, f, dy[g], P, sg));
-        e->launches += 1;
-        continue;
-      }
       if (e->peer) RC(launch_peer_finalize(e->peer, partials, r, f, sg));
       else RC(launch_partials_finalize(partials, r, f, sg));
       RC(launch_bn_bwd_apply(dz[g], y, bwd, bwd + 64, bwd + 128, dy[g], P, sg));
@@ -735,9 +698,8 @@ int trunk_layers_backward_multi(EngineImpl* const* es, int n, cudaStream_t st) {
       const Layout& L = es[g]->L;
       d_p1[g] = es[g]->keep_grads ? es[g]->ws + L.kd_p1[b] : dother[g];
       in[g] = d_y[g]; out[g] = d_p1[g]; mask[g] = es[g]->ws + L.z1[b]; woff[g] = es[g]->po.rb_d[1][b];   // ReLU backward via mask
-      sy[g] = es[g]->ws + L.y1[b];
     }
-    RC(grouped_conv3x3(es, n, in, woff, nullptr, nullptr, mask, out, epi_sums, &rows, st, sy));
+    RC(grouped_conv3x3(es, n, in, woff, nullptr, nullptr, mask, out, false, nullptr, st));
     // z1 = relu(bn1(y1))
     for (int g = 0; g < n; ++g) d_y[g] = es[g]->ws + es[g]->L.dyall + es[g]->L.slot * size_t(2 * b);
     RC(bn_bwd_stage(b, 0, d_p1, d_y));
@@ -745,9 +707,8 @@ int trunk_layers_backward_multi(EngineImpl* const* es, int n, cudaStream_t st) {
       const Layout& L = es[g]->L;
       d_in[g] = es[g]->keep_grads ? es[g]->ws + L.kd_in[b] : dother[g];
       in[g] = d_y[g]; out[g] = d_in[g]; res[g] = dout[g]; woff[g] = es[g]->po.rb_d[0][b];               // + skip gradient
-      if (b > 0) sy[g] = es[g]->ws + L.y2[b - 1];
     }
-    RC(grouped_conv3x3(es, n, in, woff, nullptr, res, nullptr, out, epi_sums && b > 0, &rows, st, sy));
+    RC(grouped_conv3x3(es, n, in, woff, nullptr, res, nullptr, out, false, nullptr, st));
     for (int g = 0; g < n; ++g) {
       if (es[g]->keep_grads) { dout[g] = d_in[g]; } else { void* t = dout[g]; dout[g] = dother[g]; dother[g] = t; }
     }
@@ -784,7 +745,7 @@ int generator_trunk_error(GeneratorEngine* g) {
   EngineImpl* e = static_cast<EngineImpl*>(g);
   if (!e->ws) return 0;
   unsigned int v = 0;
-  if (cudaMemcpy(&v, e->ws + e->L.ticket + 128, 4, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+  if (cudaMemcpy(&v, e->ws + e->L.trunk_err, 4, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
   return int(v);
 }
 int generator_prof_layers(const GeneratorEngine* g) { return g->prof_layers; }
@@ -824,13 +785,7 @@ GeneratorEngine* generator_create(int N, int H, int W, int n_res, int n_up) {
   EngineImpl* e = new EngineImpl();
   e->N = N; e->H = H; e->W = W; e->n_res = n_res; e->n_up = n_up;
   {
-    const char* ev = getenv("SRG_FUSE_BWD_STATS");
-    e->fuse_bwd_stats = ev != nullptr && ev[0] == '1';
-    ev = getenv("SRG_REDUCE_FINAL");
-    e->reduce_final = ev != nullptr && ev[0] == '1';
-    ev = getenv("SRG_FIN_FUSED");
-    e->fin_fused = ev != nullptr && ev[0] == '1';
-    ev = getenv("SRG_WGRAD_BATCHED");
+    const char* ev = getenv("SRG_WGRAD_BATCHED");
     e->wgrad_batched = !(ev != nullptr && ev[0] == '0');
   }
   // ---- parameters in the reference's registration order (src/models.py:53-78)
@@ -985,7 +940,7 @@ int generator_bind(GeneratorEngine* g, float* master, float* grads, float* bn_bu
   e->master = master; e->grads = grads; e->bn_buffers = bn_buffers;
   e->ws = reinterpret_cast<uint8_t*>(ws); e->ws_bytes = ws_bytes; e->ws_training = training != 0;
   e->L = make_layout(*e, training != 0);
-  if (cudaMemset(e->ws + e->L.ticket, 0, 256) != cudaSuccess) { set_error("generator_bind: memset failed"); return -29; }
+  if (cudaMemset(e->ws + e->L.trunk_err, 0, 4) != cudaSuccess) { set_error("generator_bind: memset failed"); return -29; }
   e->trunk_ok = false;
   e->last_frozen = false;
   e->tile_n = 0;
@@ -1190,21 +1145,6 @@ int forward_impl(EngineImpl* e, const float* lr, void* sr, int training, int upd
     if (frozen) {
       e->launches += 1;
       return launch_bn_apply(y, coef, coef + 64, skip, relu, out, P, st);
-    }
-    if (e->fin_fused && !e->allreduce && !e->peer) {
-      // single GPU: the finalize runs inside the apply pass (every CTA re-reduces the partial rows): one launch, not two
-      snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.weight", b, k + 1);
-      const float* gamma = e->master + poff(*e, nm);
-      snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.bias", b, k + 1);
-      const float* beta = e->master + poff(*e, nm);
-      snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.running_mean", b, k + 1);
-      float* rm = e->bn_buffers + boff(*e, nm);
-      ReduceFinalize f; memset(&f, 0, sizeof(f));
-      f.mode = RF_BN_FWD; f.count = double(P); f.eps = kBnEps; f.momentum = kBnMomentum; f.gamma = gamma; f.beta = beta;
-      f.running_mean = update_running ? rm : nullptr; f.running_var = update_running ? rm + 64 : nullptr;
-      f.out0 = coef; f.out1 = coef + 64; f.out2 = coef + 128; f.out3 = coef + 192;
-      e->launches += 1;
-      return launch_bn_apply_fin(y, reinterpret_cast<const float*>(ws + L.partials), stats_rows, f, skip, relu, out, P, st);
     }
     RC(bn_coeffs(b, k, y));
     e->launches += 1;
@@ -1477,11 +1417,8 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     return launch_partials_finalize(partials, reduce_blocks(pixels), f, st);
   };
   // dgrad of a 3x3 conv whose output gradient has `chunks`*64 channels (4 pixel-shuffle views when chunks == 4)
-  int bwd_stats_rows = 0;
-  // stats_y != null: the epilogue also accumulates sum(out) and sum(out * stats_y) per channel (BatchNorm backward
-  // statistics of the NEXT step, which consumes `out` as dz and stats_y as the saved conv output)
   auto dgrad3x3 = [&](const void* dy_base, int gh, int gw, bool dy_ps, int64_t w_off, const void* residual, const void* mask,
-                      void* out, const void* stats_y) -> int {
+                      void* out) -> int {
     ConvGemmArgs a; memset(&a, 0, sizeof(a));
     a.N = N; a.H = gh; a.W = gw; set_taps_3x3(a);
     if (dy_ps) {
@@ -1493,10 +1430,6 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     a.in_H = gh; a.in_W = gw;
     a.weights = packed + w_off; a.cout_total = 64; a.block_n = 64;
     a.bias = nullptr; a.act = ACT_NONE; a.residual = residual; a.mask_src = mask; a.out = out; a.out_mode = OUT_NHWC;
-    // Measured twice (profiles/r01_notes.md): with the generic kernel's single epilogue group the fusion was slower than
-    // the separate 7 us reduction pass; with conv3_il's two epilogue groups the step time is unchanged within noise
-    // (11.4-11.5 ms either way) while the dgrad launches get 4 us longer, so it stays off unless SRG_FUSE_BWD_STATS=1.
-    if (stats_y != nullptr && e->fuse_bwd_stats) { a.stats = partials; a.stats_y = stats_y; bwd_stats_rows = conv_gemm_grid(a); }
     e->launches += 1;
     if (dy_ps) return launch_conv_gemm(a, st);
     ProfScope ps(e, st);
@@ -1539,7 +1472,7 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
       snprintf(nm, sizeof(nm), "upsample.%d.weight", 3 * j);
       RC(wgrad(plain_view(in_j, Hj, Wj), Hj, Wj, false, Hj, Wj, ws + L.dup[j], 4, true, e->d_wg_idx_up, nm));
     }
-    RC(dgrad3x3(ws + L.dup[j], Hj, Wj, true, po.up_d[j], nullptr, j > 0 ? in_j : nullptr, j > 0 ? ws + L.dup[j - 1] : d_trunk, nullptr));
+    RC(dgrad3x3(ws + L.dup[j], Hj, Wj, true, po.up_d[j], nullptr, j > 0 ? in_j : nullptr, j > 0 ? ws + L.dup[j - 1] : d_trunk));
   }
   }
   // ---- conv2 (trunk = conv2(x_last) + out1)
@@ -1548,19 +1481,7 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
   // The 2*n_res + 1 trunk weight gradients run as ONE batched launch at the end of backward (wgrad3_batched_kernel):
   // x of layer l = 2*block + conv sits at out1 + l * 2 * slot (out[b-1] | z1[b] are two slots apart, conv2 reads out[last]),
   // dy of layer l at dyall + l * slot.  SRG_WGRAD_BATCHED=0 (or a non-uniform layout) keeps one launch per layer.
-  bool batched = e->wgrad_batched && e->n_res > 0;
-  for (int b = 0; b < e->n_res && batched; ++b) {
-    const size_t x1 = b > 0 ? L.out[b - 1] : L.out1;
-    if (x1 != L.out1 + size_t(2 * b) * 2 * L.slot || L.z1[b] != L.out1 + size_t(2 * b + 1) * 2 * L.slot) batched = false;
-  }
-  if (batched && L.out[e->n_res - 1] != L.out1 + size_t(2 * e->n_res) * 2 * L.slot) batched = false;
-  if (batched) {
-    // the partial-set workspace was sized for 148 SMs at create time: a device that splits the work differently keeps
-    // the per-layer launches instead of overrunning it
-    WgradBatchArgs probe; memset(&probe, 0, sizeof(probe));
-    probe.N = N; probe.H = H; probe.W = W; probe.n_layers = 2 * e->n_res + 1;
-    if (wgrad3_batched_partials_floats(probe) > L.wgb_floats) batched = false;
-  }
+  const bool batched = wgrad_layout_batched(*e, N);
   if (!batched && pre && pg) RC(wgrad(plain_view(x_last, H, W), H, W, false, H, W, d_trunk, 1, false, e->d_wg_idx_c3x3, "conv2.weight"));
   const bool keep = e->keep_grads;
   void* dout = keep ? ws + L.kd_last : ws + L.g[0];
@@ -1580,7 +1501,7 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     // split execution on the per-layer path: generators_trunk() ran (or will run) the dgrad chain as grouped launches
     dout = layers_dout(*e);
   } else {
-    RC(dgrad3x3(d_trunk, H, W, false, po.conv2_d, nullptr, nullptr, dout, e->n_res > 0 ? ws + L.y2[e->n_res - 1] : nullptr));
+    RC(dgrad3x3(d_trunk, H, W, false, po.conv2_d, nullptr, nullptr, dout));
   }
   // ---- residual blocks, last to first (src/models.py:21-25)
   float* bwd = reinterpret_cast<float*>(ws + L.bwdcoef);
@@ -1590,15 +1511,12 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     const int64_t go = poff(*e, nm);
     snprintf(nm, sizeof(nm), "residual_blocks.%d.bn%d.bias", b, k + 1);
     const int64_t bo = poff(*e, nm);
-    // sum dz and sum dz*y: either accumulated by the dgrad kernel that produced dz (fuse_bwd_stats) or by one pass here
-    int rows = bwd_stats_rows;
+    // sum dz and sum dz*y
+    RC(launch_chan_reduce(dz, y, P, partials, st));
+    const int rows = reduce_blocks(P);
+    e->launches += 1;
     if (frozen) {
       // running statistics: no cross-rank exchange, dy = gamma * inv * dz, and the preceding conv's bias gets A * sum(dz)
-      if (!e->fuse_bwd_stats) {
-        RC(launch_chan_reduce(dz, y, P, partials, st));
-        rows = reduce_blocks(P);
-        e->launches += 1;
-      }
       ReduceFinalize f; memset(&f, 0, sizeof(f));
       f.mode = RF_BN_BWD_FROZEN; f.count = double(P); f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
       if (pg) {
@@ -1612,28 +1530,10 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     }
     float* dgamma = pg ? e->grads + go : nullptr;
     float* dbeta = pg ? e->grads + bo : nullptr;
-    if (!e->fuse_bwd_stats && !e->allreduce && !e->peer && e->reduce_final) {
-      // single GPU: the reduction's last block finalizes (atomic ticket): no finalize launch on the backward chain
-      ReduceFinalize f; memset(&f, 0, sizeof(f));
-      f.mode = RF_BN_BWD; f.count = double(P); f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
-      f.dgamma = dgamma; f.dbeta = dbeta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
-      RC(launch_chan_reduce_final(dz, y, P, partials, reinterpret_cast<unsigned int*>(ws + L.ticket), f, st));
-      e->launches += 2;
-      return launch_bn_bwd_apply(dz, y, bwd, bwd + 64, bwd + 128, dy, P, st);
-    }
-    if (!e->fuse_bwd_stats) {
-      RC(launch_chan_reduce(dz, y, P, partials, st));
-      rows = reduce_blocks(P);
-      e->launches += 1;
-    }
     if (!e->allreduce || e->peer) {
       ReduceFinalize f; memset(&f, 0, sizeof(f));
       f.mode = RF_BN_BWD; f.count = double(P) * e->world; f.gamma = e->master + go; f.save_mean = coef + 128; f.save_inv = coef + 192;
       f.dgamma = dgamma; f.dbeta = dbeta; f.out0 = bwd; f.out1 = bwd + 64; f.out2 = bwd + 128;
-      if (!e->peer && e->fin_fused) {
-        e->launches += 1;
-        return launch_bn_bwd_apply_fin(dz, y, partials, rows, f, dy, P, st);
-      }
       if (e->peer) RC(launch_peer_finalize(e->peer, partials, rows, f, st));
       else RC(launch_partials_finalize(partials, rows, f, st));
       e->launches += 2;
@@ -1656,12 +1556,12 @@ int backward_impl(EngineImpl* e, const float* dsr, int phases, bool param_grads,
     RC(bn_backward(b, 1, dout, ws + L.y2[b], d_y2));
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv2.weight", b);
     if (!batched && pg) RC(wgrad(plain_view(ws + L.z1[b], H, W), H, W, false, H, W, d_y2, 1, false, e->d_wg_idx_c3x3, nm));
-    RC(dgrad3x3(d_y2, H, W, false, po.rb_d[1][b], nullptr, ws + L.z1[b], d_p1, ws + L.y1[b]));   // ReLU backward via mask
+    RC(dgrad3x3(d_y2, H, W, false, po.rb_d[1][b], nullptr, ws + L.z1[b], d_p1));   // ReLU backward via mask
     // z1 = relu(bn1(y1))
     RC(bn_backward(b, 0, d_p1, ws + L.y1[b], d_y1));
     snprintf(nm, sizeof(nm), "residual_blocks.%d.conv1.weight", b);
     if (!batched && pg) RC(wgrad(plain_view(x_in, H, W), H, W, false, H, W, d_y1, 1, false, e->d_wg_idx_c3x3, nm));
-    RC(dgrad3x3(d_y1, H, W, false, po.rb_d[0][b], dout, nullptr, d_in, b > 0 ? ws + L.y2[b - 1] : nullptr));   // + skip gradient
+    RC(dgrad3x3(d_y1, H, W, false, po.rb_d[0][b], dout, nullptr, d_in));   // + skip gradient
     if (keep) { dout = d_in; } else { void* t = dout; dout = dother; dother = t; }
   }
   if (!post) return 0;

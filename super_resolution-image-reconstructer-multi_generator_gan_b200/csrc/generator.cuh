@@ -61,18 +61,9 @@ struct GeneratorEngine {
   struct PeerSync* peer = nullptr;   // NVLink peer-memory exchange fused with the finalize (preferred over `allreduce`)
   int world = 1;
   long long launches = 0;  // kernels launched so far (bench bookkeeping)
-  // optional CUDA-event timing of the dominant kernel class (3x3 64->64 fprop/dgrad conv_gemm launches)
-  bool fuse_bwd_stats = false;  // BatchNorm-backward sums in the dgrad epilogue instead of a separate pass (SRG_FUSE_BWD_STATS=1: on)
-  // single GPU: BatchNorm statistics finalize inside the apply / backward-apply pass (SRG_FIN_FUSED=1).  Measured on B200
-  // (profiles/r02_notes.md): one generator alone 3.94 -> 3.84 ms per step, but three generators as parallel graph branches
-  // 11.08 -> 11.4-11.7 ms (the fatter apply CTAs take bandwidth from the other branches' tensor-core kernels), so it is off
-  // by default
-  bool fin_fused = false;
-  // single GPU, backward: the BatchNorm-backward reduction's last block finalizes the coefficients (SRG_REDUCE_FINAL=1).
-  // Measured: 96 fewer launches per 3-generator step, step time unchanged (10.69 vs 10.69-10.72 ms), so the two-launch form stays
-  bool reduce_final = false;
   bool wgrad_batched = true;    // trunk weight gradients in one batched launch at the end of backward (SRG_WGRAD_BATCHED=0: off)
   bool keep_grads = false; // debug: keep every inter-layer gradient in its own named buffer (parity tests)
+  // optional CUDA-event timing of the dominant kernel class (3x3 64->64 fprop/dgrad conv_gemm launches)
   bool prof_on = false;
   std::vector<cudaEvent_t> prof_events;   // pairs (start, stop)
   size_t prof_used = 0;

@@ -36,15 +36,15 @@ struct DeviceOnce {
   }
 };
 
-// SRG_PDL (read once): 0 = plain stream-order launches everywhere (a kernel timeline then shows each kernel's own duration
-// instead of one that starts while the predecessor is still running); 1 = every launch_pdl() kernel may start early; 2
-// (default) = only grids of at most 8 blocks (the single-block finalize kernels) and inference (`exclusive`) convolutions start
-// early: a big grid parked at griddepcontrol.wait holds registers / shared memory that a ready kernel of another stream could
-// use.  Measured on the cfg2 training step (profiles/r02_ab_pdl_grouped.log): 9.61-9.64 ms (2) vs 9.69-9.74 ms (1).
-inline int pdl_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SRG_PDL"); v = e ? atoi(e) : 2; }
-  return v;
+// Only grids of at most 8 blocks (the single-block finalize kernels) and inference (`exclusive`) convolutions start early: a
+// big grid parked at griddepcontrol.wait holds registers / shared memory that a ready kernel of another stream could use.
+// Measured on the cfg2 training step (profiles/r02_ab_pdl_grouped.log): 9.61-9.64 ms vs 9.69-9.74 ms with every launch_pdl()
+// kernel starting early.
+// SRG_PDL=0 (read once) is a diagnostic: plain stream-order launches everywhere, so that a kernel timeline shows each
+// kernel's own duration instead of one that starts while the predecessor is still running.
+inline bool pdl_enabled() {
+  static const bool on = [] { const char* e = getenv("SRG_PDL"); return e == nullptr || atoi(e) != 0; }();
+  return on;
 }
 
 template <typename... KArgs, typename... Args>
@@ -65,30 +65,13 @@ inline cudaError_t launch_with_pdl_attr(bool early, void (*kernel)(KArgs...), di
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  const int mode = pdl_mode();
-  const bool early = mode == 1 || (mode == 2 && grid.x * grid.y * grid.z <= 8);
+  const bool early = pdl_enabled() && grid.x * grid.y * grid.z <= 8;
   return launch_with_pdl_attr(early, kernel, grid, block, smem, st, std::forward<Args>(args)...);
 }
 // inference launches: a chain of SM-exclusive convolutions on one stream with nothing else to schedule -- early start pays
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl_exclusive(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  return launch_with_pdl_attr(pdl_mode() != 0, kernel, grid, block, smem, st, std::forward<Args>(args)...);
-}
-
-// A/B switches (read once): SRG_PDL_CONV=0 launches the SM-exclusive convolution kernels WITHOUT the attribute (a CTA that
-// is resident early holds ~190 KB of shared memory while it waits for its predecessor, which keeps another graph branch's
-// ready convolution off that SM); SRG_PDL_EW_LATE=1 makes the elementwise producers of a convolution operand trigger their
-// dependents at the END of their loop instead of at the start (the convolution still pre-pays its launch latency).
-inline bool pdl_conv() { static int v = -1; if (v < 0) { const char* e = getenv("SRG_PDL_CONV"); v = (e && e[0] == '0') ? 0 : 1; } return v != 0; }
-inline int pdl_ew_late() { static int v = -1; if (v < 0) { const char* e = getenv("SRG_PDL_EW_LATE"); v = (e && e[0] == '1') ? 1 : 0; } return v; }
-
-// pdl: 0 = never early, 1 = as launch_pdl() decides, 2 = inference launch (launch_pdl_exclusive)
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_opt_pdl(int pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                  Args&&... args) {
-  if (pdl == 2) return launch_pdl_exclusive(kernel, grid, block, smem, st, std::forward<Args>(args)...);
-  if (pdl == 1) return launch_pdl(kernel, grid, block, smem, st, std::forward<Args>(args)...);
-  return launch_with_pdl_attr(false, kernel, grid, block, smem, st, std::forward<Args>(args)...);
+  return launch_with_pdl_attr(pdl_enabled(), kernel, grid, block, smem, st, std::forward<Args>(args)...);
 }
 
 // Column sum of a [rows][128] fp32 partial-sum table for row lane rl of 8 (rows rl, rl+8, ...), fp64, FIXED order: four

@@ -933,33 +933,25 @@ __global__ void __launch_bounds__(kTrThreads, 1) trunk_kernel(const __grid_const
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-int g_trunk_fused = -1;
+int g_trunk_fused = 2;              // 0: off, 1: on, 2: automatic (set_trunk_fused)
 long long* g_trunk_prof = nullptr;     // SRG_TRUNK_PROF=1: role timers + event trace of the last launch (debug)
 
 }  // namespace
 
-// -1: not read yet, 0: off, 1: on, 2: automatic (default)
-static int trunk_fused_mode() {
-  if (g_trunk_fused < 0) {
-    const char* ev = getenv("SRG_TRUNK_FUSED");
-    g_trunk_fused = (ev == nullptr || ev[0] == '\0') ? 2 : (ev[0] == '0' ? 0 : 1);
-  }
-  return g_trunk_fused;
-}
-bool trunk_fused_enabled() { return trunk_fused_mode() != 0; }
+bool trunk_fused_enabled() { return g_trunk_fused != 0; }
 // Measured on B200 (profiles/r02_notes.md): with at most one tile per SM and layer the step is launch-latency bound and
 // the fused kernel wins (8x3x64x64: 2.21 vs 2.69 ms per eager generator step); at the cfg2 geometry (4 tiles per SM)
 // its serial statistics -> barrier -> apply chain per layer loses to the per-layer launches, whose gaps the K
 // generators' graph branches fill (12.6 vs 11.0 ms per 3-generator step).  Automatic mode picks accordingly;
-// SRG_TRUNK_FUSED=1 / srg_set_trunk_fused(1) forces the fused kernel wherever it applies.
+// srg_set_trunk_fused(1) forces the fused kernel wherever it applies.
 bool trunk_fused_preferred(int N, int H, int W) {
-  const int mode = trunk_fused_mode();
+  const int mode = g_trunk_fused;
   if (mode != 2) return mode == 1;
   const int grid = trunk_grid(N, H, W);
   return grid > 0 && N * ((H + 31) / 32) * ((W + 7) / 8) <= grid;
 }
 int set_trunk_fused(int on) {
-  const int old = trunk_fused_mode();
+  const int old = g_trunk_fused;
   g_trunk_fused = on < 0 || on > 2 ? 2 : on;
   return old;
 }

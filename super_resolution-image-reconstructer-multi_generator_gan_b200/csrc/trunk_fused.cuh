@@ -71,7 +71,7 @@ struct TrunkArgs {
 int trunk_grid(int N, int H, int W);
 size_t trunk_sync_bytes(int N, int H, int W);   // device scratch behind TrunkGen::sync (barrier words, flags, published sums)
 int launch_trunk(const TrunkArgs& a, cudaStream_t stream);
-// process-wide switch: 0 = never, 1 = wherever the kernel applies, 2 = automatic (default; SRG_TRUNK_FUSED=0/1 overrides):
+// process-wide switch: 0 = never, 1 = wherever the kernel applies, 2 = automatic (default):
 // fused when a layer has at most one 32x8-pixel tile per SM (launch-latency bound sizes), per-layer launches otherwise
 bool trunk_fused_enabled();
 bool trunk_fused_preferred(int N, int H, int W);

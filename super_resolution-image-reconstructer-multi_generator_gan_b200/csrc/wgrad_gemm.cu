@@ -375,7 +375,7 @@ int launch_wgrad3x3(const WgradArgs& a, cudaStream_t stream) {
   p.splits = splits;
   p.n_stages = 3;
   p.partials = a.partials;
-  p.pol_in = l2_hints() >= 4 ? kL2EvictFirst : kL2EvictNormal;
+  p.pol_in = kL2EvictNormal;
   p.dy_c0_step = a.dy_views == 1 ? 64 : 0;
   {
     uint64_t dims[4] = {64, uint64_t(a.in_W), uint64_t(a.in_H), uint64_t(a.N)};
@@ -637,7 +637,7 @@ int launch_wgrad3x3_batched(const WgradBatchArgs& a, cudaStream_t stream) {
   p.max_slots = ms;
   p.n_stages = 3;
   p.partials = a.partials;
-  p.pol_in = l2_hints() >= 4 ? kL2EvictFirst : kL2EvictNormal;
+  p.pol_in = kL2EvictNormal;
   {
     uint64_t dims[5] = {64, uint64_t(a.W), uint64_t(a.H), uint64_t(a.N), uint64_t(a.n_layers)};
     uint64_t xs[4] = {128, uint64_t(a.W) * 128, uint64_t(a.H) * a.W * 128, uint64_t(a.x_layer_stride_bytes)};
@@ -712,7 +712,7 @@ int launch_wgrad_gemm(const WgradArgs& a, cudaStream_t stream) {
   if (stages < 1) { set_error("wgrad: stage does not fit in shared memory (%u B)", p.stage_bytes); return -6; }
   p.n_stages = stages;
   p.partials = a.partials;
-  p.pol_in = l2_hints() >= 4 ? kL2EvictFirst : kL2EvictNormal;
+  p.pol_in = kL2EvictNormal;
   p.dy_c0_step = a.dy_views == 1 ? 64 : 0;
 
   {

@@ -457,11 +457,10 @@ class GraphedMultiGeneratorStep:
         self.lr = lr_example.detach().clone()
         self.hr = hr_example.detach().clone()
         K = len(self.generators)
-        import os
         if joint is None:
             # the joint launch pays off where the fused trunk kernel is the preferred path (see srg_set_trunk_fused);
             # warm-up falls back to per-generator branches when the engines refuse the split execution
-            joint = K <= 4 and os.environ.get("SRG_JOINT_TRUNK", "1") != "0"
+            joint = K <= 4
         self.joint = bool(joint)
         self.streams = [torch.cuda.Stream() for _ in range(K)]
         snaps = []

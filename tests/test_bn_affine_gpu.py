@@ -100,14 +100,11 @@ def _grads(g):
 
 
 # ------------------------------------------------------------------------------------------------ a. training, per layer
-TRAIN_MODES = [pytest.param(0, None, id="per-layer"), pytest.param(1, None, id="fused-trunk"),
-               pytest.param(0, "SRG_FIN_FUSED", id="fin-fused"), pytest.param(0, "SRG_REDUCE_FINAL", id="reduce-final")]
+TRAIN_MODES = [pytest.param(0, id="per-layer"), pytest.param(1, id="fused-trunk")]
 
 
-def _train_run(S, monkeypatch, sd, x, dsr, trunk_mode, switch, names):
+def _train_run(S, sd, x, dsr, trunk_mode, names):
     L = S.lib()
-    if switch:
-        monkeypatch.setenv(switch, "1")                 # read at engine creation
     old = L.srg_set_trunk_fused(trunk_mode)
     try:
         g = _module(S, sd).train()
@@ -122,24 +119,22 @@ def _train_run(S, monkeypatch, sd, x, dsr, trunk_mode, switch, names):
         return T, _grads(g), _cpu_state(g)
     finally:
         L.srg_set_trunk_fused(old)
-        if switch:
-            monkeypatch.delenv(switch)
 
 
-@pytest.mark.parametrize("trunk_mode,switch", TRAIN_MODES)
-def test_training_per_layer_all_blocks(S, monkeypatch, trunk_mode, switch):
+@pytest.mark.parametrize("trunk_mode", TRAIN_MODES)
+def test_training_per_layer_all_blocks(S, trunk_mode):
     """2x3x16x24, all 16 blocks, float64 references"""
     sd = _state(31)
     gen = torch.Generator().manual_seed(32)
     x, dsr = torch.rand(2, 3, 16, 24, generator=gen), torch.randn(2, 3, 64, 96, generator=gen) * 1e-3
-    T, G, after = _train_run(S, monkeypatch, sd, x, dsr, trunk_mode, switch, _trunk_names(16))
+    T, G, after = _train_run(S, sd, x, dsr, trunk_mode, _trunk_names(16))
     bad = Bad()
     check_trunk(bad, "", T, G, B.to_double(sd), after, range(16), 16, torch.float64)
     assert not bad, bad
 
 
-@pytest.mark.parametrize("trunk_mode,switch", TRAIN_MODES)
-def test_training_per_layer_cfg2(S, monkeypatch, trunk_mode, switch):
+@pytest.mark.parametrize("trunk_mode", TRAIN_MODES)
+def test_training_per_layer_cfg2(S, trunk_mode):
     """16x3x96x96 (BASELINE configs[1]): blocks 0, 7 and 15, the layers test_full_size_layers_against_fp32_oracle_cfg2
     walks, fp32 references"""
     sd = _state(33)
@@ -147,7 +142,7 @@ def test_training_per_layer_cfg2(S, monkeypatch, trunk_mode, switch):
     x, dsr = torch.rand(16, 3, 96, 96, generator=gen), torch.randn(16, 3, 384, 384, generator=gen) * 1e-4
     names = ["out1", "d_last", "rb1.d_in", "rb6.out", "rb8.d_in", "rb14.out"] + \
         [f"rb{b}.{n}" for b in (0, 7, 15) for n in ("y1", "z1", "y2", "out", "d_y2", "d_pre1", "d_y1", "d_in")]
-    T, G, after = _train_run(S, monkeypatch, sd, x, dsr, trunk_mode, switch, names)
+    T, G, after = _train_run(S, sd, x, dsr, trunk_mode, names)
     bad = Bad()
     check_trunk(bad, "", T, G, sd, after, (0, 7, 15), 16, torch.float32)
     assert not bad, bad
@@ -268,7 +263,7 @@ EVAL_CASES = [
 
 @pytest.mark.parametrize("n_res,upscale,shape", EVAL_CASES)
 def test_eval_forward_against_oracle(S, n_res, upscale, shape):
-    """The eval forward (BatchNorm folded into the conv epilogue, bn_eval_coeffs_all_kernel) for conv variants 0-3.  End to
+    """The eval forward (BatchNorm folded into the conv epilogue, bn_eval_coeffs_all_kernel) for conv variants 0 and 1.  End to
     end against O.srresnet_forward(training=False) with the calibrated bounds of bn_affine_state; for 1-2 blocks also
     each stored segment at TOL_LAYER, fed the engine's own input: the folded trunk from out1, every up-sampling stage, the
     output conv."""
@@ -288,7 +283,7 @@ def test_eval_forward_against_oracle(S, n_res, upscale, shape):
     L = S.lib()
     bad = Bad()
     figures = []
-    for variant in range(4):
+    for variant in range(2):
         old = L.srg_set_conv_variant(variant)
         try:
             with torch.no_grad():

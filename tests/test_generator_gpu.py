@@ -670,7 +670,7 @@ def test_full_size_properties_cfg2(S):
 
 
 def test_kernel_families_agree_at_full_size_cfg2(S):
-    """The specialised convolution kernels (conv3_il in both strip forms, conv9_rows, batched weight gradients) against
+    """The specialised convolution kernels (conv3_il, conv9_rows, batched weight gradients) against
     the generic strip kernel at the BASELINE configs[1] geometry: same bf16 operands and fp32 accumulation in a
     different tap order; every one of the 37 layers stores bf16, so a different accumulation order flips roundings
     and the families agree to bf16 storage noise compounded over the depth (measured 47 dB), not to fp32 noise."""
@@ -682,7 +682,7 @@ def test_kernel_families_agree_at_full_size_cfg2(S):
     state = {k: v.clone() for k, v in g.state_dict().items()}
     outs, grads = {}, {}
     try:
-        for variant in (1, 2, 3):
+        for variant in (1, 0):
             L.srg_set_conv_variant(variant)
             g.load_state_dict(state)
             g.eval()
@@ -696,7 +696,7 @@ def test_kernel_families_agree_at_full_size_cfg2(S):
             grads[variant] = g.flat_grads().clone()
     finally:
         L.srg_set_conv_variant(0)
-    for variant in (2, 3):
+    for variant in (0,):
         mse = float(((outs[variant] - outs[1]).double() ** 2).mean())
         assert mse < 1e-4 * float((outs[1].double() ** 2).mean()), (variant, mse)               # > 40 dB
         assert maxrel(outs[variant], outs[1]) < 5e-2, (variant, maxrel(outs[variant], outs[1]))
@@ -705,7 +705,6 @@ def test_kernel_families_agree_at_full_size_cfg2(S):
         # (test_backward_layers_isolated), here only gross disagreement is excluded
         rel = float((grads[variant] - grads[1]).norm() / grads[1].norm())
         assert rel < 0.3, (variant, rel)
-    assert maxrel(outs[2], outs[3]) < 5e-2      # same operands, MMAs issued in a different order (strip-major vs parity-major)
 
 
 def test_full_size_layers_against_fp32_oracle_cfg2(S):
@@ -901,38 +900,3 @@ def test_eval_forward_streams_frames_bit_identically(S):
     with torch.no_grad():
         g(x)
     assert g.last_engine().N == 5
-
-
-@pytest.mark.parametrize("switch", ["SRG_FIN_FUSED", "SRG_REDUCE_FINAL"])
-def test_finalize_fused_batchnorm_passes_match_separate_finalize(S, monkeypatch, switch):
-    """SRG_FIN_FUSED=1 (BatchNorm statistics finalize inside the apply / backward-apply pass, csrc/elementwise.cu
-    bn_apply_fin / bn_bwd_apply_fin) and SRG_REDUCE_FINAL=1 (the BatchNorm-backward reduction's last block finalizes,
-    chan_reduce_final_kernel) against the default two-launch form on the same weights and inputs: same partial
-    sums, summed in fp64 in a different fixed order, so intermediates agree to a bf16 ulp in the first block and the
-    parameter gradients to rounding noise through the chain."""
-    res = []
-    old_mode = S.lib().srg_set_trunk_fused(0)             # per-layer launches (the tiny geometry would pick the fused trunk)
-    for flag in ("0", "1"):
-        monkeypatch.setenv(switch, flag)                  # read at engine creation
-        torch.manual_seed(11)
-        g = S.SRResNet().cuda().train()
-        torch.manual_seed(12)
-        x = torch.rand(3, 3, 40, 24).cuda()
-        y = g(x)
-        y.backward(torch.sin(torch.arange(y.numel(), device="cuda", dtype=torch.float32)).reshape(y.shape) * 1e-3)
-        torch.cuda.synchronize()
-        eng = g.last_engine()
-        T = {n: eng.named_tensor(n).float().clone() for n in ("rb0.y1", "rb0.z1", "rb0.out", "rb15.out", "trunk")}
-        res.append((y.detach().clone(), T, {k: p.grad.detach().clone() for k, p in g.named_parameters()},
-                    {k: v.clone() for k, v in g.state_dict().items() if "running" in k}, S.lib().srg_generator_launch_count(eng.handle)))
-    S.lib().srg_set_trunk_fused(old_mode)
-    (y0, T0, G0, R0, n0), (y1, T1, G1, R1, n1) = res
-    assert n1 < n0                                        # 64 (32 with SRG_REDUCE_FINAL) fewer launches per forward + backward
-    for n in ("rb0.y1", "rb0.z1", "rb0.out"):
-        assert maxrel(T1[n], T0[n]) < 4e-3, n
-    assert maxrel(y1, y0) < 5e-2
-    for k in R0:
-        assert maxrel(R1[k], R0[k]) < (1e-5 if k.startswith("residual_blocks.0.bn1") else 1e-2), k
-    for k in G0:
-        if float(G0[k].abs().max()) > 0:
-            assert l2rel(G1[k], G0[k]) < 0.35, (k, l2rel(G1[k], G0[k]))

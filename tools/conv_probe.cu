@@ -51,7 +51,7 @@ struct Problem {
   bool residual, mask;
   int out_mode;
   bool stats;                // exercise the fused BatchNorm-statistics epilogue (timing only)
-  int variant;               // ConvGemmArgs::variant: 1 = generic strip kernel, 2 = row-interleaved conv3_il
+  int variant;               // ConvGemmArgs::variant: 0 = specialised kernels (conv3_il, conv9_rows), 1 = generic strip kernel
 };
 
 static int run(const Problem& pr, int timing_iters) {
@@ -131,11 +131,6 @@ static int run(const Problem& pr, int timing_iters) {
   a.out = dout; a.out_mode = pr.out_mode; a.variant = pr.variant;
   float* dstats = nullptr;
   if (pr.stats) { CK(cudaMalloc(&dstats, 148 * 128 * 4)); a.stats = dstats; }
-  static void* dstats_y = nullptr;        // second factor of the product statistics (timing only): a separate tensor of the output's geometry
-  if (pr.stats && getenv("PROBE_STATS_Y") != nullptr) {
-    if (!dstats_y) { CK(cudaMalloc(&dstats_y, size_t(48) * 96 * 96 * 64 * 2)); CK(cudaMemset(dstats_y, 0, size_t(48) * 96 * 96 * 64 * 2)); }
-    a.stats_y = dstats_y;
-  }
 
   int rc = launch_conv_gemm(a, 0);
   if (rc != 0) { printf("[%s] launch rc=%d err=%s\n", pr.name, rc, last_error()); return 1; }
@@ -488,12 +483,12 @@ int main(int argc, char** argv) {
   const int iters = argc > 1 ? atoi(argv[1]) : 0;
   int fails = 0;
   if (getenv("PROBE_IL_ONLY") != nullptr) {   // quick mode: the cfg2 trunk cases of the row-interleaved kernel only
-    { Problem p = conv3x3("perf_il_trunk_16x96x96", 16, 96, 96, 64, false); p.variant = 3; fails += run(p, iters); }
-    { Problem p = conv3x3("perf_il_trunk_stats", 16, 96, 96, 64, false); p.variant = 3; p.stats = true; fails += run(p, iters); }
-    { Problem p = conv3x3("perf_il_trunk_mask", 16, 96, 96, 64, false); p.variant = 3; p.mask = true; p.bias = false; fails += run(p, iters); }
-    { Problem p = conv3x3("perf_il_trunk_residual", 16, 96, 96, 64, false); p.variant = 3; p.residual = true; p.bias = false; fails += run(p, iters); }
-    { Problem p = conv3x3("perf_il_trunk_mask_stats", 16, 96, 96, 64, false); p.variant = 3; p.mask = true; p.bias = false; p.stats = true; fails += run(p, iters); }
-    { Problem p = conv3x3("perf_il_trunk_48x96x96", 48, 96, 96, 64, false); p.variant = 3; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_16x96x96", 16, 96, 96, 64, false); p.variant = 0; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_stats", 16, 96, 96, 64, false); p.variant = 0; p.stats = true; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_mask", 16, 96, 96, 64, false); p.variant = 0; p.mask = true; p.bias = false; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_residual", 16, 96, 96, 64, false); p.variant = 0; p.residual = true; p.bias = false; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_mask_stats", 16, 96, 96, 64, false); p.variant = 0; p.mask = true; p.bias = false; p.stats = true; fails += run(p, iters); }
+    { Problem p = conv3x3("perf_il_trunk_48x96x96", 48, 96, 96, 64, false); p.variant = 0; fails += run(p, iters); }
     printf("PROBE %s (%d failing cases)\n", fails == 0 ? "PASS" : "FAIL", fails);
     return fails == 0 ? 0 : 1;
   }
@@ -567,12 +562,13 @@ int main(int argc, char** argv) {
       p.TH = 4; p.TW = 32;
       p.n_strips = 1; p.n_taps = 9; p.strip_rows = 4 + 8; p.strip_dh = -4; p.strip_dw[0] = 0;
       for (int r = 0; r < 9; ++r) p.tap_row[r] = r;
-      p.block_n = 32; p.out_mode = OUT_FOLD9_NCHW; p.variant = 2;
+      p.block_n = 32; p.out_mode = OUT_FOLD9_NCHW; p.variant = 0;
       fails += run(p, 0);
     }
   }
-  for (int var = 2; var <= 3; ++var) {  // row-interleaved 3x3 kernel (conv3_il): 2 = one 8-pixel strip per shift, 3 = one 10-pixel strip
-    printf("-- conv3_il variant %d\n", var);
+  {  // row-interleaved 3x3 kernel (conv3_il)
+    const int var = 0;
+    printf("-- conv3_il\n");
     Problem p = conv3x3("il_small", 2, 32, 24, 64, false); p.variant = var; fails += run(p, 0);
     Problem r = conv3x3("il_ragged", 3, 40, 20, 64, false); r.variant = var; fails += run(r, 0);
     Problem o = conv3x3("il_odd_rows", 2, 37, 13, 64, false); o.variant = var; o.act = ACT_RELU; fails += run(o, 0);
@@ -582,8 +578,9 @@ int main(int argc, char** argv) {
     Problem t = conv3x3("il_many_tiles", 5, 96, 96, 64, false); t.variant = var; t.residual = true; fails += run(t, 0);
   }
   if (iters > 0) {
-    for (int var = 2; var <= 3; ++var) {
-      printf("-- conv3_il variant %d\n", var);
+    {
+      const int var = 0;
+      printf("-- conv3_il\n");
       { Problem p = conv3x3("perf_il_trunk_16x96x96", 16, 96, 96, 64, false); p.variant = var; fails += run(p, iters); }
       { Problem p = conv3x3("perf_il_trunk_stats", 16, 96, 96, 64, false); p.variant = var; p.stats = true; fails += run(p, iters); }
       { Problem p = conv3x3("perf_il_trunk_mask", 16, 96, 96, 64, false); p.variant = var; p.mask = true; p.bias = false; fails += run(p, iters); }
@@ -601,7 +598,7 @@ int main(int argc, char** argv) {
       Problem f = conv3x3("perf_c9rows_16x384x384", 16, 384, 384, 32, false);
       f.TH = 4; f.TW = 32; f.n_strips = 1; f.n_taps = 9; f.strip_rows = 12; f.strip_dh = -4; f.strip_dw[0] = 0;
       for (int r = 0; r < 9; ++r) f.tap_row[r] = r;
-      f.block_n = 32; f.out_mode = OUT_FOLD9_NCHW; f.variant = 2;
+      f.block_n = 32; f.out_mode = OUT_FOLD9_NCHW; f.variant = 0;
       fails += run(f, iters);
     }
     Problem f = conv3x3("perf_fold9_16x384x384", 16, 384, 384, 32, false);
